@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA engine
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port), host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also save each workload's final ADMM state as DIR/*.npy
 
 A "step" is one ADMM iteration (SURVEY §8(d)): consensus z-update + every agent's train_and_update equivalent
 (2P+1 parameter sets -> features -> Gram -> Cholesky/inverse -> fused central-difference gradient -> local
@@ -25,6 +26,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True           # the benchmark leaves the source tree as it found it (it may be read-only)
 
 WORKLOADS = {
     # BASELINE.json configs[3]: the configuration the metric is quoted on at 1/2/4/8 GPUs
@@ -42,6 +44,7 @@ WORKLOADS = {
                  N=900, d=2, encoding="chebyshev", kernel="projected", q=3, layers=1, outer="matern", agents=4, honour_outer=False),
 }
 NOISE_STD, RHO, LIP, H = 0.1, 100.0, 100.0, np.pi / 8
+HBM_COPY_GBS = 6547.5                    # denominator of the Gram's HBM roofline: copy bandwidth measured on a B200 (BASELINE.md section 2)
 
 
 def load_json(path, default=None):
@@ -76,6 +79,7 @@ class ClockSampler:
         if self.proc is None:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         self.proc.terminate()
+        self.proc.wait()
         sm, mx, reasons = [], None, set()
         for r in self.rows:
             try:
@@ -161,6 +165,15 @@ def copy_args(args, **kw):
     return out
 
 
+def dump_outputs(out_dir, workload_name, **arrays):
+    """What a caller of the timed path receives after its last step (AdmmEngine.state(): consensus z, every agent's theta and
+    psi, every agent's NLL) as float64 DIR/<workload>_<name>.npy.  Inputs are seeded, so the same arguments give the same
+    inputs on every run and two builds can be compared file by file.  A few KB per workload (A x P values)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{workload_name}_{name}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def measure(args, w, workload_name, pg, world, rank, local_rank, full):
     import torch
     import torch.distributed as dist
@@ -198,19 +211,30 @@ def measure(args, w, workload_name, pg, world, rank, local_rank, full):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    barrier()
-    e0.record()
-    for _ in range(args.steps):
-        step_fn()
-    e1.record()
-    barrier()
+    try:                                     # no nvidia-smi sampler outlives a failed step
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        barrier()
+        e0.record()
+        for _ in range(args.steps):
+            step_fn()
+        e1.record()
+        barrier()
+    finally:
+        clocks = sampler.stop() if rank == 0 else None
     ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     total_ms = float(ms.item())
-    clocks = sampler.stop() if rank == 0 else None
-    z_final, theta_final, _, nll = eng.state()
+    z_final, theta_final, psi_final, nll = eng.state()
+    if args.dump_outputs:
+        nll_all = nll
+        if world > 1:                        # z, theta, psi are replicated after the exchange; the NLLs are per rank
+            local = torch.from_numpy(nll).cuda()
+            gathered = torch.empty(world * local.numel(), dtype=local.dtype, device="cuda")
+            dist.all_gather_into_tensor(gathered, local)
+            nll_all = gathered.cpu().numpy()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, workload_name, z=z_final, theta=theta_final, psi=psi_final, nll=nll_all)
 
     # ---- per-phase device times of ONE agent step (same stream, CUDA events), after the timed region -------------
     ag = eng.agents[0]
@@ -234,8 +258,6 @@ def measure(args, w, workload_name, pg, world, rank, local_rank, full):
     timed("gradient", ag.gradient)
     fp64 = load_json(os.path.join(ROOT, "profiles", "r01_fp64_peak.json"), {})
     peak_tf = float(fp64.get("dmma_m8n8k4_tflops", 37.1))
-    peaks = load_json(os.path.join(ROOT, "MEASURED_PEAKS.json"), {})
-    hbm_peak = float(peaks.get("hbm_gbs", 6650.0))
     fpe = flops_per_entry(w)
     np_pad = ((n_i + 127) // 128) * 128
     grad_flops = 2 * P * n_i * n_i * fpe                     # algorithmic: full squares of the 2P shifted Grams
@@ -262,7 +284,7 @@ def measure(args, w, workload_name, pg, world, rank, local_rank, full):
                              "64x64 tiles only (symmetry), same per-entry count: the fraction of the pipe's peak that is comparable with 1"},
         "factor": {"bound": "fp64-dmma", "achieved": chol_flops / (phases["factor"] * 1e-3) / 1e12, "peak": peak_tf, "unit": "TFLOP/s",
                    "note": "n^3 flops: potrf + triangular inverse + inverse product, DMMA.8x8x4 trailing updates"},
-        "gram": {"bound": "hbm", "achieved": 8.0 * gram_entries / (phases["gram"] * 1e-3) / 1e9, "peak": hbm_peak, "unit": "GB/s",
+        "gram": {"bound": "hbm", "achieved": 8.0 * gram_entries / (phases["gram"] * 1e-3) / 1e9, "peak": HBM_COPY_GBS, "unit": "GB/s",
                  "note": "8 B per written entry of the unshifted Gram; the training Gram writes the 64x64 tiles of the lower "
                          "triangle only (all the factorisation reads)" if w["kernel"] == "projected" else "8 B per written entry of the unshifted Gram"},
     }
@@ -286,8 +308,8 @@ def measure(args, w, workload_name, pg, world, rank, local_rank, full):
     primary.update({"kernel": {"gradient": "grad_projected_dmma_kernel" if w["kernel"] == "projected" else "fidelity_dmma_kernel<1>",
                                "factor": "gemm_group_kernel" if os.environ.get("DQGP_GEMM_NO_TMAP") else "gemm_group_tmap_kernel", "gram": "gram_projected_dmma_kernel",
                                "statevector": ("statevec_lc2_kernel<%d>" if w["encoding"] in ("yz_cx", "kyriienko") else "statevec_lc_kernel<%d>") % w["q"]}[dominant], "phase": dominant,
-                    "traffic": None, "peak_source": "profiles/r01_fp64_peak.json (measured on this pool: pure DMMA/DFMA issue loops)"
-                    if primary["bound"] != "hbm" else "MEASURED_PEAKS.json"})
+                    "traffic": None, "peak_source": "profiles/r01_fp64_peak.json (pure DMMA/DFMA issue loops measured on a B200)"
+                    if primary["bound"] != "hbm" else "BASELINE.md section 2 (HBM copy, read + write, measured on a B200)"})
 
     tk = traffic.get(primary["kernel"].replace("grad_projected_kernel", "grad_projected_dmma_kernel"), {})
     if tk.get("dram_bytes"):
@@ -416,22 +438,17 @@ def run_reference(args, w):
     P = circuits.num_parameters(w["encoding"], w["q"], w["layers"])
     n_i = w["N"] // w["agents"]
     S = 2 * P + 1
-    requested_steps, requested_warmup = args.steps, args.warmup
-    vals, t_start, budget_s = [], time.perf_counter(), 150.0
+    vals = []
     for i in range(args.warmup + args.steps):
         r = cpu_reference_sample(w, n_i, P)
         if i >= args.warmup:
             vals.append(r)
-        elif time.perf_counter() - t_start > budget_s / 3:
-            args.warmup = i + 1                         # each sample is seconds of CPU work: cap the untimed part
-        if vals and time.perf_counter() - t_start > budget_s:
-            break                                       # keep the whole run within a few minutes (bounded sample)
     v = float(np.mean([r["value"] for r in vals]))
     base = dict(vals[-1]); base["value"] = v
     line = {"impl": "reference", "metric": "quantum_kernel_entries_per_s", "value": v, "unit": "entries/s",
             # each "step" of this arm is a BOUNDED SAMPLE of one iteration (see cpu_baseline.sample), not a whole iteration:
             # ms_per_step and admm_iters_per_s are extrapolations from the measured entries/s
-            "extrapolated": True, "steps_requested": requested_steps, "warmup_requested": requested_warmup,
+            "extrapolated": True,
             "admm_iters_per_s": v / (w["agents"] * S * n_i * n_i), "n_gpus": world, "steps": len(vals), "warmup": args.warmup,
             "ms_per_step": 1e3 * (w["agents"] * S * n_i * n_i) / v, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
             "dtype": "f64", "data": "synthetic",
@@ -457,7 +474,13 @@ def main():
     ap.add_argument("--skip-e2e", action="store_true", help="profiling runs only")
     ap.add_argument("--outer-blocks", type=int, default=0, help="Cholesky outer panel width in 128-blocks (0 = engine default)")
     ap.add_argument("--graph", default="auto", choices=["auto", "on", "off"], help="replay the iteration as a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, save each measured workload's final z / theta / psi / per-agent NLL as DIR/<workload>_<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times Gram samples, not whole iterations)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = max(args.warmup, 1)
     w = WORKLOADS[args.workload]
