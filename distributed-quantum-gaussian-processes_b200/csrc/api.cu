@@ -23,7 +23,7 @@ int dqgp_dgemm(int a_k_contig, int b_k_contig, int M, int N, int K, double alpha
     DQGP_CUDA(cudaMallocAsync(&d_t, sizeof t, st));
     DQGP_CUDA(cudaMemcpyAsync(d_t, &t, sizeof t, cudaMemcpyHostToDevice, st));
     DQGP_CUDA(cudaStreamSynchronize(st));   // `t` lives on this stack frame
-    gemm_register_maps(d_t, &t, 1);          // tensor maps of the operands (DQGP_GEMM_NO_TMAP: none)
+    gemm_register_maps(d_t, &t, 1);          // tensor maps of the operands
     int rc = launch_gemm_group(d_t, 1, t.tiles, st);
     DQGP_CUDA(cudaStreamSynchronize(st));    // the maps (if any) are freed below
     gemm_unregister_maps(d_t);

@@ -797,7 +797,7 @@ static int solver_create_impl(int n, int outer_blocks, int lean, dqgp_solver** o
 
     e = cudaMalloc(&s->d_tasks, sizeof(GemmTask) * tasks.size());
     if (e == cudaSuccess) e = cudaMemcpy(s->d_tasks, tasks.data(), sizeof(GemmTask) * tasks.size(), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) gemm_register_maps(s->d_tasks, tasks.data(), (int)tasks.size());      // tensor maps of the operands (DQGP_GEMM_NO_TMAP: none)
+    if (e == cudaSuccess) gemm_register_maps(s->d_tasks, tasks.data(), (int)tasks.size());      // tensor maps of the operands
     if (e == cudaSuccess) {
         int lo = 0, hi = 0;
         cudaDeviceGetStreamPriorityRange(&lo, &hi);

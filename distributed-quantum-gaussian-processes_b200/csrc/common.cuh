@@ -125,7 +125,7 @@ struct SvPass {
     int lead_end, trail_begin;
 };
 
-// Plan of the CX-free simulator (statevec_lc2_kernel<.., MAPPED = true>): circuits made of 1-qubit gates and CX only.  A CX is never
+// Plan of the CX-free simulator (statevec_lc2_kernel): circuits made of 1-qubit gates and CX only.  A CX is never
 // executed: amplitudes stay where they are and the map from LOGICAL basis index x to PHYSICAL position p = M x (M over GF(2), one
 // column mask per logical qubit) absorbs it - CX(c -> t) replaces the control's mask m_c by m_c ^ m_t.  A pass applies the fused 2x2
 // unitaries of <= 3 logical qubits: a thread owns the coset of span{bm} selected by the bits of its index (bit i <-> rest[i]),

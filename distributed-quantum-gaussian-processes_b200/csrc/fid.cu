@@ -6,8 +6,7 @@
 // MODE 0 writes the Gram (FidelityKernel.evaluate, reference main.py:118-124); MODE 1 is the fused central-difference
 // gradient over the 2P shifted state sets (agent_riemannian.py:270-275,431-436), lower tiles only, B = A^-1 - alpha
 // alpha^T in registers, deterministic two-stage reduction.  Operand chunks of 32 doubles stream through a
-// double-buffered cp.async ring.  Replaces the SIMT kernels of gram.cu / grad.cu (kept behind DQGP_FID_SIMT).
-#include <cstdlib>
+// double-buffered ring filled by the TMA engine.
 #include <cstring>
 #include "pairwise.cuh"
 #include "tensormap.cuh"
@@ -19,20 +18,8 @@ constexpr int FD_PITCH = FD_KC + 4;            // = 4 (mod 16): conflict-free fr
 constexpr int FD_STAGE = 2 * PW_TILE * FD_PITCH;
 constexpr size_t FD_SMEM = sizeof(double) * 2 * FD_STAGE;
 
-__device__ __forceinline__ void fd_stage(double* buf, const double* __restrict__ S1, const double* __restrict__ S2, int row0,
-                                         int col0, int n1, int n2, int d2, int k0, int kc) {
-    const int r = threadIdx.x >> 2, l4 = threadIdx.x & 3;
-    const double* src_r = S1 + (size_t)min(row0 + r, n1 - 1) * d2 + k0;
-    const double* src_c = S2 + (size_t)min(col0 + r, n2 - 1) * d2 + k0;
-    double* dst_r = buf + r * FD_PITCH;
-    double* dst_c = buf + PW_TILE * FD_PITCH + r * FD_PITCH;
-    for (int k = 2 * l4; k < kc; k += 8) {
-        cp_async16(dst_r + k, src_r + k);
-        cp_async16(dst_c + k, src_c + k);
-    }
-}
-
-// the same chunk through the bulk-copy (TMA) engine: one cp.async.bulk per state row (kc doubles), bytes counted on `bar`
+// MODE 0 (two state arrays): one chunk through the bulk-copy (TMA) engine, one cp.async.bulk per state row (kc doubles, a multiple of
+// 16 bytes from a 16-byte aligned row), bytes counted on `bar`
 __device__ __forceinline__ void fd_stage_bulk(double* buf, const double* __restrict__ S1, const double* __restrict__ S2, int row0,
                                               int col0, int n1, int n2, int d2, int k0, int kc, unsigned long long* bar) {
     if (threadIdx.x == 0) mbar_arrive_expect_tx(bar, 2u * PW_TILE * kc * sizeof(double));
@@ -43,7 +30,7 @@ __device__ __forceinline__ void fd_stage_bulk(double* buf, const double* __restr
     }
 }
 
-// ... and as two boxes of a 3-D tensor map over Psi = [set][state][2 * 2^q doubles] (TMA proper, SASS UTMALDG), issued by one thread: box =
+// MODE 1 (one state array): the chunk as two boxes of a 3-D tensor map over Psi = [set][state][2 * 2^q doubles] (TMA proper, SASS UTMALDG), issued by one thread: box =
 // 64 states x FD_PITCH doubles starting at the chunk; the four doubles beyond the chunk land in the padding of the fragment layout (never
 // read), states beyond n arrive as zero rows (their bracket weights are zero).
 __device__ __forceinline__ void fd_stage_tmap(double* buf, const void* tmap, int set, int row0, int col0, int k0, unsigned long long* bar) {
@@ -54,8 +41,8 @@ __device__ __forceinline__ void fd_stage_tmap(double* buf, const void* tmap, int
     }
 }
 
-// TMAP (MODE 1 only: one state array): stage through the tensor map `tmap`
-template <int MODE, bool BULK = true, bool TMAP = false>
+// dim = 2^q amplitudes (d2 = 2 dim doubles, q >= 1) and 16-byte aligned states: the host entry points check both
+template <int MODE>
 __global__ void __launch_bounds__(PW_THREADS, 1) fidelity_dmma_kernel(const double* __restrict__ Psi1, int n1,
                                                                       const double* __restrict__ Psi2, int n2, int d2, int n_sets,
                                                                       double* __restrict__ K, int ldk,
@@ -66,10 +53,8 @@ __global__ void __launch_bounds__(PW_THREADS, 1) fidelity_dmma_kernel(const doub
     extern __shared__ __align__(128) double fd_smem[];
     __shared__ double s_red[2][PW_THREADS / 32];
     __shared__ __align__(8) unsigned long long s_bar[2];
-    if (BULK) {
-        if (threadIdx.x == 0) { mbar_init(&s_bar[0], 1); mbar_init(&s_bar[1], 1); mbar_fence_init(); }
-        __syncthreads();
-    }
+    if (threadIdx.x == 0) { mbar_init(&s_bar[0], 1); mbar_init(&s_bar[1], 1); mbar_fence_init(); }
+    __syncthreads();
     int bi, bj;
     if (MODE == 1) {
         bi = int((sqrt(8.0 * blockIdx.x + 1.0) - 1.0) * 0.5);
@@ -106,16 +91,13 @@ __global__ void __launch_bounds__(PW_THREADS, 1) fidelity_dmma_kernel(const doub
     const size_t set_stride1 = (size_t)n1 * d2, set_stride2 = (size_t)n2 * d2;
     const int first_set = (MODE == 1) ? 1 : 0;
     const int total = n_sets * n_chunks;
-    if (TMAP) fd_stage_tmap(fd_smem, &tmap, first_set, row0, col0, 0, &s_bar[0]);
-    else if (BULK) fd_stage_bulk(fd_smem, Psi1 + first_set * set_stride1, Psi2 + first_set * set_stride2, row0, col0, n1, n2, d2, 0, kc, &s_bar[0]);
-    else fd_stage(fd_smem, Psi1 + first_set * set_stride1, Psi2 + first_set * set_stride2, row0, col0, n1, n2, d2, 0, kc);
-    cp_async_commit();
+    if (MODE == 1) fd_stage_tmap(fd_smem, &tmap, first_set, row0, col0, 0, &s_bar[0]);
+    else fd_stage_bulk(fd_smem, Psi1 + first_set * set_stride1, Psi2 + first_set * set_stride2, row0, col0, n1, n2, d2, 0, kc, &s_bar[0]);
     double re[2][4][2], im[2][4][2];
     double pplus = 0.0;
     for (int it = 0; it < total; ++it) {
         const int set = it / n_chunks, ch = it - set * n_chunks;
-        if (BULK) mbar_wait(&s_bar[it & 1], (it >> 1) & 1);
-        else cp_async_wait<0>();
+        mbar_wait(&s_bar[it & 1], (it >> 1) & 1);
         __syncthreads();
         if (MODE == 1 && ch == 0 && set >= 2 && (set & 1) == 0 && threadIdx.x == 0) {
             const int i = (set >> 1) - 1;
@@ -126,16 +108,12 @@ __global__ void __launch_bounds__(PW_THREADS, 1) fidelity_dmma_kernel(const doub
         }
         if (it + 1 < total) {
             const int ns = (it + 1) / n_chunks, nch = (it + 1) - ns * n_chunks;
-            if (TMAP)
+            if (MODE == 1)
                 fd_stage_tmap(fd_smem + ((it + 1) & 1) * FD_STAGE, &tmap, first_set + ns, row0, col0, nch * kc, &s_bar[(it + 1) & 1]);
-            else if (BULK)
+            else
                 fd_stage_bulk(fd_smem + ((it + 1) & 1) * FD_STAGE, Psi1 + (size_t)(first_set + ns) * set_stride1,
                               Psi2 + (size_t)(first_set + ns) * set_stride2, row0, col0, n1, n2, d2, nch * kc, kc, &s_bar[(it + 1) & 1]);
-            else
-                fd_stage(fd_smem + ((it + 1) & 1) * FD_STAGE, Psi1 + (size_t)(first_set + ns) * set_stride1,
-                         Psi2 + (size_t)(first_set + ns) * set_stride2, row0, col0, n1, n2, d2, nch * kc, kc);
         }
-        cp_async_commit();
         if (ch == 0) {
 #pragma unroll
             for (int rb = 0; rb < 2; ++rb)
@@ -211,9 +189,6 @@ static int fd_attr() {
     if (!done) {
         DQGP_CUDA(cudaFuncSetAttribute(fidelity_dmma_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FD_SMEM));
         DQGP_CUDA(cudaFuncSetAttribute(fidelity_dmma_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FD_SMEM));
-        DQGP_CUDA(cudaFuncSetAttribute(fidelity_dmma_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FD_SMEM));
-        DQGP_CUDA(cudaFuncSetAttribute(fidelity_dmma_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FD_SMEM));
-        DQGP_CUDA(cudaFuncSetAttribute(fidelity_dmma_kernel<1, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FD_SMEM));
         done = true;
     }
     return 0;
@@ -223,11 +198,9 @@ int fidelity_gram_dmma(const double* Psi1, int n1, const double* Psi2, int n2, i
     int rc = fd_attr();
     if (rc) return rc;
     dim3 grid((n2 + PW_TILE - 1) / PW_TILE, (n1 + PW_TILE - 1) / PW_TILE);
-    static const bool no_bulk = getenv("DQGP_FID_NO_BULK") != nullptr;      // A/B: per-thread cp.async staging
     CUtensorMap tmap;                                                       // unused by the Gram (two state arrays): per-row bulk copies
     memset(&tmap, 0, sizeof(tmap));
-    if (no_bulk) fidelity_dmma_kernel<0, false><<<grid, PW_THREADS, FD_SMEM, st>>>(Psi1, n1, Psi2, n2, 2 * dim, 1, K, ldk, nullptr, 0, nullptr, 0, nullptr, tmap);
-    else fidelity_dmma_kernel<0><<<grid, PW_THREADS, FD_SMEM, st>>>(Psi1, n1, Psi2, n2, 2 * dim, 1, K, ldk, nullptr, 0, nullptr, 0, nullptr, tmap);
+    fidelity_dmma_kernel<0><<<grid, PW_THREADS, FD_SMEM, st>>>(Psi1, n1, Psi2, n2, 2 * dim, 1, K, ldk, nullptr, 0, nullptr, 0, nullptr, tmap);
     DQGP_LAUNCH_CHECK("fidelity_dmma_kernel<0>");
     return 0;
 }
@@ -236,15 +209,13 @@ int fidelity_grad_dmma(const double* Ainv, int ld, const double* alpha, const do
                        int tiles, cudaStream_t st) {
     int rc = fd_attr();
     if (rc) return rc;
-    static const bool no_bulk = getenv("DQGP_FID_NO_BULK") != nullptr;
-    // the state tiles of a parameter set as two boxes of a 3-D tensor map (one issuing thread) unless DQGP_FID_NO_TMAP is set or the
-    // driver refuses the map
+    // the state tiles of a parameter set as two boxes of a 3-D tensor map (one issuing thread).  For the arguments the entry point
+    // accepts (16-byte aligned base, 16 dim-byte rows, box of 36 x 64, dimensions below 2^32) the driver has no reason to refuse it.
     CUtensorMap tmap;
     memset(&tmap, 0, sizeof(tmap));
-    const bool have_tmap = !no_bulk && getenv("DQGP_FID_NO_TMAP") == nullptr && make_rows_tensor_map(&tmap, Psi, 2 * dim, n, 2 * P + 1, FD_PITCH, PW_TILE);
-    if (no_bulk) fidelity_dmma_kernel<1, false><<<tiles, PW_THREADS, FD_SMEM, st>>>(Psi, n, Psi, n, 2 * dim, 2 * P, nullptr, 0, Ainv, ld, alpha, P, partial, tmap);
-    else if (have_tmap) fidelity_dmma_kernel<1, true, true><<<tiles, PW_THREADS, FD_SMEM, st>>>(Psi, n, Psi, n, 2 * dim, 2 * P, nullptr, 0, Ainv, ld, alpha, P, partial, tmap);
-    else fidelity_dmma_kernel<1><<<tiles, PW_THREADS, FD_SMEM, st>>>(Psi, n, Psi, n, 2 * dim, 2 * P, nullptr, 0, Ainv, ld, alpha, P, partial, tmap);
+    DQGP_REQUIRE(make_rows_tensor_map(&tmap, Psi, 2 * dim, n, 2 * P + 1, FD_PITCH, PW_TILE),
+                 "dqgp_grad_fidelity: the driver refused the tensor map of the states (n %d, dim %d, P %d)", n, dim, P);
+    fidelity_dmma_kernel<1><<<tiles, PW_THREADS, FD_SMEM, st>>>(Psi, n, Psi, n, 2 * dim, 2 * P, nullptr, 0, Ainv, ld, alpha, P, partial, tmap);
     DQGP_LAUNCH_CHECK("fidelity_dmma_kernel<1>");
     return 0;
 }

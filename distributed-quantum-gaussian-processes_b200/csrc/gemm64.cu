@@ -7,7 +7,6 @@
 // A launch covers a *group* of independent tasks (device-resident table) so the many small products of
 // the recursive triangular inverse fill the machine in one launch.  Roofline: FP64 pipe (DMMA and DFMA
 // share it on B200: 37.1 TFLOP/s measured, profiles/r01_fp64_peak.json).
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 #include "gemm64.cuh"
@@ -37,21 +36,7 @@ __device__ __forceinline__ void gm_load_operand(double* sm, const double* __rest
     }
 }
 
-// The same operand tile through the bulk-copy (TMA) engine: one cp.async.bulk per contiguous run - a tile row of 16 k values (128 B)
-// when k is contiguous, a k-row of ROWS values otherwise - straight into the padded fragment layout, bytes counted on `bar`.
-// Threads [t0, t0 + copies) issue one copy each.
-template <int ROWS, int PITCH_R>
-__device__ __forceinline__ void gm_load_operand_bulk(double* sm, const double* __restrict__ g, int ld, int row0, int k0, int k_contig, int t0,
-                                                     unsigned long long* bar) {
-    const int i = (int)threadIdx.x - t0;
-    if (k_contig) {
-        if (i >= 0 && i < ROWS) bulk_copy_g2s(sm + i * GM_PITCH_K, g + (size_t)(row0 + i) * ld + k0, GM_KC * sizeof(double), bar);
-    } else {
-        if (i >= 0 && i < GM_KC) bulk_copy_g2s(sm + i * PITCH_R, g + (size_t)(k0 + i) * ld + row0, ROWS * sizeof(double), bar);
-    }
-}
-
-template <typename S, int AK, int BK, bool BULK, bool TMAP = false>
+template <typename S, int AK, int BK, bool TMAP>
 __device__ __forceinline__ void gemm_tile(const GemmTask& T, int local, double* gm_smem, const CUtensorMap* tmaps = nullptr);
 
 __device__ __forceinline__ int gm_find_task(const GemmTask* __restrict__ tasks, int n_tasks, int tile) {
@@ -63,7 +48,7 @@ __device__ __forceinline__ int gm_find_task(const GemmTask* __restrict__ tasks, 
     return lo;
 }
 
-template <typename S, bool BULK, bool TMAP = false>
+template <typename S, bool TMAP>
 __device__ __forceinline__ void gm_dispatch(const GemmTask* __restrict__ tasks, int n_tasks, double* gm_smem, const CUtensorMap* maps = nullptr) {
     // locate the task that owns this tile (tables are short: <= a few hundred entries)
     const int ti = gm_find_task(tasks, n_tasks, blockIdx.x);
@@ -72,9 +57,9 @@ __device__ __forceinline__ void gm_dispatch(const GemmTask* __restrict__ tasks, 
     const CUtensorMap* tm = TMAP ? maps + 2 * ti : nullptr;      // this task's A and B operand maps
     // operand layouts are compile-time inside the tile routine (no predicated duplicate fragment loads)
     if (T.a_k_contig) {
-        if (T.b_k_contig) gemm_tile<S, 1, 1, BULK, TMAP>(T, local, gm_smem, tm); else gemm_tile<S, 1, 0, BULK, TMAP>(T, local, gm_smem, tm);
+        if (T.b_k_contig) gemm_tile<S, 1, 1, TMAP>(T, local, gm_smem, tm); else gemm_tile<S, 1, 0, TMAP>(T, local, gm_smem, tm);
     } else {
-        if (T.b_k_contig) gemm_tile<S, 0, 1, BULK, TMAP>(T, local, gm_smem, tm); else gemm_tile<S, 0, 0, BULK, TMAP>(T, local, gm_smem, tm);
+        if (T.b_k_contig) gemm_tile<S, 0, 1, TMAP>(T, local, gm_smem, tm); else gemm_tile<S, 0, 0, TMAP>(T, local, gm_smem, tm);
     }
 }
 
@@ -86,38 +71,24 @@ __global__ void __launch_bounds__(GemmSmall::THREADS, 4) gemm_small_kernel(const
     extern __shared__ __align__(16) double gm_smem[];
     gm_dispatch<GemmSmall, false>(tasks, n_tasks, gm_smem);
 }
-// Operand tiles through the bulk-copy (TMA) engine + mbarrier: MEASURED SLOWER than the per-thread cp.async ring and therefore an
-// opt-in (DQGP_GEMM_BULK=1, A/B runs): dqgp_dgemm 8192^3 30.0 against 32.9 TFLOP/s, one config-4 factorisation 21.98 against
-// 20.39 ms (round 2, same box, back to back).  This kernel keeps the DMMA pipe 90.6% busy (profiles/r02_gemm_8192.txt: stalls are
-// math-pipe throttle 48%, wait 21%, barrier 8%; issue slots 18% used), so the copy instructions it saves were never the limit, while
-// 192 copies of 128 B per 16-deep k-chunk (the padded, bank-conflict-free fragment layout rules out one tensor-map box per tile: a
-// TMA swizzle leaves the 8-byte m8n8k4 fragments 2-way conflicted) and 256 threads polling the stage's mbarrier cost pipe time.
-// The fused gradient and the fidelity kernel, which had slack (71% / 62% of the pipe), gain 7-16% / 3% from the same change.
-__global__ void __launch_bounds__(GemmBig::THREADS, 2) gemm_group_bulk_kernel(const GemmTask* __restrict__ tasks, int n_tasks) {
-    extern __shared__ __align__(16) double gm_smem[];
-    gm_dispatch<GemmBig, true>(tasks, n_tasks, gm_smem);
-}
-__global__ void __launch_bounds__(GemmSmall::THREADS, 4) gemm_small_bulk_kernel(const GemmTask* __restrict__ tasks, int n_tasks) {
-    extern __shared__ __align__(16) double gm_smem[];
-    gm_dispatch<GemmSmall, true>(tasks, n_tasks, gm_smem);
-}
 // Operand tiles as TWO tensor-map boxes per k-chunk (TMA proper, SASS UTMALDG.2D), issued by one thread: the box is as wide as the padded
 // shared-memory pitch (20 for k-contiguous operands: the 4 doubles beyond the chunk are the next chunk's, never read; BM + 4 / BN + 4
-// otherwise), so the fragment layout stays bank-conflict-free without a swizzle.  The DEFAULT for every registered task table
-// (DQGP_GEMM_NO_TMAP=1 restores the cp.async ring): same box, one issuing thread instead of 768 LDGSTS per chunk - measured on one
-// B200, alternating runs: lauum 5.73 -> 5.31 ms (32.0 -> 34.5 TF = 0.93 of the FP64 peak), triangular inverse 6.15 -> 5.80 ms, potrf
+// otherwise), so the fragment layout stays bank-conflict-free without a swizzle.  Used for every registered task table whose maps the
+// driver accepted: same box, one issuing thread instead of 768 LDGSTS per chunk - measured on one B200 against the cp.async ring,
+// alternating runs: lauum 5.73 -> 5.31 ms (32.0 -> 34.5 TF = 0.93 of the FP64 peak), triangular inverse 6.15 -> 5.80 ms, potrf
 // 8.13 -> 7.79 ms, a lone n = 8192 factorisation 20.02 -> 18.89 ms, the N = 1 iteration of config 4 227.9 -> 219.2 ms; bit-identical
-// results.  (The per-row bulk copies above lost; what they lacked was the single issuing thread.)
+// results.  (A round-2 variant with one cp.async.bulk per tile row lost to the cp.async ring - dqgp_dgemm 8192^3 30.0 against
+// 32.9 TFLOP/s, 192 copies and 256 threads polling an mbarrier per chunk - and was removed; what it lacked was the single issuing thread.)
 __global__ void __launch_bounds__(GemmBig::THREADS, 2) gemm_group_tmap_kernel(const GemmTask* __restrict__ tasks, int n_tasks,
                                                                               const CUtensorMap* __restrict__ maps) {
     extern __shared__ __align__(128) double gm_smem_t[];
-    gm_dispatch<GemmBig, true, true>(tasks, n_tasks, gm_smem_t, maps);
+    gm_dispatch<GemmBig, true>(tasks, n_tasks, gm_smem_t, maps);
 }
 
-template <typename S, int AK, int BK, bool BULK, bool TMAP>
+template <typename S, int AK, int BK, bool TMAP>
 __device__ __forceinline__ void gemm_tile(const GemmTask& T, int local, double* gm_smem, const CUtensorMap* tmaps) {
     __shared__ __align__(8) unsigned long long gm_bar[GM_STAGES];
-    if (BULK) {
+    if (TMAP) {
         if (threadIdx.x == 0) {
 #pragma unroll
             for (int s = 0; s < GM_STAGES; ++s) mbar_init(&gm_bar[s], 1);
@@ -172,9 +143,6 @@ __device__ __forceinline__ void gemm_tile(const GemmTask& T, int local, double* 
     auto stage_a = [&](int s) { return gm_smem + (size_t)s * GM_STAGE_DOUBLES; };
     auto stage_b = [&](int s) { return gm_smem + (size_t)s * GM_STAGE_DOUBLES + GM_A_DOUBLES; };
 
-    constexpr unsigned STAGE_BYTES = (GM_BM + GM_BN) * GM_KC * sizeof(double);
-    constexpr int B_T0 = AK ? GM_BM : GM_KC;          // first thread that copies the B operand (after the A operand's copies)
-    static_assert(GM_BM + GM_BN <= S::THREADS, "one bulk copy per thread");
     constexpr unsigned TM_BYTES = ((AK ? GM_BM * GM_PITCH_K : GM_KC * GM_PITCH_M) + (BK ? GM_BN * GM_PITCH_K : GM_KC * GM_PITCH_N)) * sizeof(double);
     auto fill = [&](int s, int c) {
         if (TMAP) {
@@ -184,10 +152,6 @@ __device__ __forceinline__ void gemm_tile(const GemmTask& T, int local, double* 
                 if (AK) tensor_copy_2d_g2s(stage_a(s), tmaps, k, m0, &gm_bar[s]); else tensor_copy_2d_g2s(stage_a(s), tmaps, m0, k, &gm_bar[s]);
                 if (BK) tensor_copy_2d_g2s(stage_b(s), tmaps + 1, k, n0, &gm_bar[s]); else tensor_copy_2d_g2s(stage_b(s), tmaps + 1, n0, k, &gm_bar[s]);
             }
-        } else if (BULK) {
-            if (threadIdx.x == 0) mbar_arrive_expect_tx(&gm_bar[s], STAGE_BYTES);
-            gm_load_operand_bulk<GM_BM, GM_PITCH_M>(stage_a(s), T.A, T.lda, m0, kb + c * GM_KC, AK, 0, &gm_bar[s]);
-            gm_load_operand_bulk<GM_BN, GM_PITCH_N>(stage_b(s), T.B, T.ldb, n0, kb + c * GM_KC, BK, B_T0, &gm_bar[s]);
         } else {
             gm_load_operand<GM_BM, GM_PITCH_M, S::THREADS>(stage_a(s), T.A, T.lda, m0, kb + c * GM_KC, AK);
             gm_load_operand<GM_BN, GM_PITCH_N, S::THREADS>(stage_b(s), T.B, T.ldb, n0, kb + c * GM_KC, BK);
@@ -196,16 +160,16 @@ __device__ __forceinline__ void gemm_tile(const GemmTask& T, int local, double* 
 #pragma unroll
     for (int s = 0; s < GM_STAGES - 1; ++s) {
         if (s < n_chunks) fill(s, s);
-        if (!BULK) cp_async_commit();
+        if (!TMAP) cp_async_commit();
     }
     for (int ch = 0; ch < n_chunks; ++ch) {
-        if (BULK) mbar_wait(&gm_bar[ch % GM_STAGES], (ch / GM_STAGES) & 1);
+        if (TMAP) mbar_wait(&gm_bar[ch % GM_STAGES], (ch / GM_STAGES) & 1);
         else cp_async_wait<GM_STAGES - 2>();
         __syncthreads();
         {
             const int nx = ch + GM_STAGES - 1;
             if (nx < n_chunks) fill(nx % GM_STAGES, nx);
-            if (!BULK) cp_async_commit();
+            if (!TMAP) cp_async_commit();
         }
         const double* As = stage_a(ch % GM_STAGES);
         const double* Bs = stage_b(ch % GM_STAGES);
@@ -232,7 +196,7 @@ __device__ __forceinline__ void gemm_tile(const GemmTask& T, int local, double* 
                 for (int j = 0; j < NI; ++j) dmma884(acc[i][j][0], acc[i][j][1], a[i], b[j]);
         }
     }
-    if (!BULK) cp_async_wait<0>();
+    if (!TMAP) cp_async_wait<0>();
 
     // epilogue: each lane owns 2 adjacent doubles per 8x8 block -> 16-byte accesses
 #pragma unroll
@@ -260,8 +224,6 @@ int gemm_init() {
     if (dev >= 0 && dev < 64 && done[dev]) return 0;
     DQGP_CUDA(cudaFuncSetAttribute(gemm_group_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GemmBig::SMEM_BYTES));
     DQGP_CUDA(cudaFuncSetAttribute(gemm_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GemmSmall::SMEM_BYTES));
-    DQGP_CUDA(cudaFuncSetAttribute(gemm_group_bulk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GemmBig::SMEM_BYTES));
-    DQGP_CUDA(cudaFuncSetAttribute(gemm_small_bulk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GemmSmall::SMEM_BYTES));
     DQGP_CUDA(cudaFuncSetAttribute(gemm_group_tmap_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GemmBig::SMEM_BYTES + 128));
     if (dev >= 0 && dev < 64) done[dev] = true;
     return 0;
@@ -270,10 +232,9 @@ int gemm_init() {
 // ---- tensor maps: registered task tables -> device arrays of (A map, B map) per task -----------------------------------------
 struct GemmMapTable { const GemmTask* d_tasks; int n; CUtensorMap* d_maps; };
 static std::vector<GemmMapTable>& gemm_map_tables() { static std::vector<GemmMapTable> t; return t; }
-static bool gemm_use_tmap() { static const bool on = getenv("DQGP_GEMM_NO_TMAP") == nullptr; return on; }
 
 void gemm_register_maps(const GemmTask* d_tasks, const GemmTask* h_tasks, int n_tasks) {
-    if (!gemm_use_tmap() || n_tasks <= 0) return;
+    if (n_tasks <= 0) return;
     std::vector<CUtensorMap> maps(2 * (size_t)n_tasks);
     memset(maps.data(), 0, sizeof(CUtensorMap) * maps.size());
     for (int i = 0; i < n_tasks; ++i) {
@@ -301,17 +262,13 @@ int launch_gemm_group(const GemmTask* d_tasks, int n_tasks, int total_tiles, cud
     if (n_tasks <= 0 || total_tiles <= 0) return 0;
     int rc = gemm_init();
     if (rc) return rc;
-    if (gemm_use_tmap()) {
-        for (const GemmMapTable& tab : gemm_map_tables())
-            if (d_tasks >= tab.d_tasks && d_tasks + n_tasks <= tab.d_tasks + tab.n) {
-                gemm_group_tmap_kernel<<<total_tiles, GemmBig::THREADS, GemmBig::SMEM_BYTES + 128, st>>>(d_tasks, n_tasks, tab.d_maps + 2 * (d_tasks - tab.d_tasks));
-                DQGP_LAUNCH_CHECK("gemm_group_tmap_kernel");
-                return 0;
-            }
-    }
-    static const bool use_bulk = getenv("DQGP_GEMM_BULK") != nullptr;
-    if (use_bulk) gemm_group_bulk_kernel<<<total_tiles, GemmBig::THREADS, GemmBig::SMEM_BYTES, st>>>(d_tasks, n_tasks);
-    else gemm_group_kernel<<<total_tiles, GemmBig::THREADS, GemmBig::SMEM_BYTES, st>>>(d_tasks, n_tasks);
+    for (const GemmMapTable& tab : gemm_map_tables())
+        if (d_tasks >= tab.d_tasks && d_tasks + n_tasks <= tab.d_tasks + tab.n) {
+            gemm_group_tmap_kernel<<<total_tiles, GemmBig::THREADS, GemmBig::SMEM_BYTES + 128, st>>>(d_tasks, n_tasks, tab.d_maps + 2 * (d_tasks - tab.d_tasks));
+            DQGP_LAUNCH_CHECK("gemm_group_tmap_kernel");
+            return 0;
+        }
+    gemm_group_kernel<<<total_tiles, GemmBig::THREADS, GemmBig::SMEM_BYTES, st>>>(d_tasks, n_tasks);
     DQGP_LAUNCH_CHECK("gemm_group_kernel");
     return 0;
 }
@@ -320,9 +277,7 @@ int launch_gemm_group_small(const GemmTask* d_tasks, int n_tasks, int total_tile
     if (n_tasks <= 0 || total_tiles <= 0) return 0;
     int rc = gemm_init();
     if (rc) return rc;
-    static const bool use_bulk = getenv("DQGP_GEMM_BULK") != nullptr;
-    if (use_bulk) gemm_small_bulk_kernel<<<total_tiles, GemmSmall::THREADS, GemmSmall::SMEM_BYTES, st>>>(d_tasks, n_tasks);
-    else gemm_small_kernel<<<total_tiles, GemmSmall::THREADS, GemmSmall::SMEM_BYTES, st>>>(d_tasks, n_tasks);
+    gemm_small_kernel<<<total_tiles, GemmSmall::THREADS, GemmSmall::SMEM_BYTES, st>>>(d_tasks, n_tasks);
     DQGP_LAUNCH_CHECK("gemm_small_kernel");
     return 0;
 }

@@ -52,9 +52,8 @@ int launch_gemm_group(const GemmTask* d_tasks, int n_tasks, int total_tiles, cud
 // same table format with tile_begin / tiles counted in 32x32 tiles (gemm_task_tiles_small); GM_KRULE_ALL only
 int launch_gemm_group_small(const GemmTask* d_tasks, int n_tasks, int total_tiles, cudaStream_t st);
 int gemm_init();   // raises the dynamic shared memory limit once per process/device
-// Operand tiles as two tensor-map boxes per k-chunk (the default; DQGP_GEMM_NO_TMAP=1 = per-thread cp.async ring).  A task table
-// registers its host copy once; launches whose device pointer lies inside a registered table use the tensor-map kernel, others (and
-// tables whose maps the driver refused) the cp.async kernel.
+// Operand tiles as two tensor-map boxes per k-chunk.  A task table registers its host copy once; launches whose device pointer lies
+// inside a registered table use the tensor-map kernel, others (and tables whose maps the driver refused) the per-thread cp.async ring.
 void gemm_register_maps(const GemmTask* d_tasks, const GemmTask* h_tasks, int n_tasks);
 void gemm_unregister_maps(const GemmTask* d_tasks);
 

@@ -7,7 +7,6 @@
 // kernel and contracting on the fly.  Partial sums go to partial[tile][i]; a second kernel adds them in a
 // fixed order, so the result is bit-reproducible run to run (the reference rounds it to 4 decimals).
 // Bound: FP64 pipe (3m + outer-kernel flops per entry, SURVEY §8(d)); HBM traffic is one read of A^-1.
-#include <cstdlib>
 #include <cstring>
 #include "pairwise.cuh"
 #include "tensormap.cuh"
@@ -21,69 +20,6 @@ __device__ __forceinline__ void tile_from_index(int local, int& bi, int& bj) {
     bj = local - bi * (bi + 1) / 2;
 }
 
-__device__ __forceinline__ void load_bracket(const double* __restrict__ Ainv, int ld, const double* __restrict__ alpha, int n,
-                                             int row0, int col0, int ty, int tx, double weight, double (&b)[4][4]) {
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int r = row0 + ty + 16 * i;
-        const double ar = (r < n) ? alpha[r] : 0.0;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const int c = col0 + 2 * tx + 32 * (j >> 1) + (j & 1);
-            b[i][j] = (r < n && c < n) ? weight * (Ainv[(size_t)r * ld + c] - ar * alpha[c]) : 0.0;
-        }
-    }
-}
-
-__device__ __forceinline__ void block_commit(double acc, double* s_red, double* dst) {
-    acc = warp_sum(acc);
-    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = acc;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double t = 0.0;
-#pragma unroll
-        for (int w = 0; w < PW_THREADS / 32; ++w) t += s_red[w];
-        *dst = t;
-    }
-}
-
-template <int OUTER>
-__global__ void __launch_bounds__(PW_THREADS) grad_projected_kernel(const double* __restrict__ Ainv, int ld,
-                                                                    const double* __restrict__ alpha,
-                                                                    const double* __restrict__ F, int n, int m, int P,
-                                                                    OuterHyp hyp, double* __restrict__ partial) {
-    __shared__ __align__(16) double FrT[PW_MAX_M * PW_PITCH];
-    __shared__ __align__(16) double FcT[PW_MAX_M * PW_PITCH];
-    __shared__ double s_red[PW_THREADS / 32];
-    int bi, bj;
-    tile_from_index(blockIdx.x, bi, bj);
-    const int row0 = bi * PW_TILE, col0 = bj * PW_TILE;
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    double b[4][4];
-    load_bracket(Ainv, ld, alpha, n, row0, col0, ty, tx, bi == bj ? 1.0 : 2.0, b);
-    const size_t set_stride = (size_t)n * m;
-    for (int i = 0; i < P; ++i) {
-        double acc = 0.0;
-#pragma unroll 1
-        for (int sg = 0; sg < 2; ++sg) {
-            const double* Fs = F + (size_t)(1 + 2 * i + sg) * set_stride;
-            __syncthreads();
-            stage_features_T(FrT, Fs, row0, n, m);
-            stage_features_T(FcT, Fs, col0, n, m);
-            __syncthreads();
-            double d2[4][4];
-            micro_sqdist(FrT, FcT, m, ty, tx, d2);
-            double part = 0.0;
-#pragma unroll
-            for (int r = 0; r < 4; ++r)
-#pragma unroll
-                for (int c = 0; c < 4; ++c) part = fma(b[r][c], outer_eval<OUTER>(d2[r][c], hyp), part);
-            acc += sg ? -part : part;
-        }
-        block_commit(acc, s_red, partial + (size_t)blockIdx.x * P + i);
-    }
-}
-
 // ---- v2: Gram-identity formulation on the DMMA pipe ---------------------------------------------------------------
 // -gamma*||f-g||^2 = 2*gamma*f.g - gamma*||f||^2 - gamma*||g||^2: the accumulator of an 8x8 DMMA block is
 // initialised with the (pre-scaled) norms, the row operand is scaled by 2*gamma at fragment load, and m/4
@@ -91,101 +27,75 @@ __global__ void __launch_bounds__(PW_THREADS) grad_projected_kernel(const double
 // is 1 DADD + m MACs + 16 (exp) + 1 DFMA (contraction with B) on the FP64 pipe instead of 2m + 23 + 1 for the
 // direct-difference form (the absolute error of d^2 is ~1e-15, harmless for exp/Matern/ExpSine outer kernels;
 // the unshifted Gram that is *written* keeps direct differences).  CTA = 64x64 tile, 8 warps as 4x2, warp tile
-// 16x32 = 2x4 DMMA blocks; B stays in registers for all 2P sets; feature tiles double-buffered with cp.async.
+// 16x32 = 2x4 DMMA blocks; B stays in registers for all 2P sets; feature tiles double-buffered.
+constexpr int G2_STAGES = 2;
 constexpr int G2_STAGE_DOUBLES = 2 * PW_TILE * G2_PITCH + 2 * PW_TILE;
-constexpr size_t G2_SMEM = sizeof(double) * 2 * G2_STAGE_DOUBLES;
-constexpr size_t G2_SMEM_P28 = sizeof(double) * 3 * (2 * PW_TILE * 28 + 2 * PW_TILE);      // PITCH = 28, three stages
+constexpr size_t G2_SMEM = sizeof(double) * G2_STAGES * G2_STAGE_DOUBLES;
+static_assert(PW_MAX_M <= G2_PITCH, "a staged sample row holds every feature");
 
 __device__ __forceinline__ void cp_async8(void* smem, const void* gmem) {
     unsigned sa = static_cast<unsigned>(__cvta_generic_to_shared(smem));
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(sa), "l"(gmem));
 }
 
-// Stage one parameter set's row and column feature tiles (64 x m each) + their squared norms.  Four threads per
-// sample row, no integer division: thread (row = tid>>2, lane4 = tid&3) copies chunks lane4, lane4+4, ... of its row.
-// VEC=2: m even -> 16-byte cp.async (row starts are 16-byte aligned); VEC=1: 8-byte copies.
-template <int VEC, int PITCH>
-__device__ __forceinline__ void g2_stage(double* buf, const double* __restrict__ Fs, const double* __restrict__ Ns, int row0,
-                                         int col0, int n, int m) {
+__device__ __forceinline__ void g2_stage_norms(double* nr, const double* __restrict__ Ns, int row0, int col0, int n) {
+    if (threadIdx.x < PW_TILE) cp_async8(&nr[threadIdx.x], &Ns[min(row0 + threadIdx.x, n - 1)]);
+    else if (threadIdx.x < 2 * PW_TILE) cp_async8(&nr[threadIdx.x], &Ns[min(col0 + threadIdx.x - PW_TILE, n - 1)]);
+}
+
+// Stage one parameter set's row and column feature tiles (64 x m each) + their squared norms with per-thread 8-byte cp.async: four
+// threads per sample row, thread (row = tid>>2, lane4 = tid&3) copies features lane4, lane4+4, ... of its row.  Any m, any alignment.
+__device__ __forceinline__ void g2_stage(double* buf, const double* __restrict__ Fs, const double* __restrict__ Ns, int row0, int col0,
+                                         int n, int m) {
     const int r = threadIdx.x >> 2, l4 = threadIdx.x & 3;
     const double* src_r = Fs + (size_t)min(row0 + r, n - 1) * m;
     const double* src_c = Fs + (size_t)min(col0 + r, n - 1) * m;
-    double* dst_r = buf + r * PITCH;
-    double* dst_c = buf + PW_TILE * PITCH + r * PITCH;
-    if (VEC == 2) {
-        for (int k = 2 * l4; k < m; k += 8) {
-            cp_async16(dst_r + k, src_r + k);
-            cp_async16(dst_c + k, src_c + k);
-        }
-    } else {
-        for (int k = l4; k < m; k += 4) {
-            cp_async8(dst_r + k, src_r + k);
-            cp_async8(dst_c + k, src_c + k);
-        }
+    double* dst_r = buf + r * G2_PITCH;
+    double* dst_c = buf + PW_TILE * G2_PITCH + r * G2_PITCH;
+    for (int k = l4; k < m; k += 4) {
+        cp_async8(dst_r + k, src_r + k);
+        cp_async8(dst_c + k, src_c + k);
     }
-    double* nr = buf + 2 * PW_TILE * PITCH;
-    if (threadIdx.x < PW_TILE) cp_async8(&nr[threadIdx.x], &Ns[min(row0 + threadIdx.x, n - 1)]);
-    else if (threadIdx.x < 2 * PW_TILE) cp_async8(&nr[threadIdx.x], &Ns[min(col0 + threadIdx.x - PW_TILE, n - 1)]);
-}
-
-// Same tile through the bulk-copy engine (cp.async.bulk = TMA without a tensor map, SASS UBLKCP): one copy per sample row (m doubles,
-// a multiple of 16 bytes when m is even) straight into the padded row of the fragment layout, completion counted in bytes on the
-// stage's mbarrier.  The norms (8-byte granularity, not always 16-byte aligned) stay on cp.async.
-template <int PITCH>
-__device__ __forceinline__ void g2_stage_bulk(double* buf, const double* __restrict__ Fs, const double* __restrict__ Ns, int row0, int col0, int n,
-                                              int m, unsigned long long* bar) {
-    if (threadIdx.x == 0) mbar_arrive_expect_tx(bar, 2u * PW_TILE * m * sizeof(double));
-    if (threadIdx.x < 2 * PW_TILE) {
-        const int r = threadIdx.x & (PW_TILE - 1), is_col = threadIdx.x >> 6;
-        const double* src = Fs + (size_t)min((is_col ? col0 : row0) + r, n - 1) * m;
-        bulk_copy_g2s(buf + (is_col * PW_TILE + r) * PITCH, src, m * sizeof(double), bar);
-    }
-    double* nr = buf + 2 * PW_TILE * PITCH;
-    if (threadIdx.x < PW_TILE) cp_async8(&nr[threadIdx.x], &Ns[min(row0 + threadIdx.x, n - 1)]);
-    else if (threadIdx.x < 2 * PW_TILE) cp_async8(&nr[threadIdx.x], &Ns[min(col0 + threadIdx.x - PW_TILE, n - 1)]);
+    g2_stage_norms(buf + 2 * PW_TILE * G2_PITCH, Ns, row0, col0, n);
 }
 
 // Same tile as TWO boxes of a 3-D tensor map over F = [set][sample][feature] (TMA proper, SASS UTMALDG), issued by one thread: box =
-// 64 samples x PITCH features, so the features beyond m - outside the tensor - arrive as the zero padding of the fragment layout, and
-// samples beyond n as zero rows (their bracket weights are zero).  Replaces 128 per-row copies per parameter set.
-template <int PITCH>
+// 64 samples x G2_PITCH features, so the features beyond m - outside the tensor - arrive as the zero padding of the fragment layout,
+// and samples beyond n as zero rows (their bracket weights are zero).
 __device__ __forceinline__ void g2_stage_tmap(double* buf, const void* tmap, int set, const double* __restrict__ Ns, int row0, int col0, int n,
                                               unsigned long long* bar) {
     if (threadIdx.x == 0) {
-        mbar_arrive_expect_tx(bar, 2u * PW_TILE * PITCH * sizeof(double));
+        mbar_arrive_expect_tx(bar, 2u * PW_TILE * G2_PITCH * sizeof(double));
         tensor_copy_3d_g2s(buf, tmap, 0, row0, set, bar);
-        tensor_copy_3d_g2s(buf + PW_TILE * PITCH, tmap, 0, col0, set, bar);
+        tensor_copy_3d_g2s(buf + PW_TILE * G2_PITCH, tmap, 0, col0, set, bar);
     }
-    double* nr = buf + 2 * PW_TILE * PITCH;
-    if (threadIdx.x < PW_TILE) cp_async8(&nr[threadIdx.x], &Ns[min(row0 + threadIdx.x, n - 1)]);
-    else if (threadIdx.x < 2 * PW_TILE) cp_async8(&nr[threadIdx.x], &Ns[min(col0 + threadIdx.x - PW_TILE, n - 1)]);
+    g2_stage_norms(buf + 2 * PW_TILE * G2_PITCH, Ns, row0, col0, n);
 }
 
 // CLAMP: guard the exponent against arguments below -700 (only reachable when gamma * 4m > 700; features lie in [-1, 1])
-// BULK: stage the feature tiles with cp.async.bulk + mbarrier instead of per-thread cp.async (needs VEC == 2)
-// PITCH: doubles per staged sample row, = 4 (mod 8) so the DMMA fragment loads are bank-conflict-free, >= m.  With PITCH = 28 (m <= 28:
-// up to 9 qubits) a stage is 29.7 KB and THREE stages fit beside a second CTA, so a tile's copy is issued two sets ahead.
-// TMAP: the feature tiles of a parameter set arrive as two boxes of the tensor map `tmap` (needs BULK's mbarriers)
-template <int OUTER, int VEC, bool CLAMP = true, bool BULK = false, int PITCH = G2_PITCH, bool TMAP = false>
+// TMAP: the feature tiles of a parameter set arrive as two boxes of the tensor map `tmap`, completion counted on an mbarrier per stage;
+// otherwise per-thread cp.async (g2_stage)
+// G2_PITCH: doubles per staged sample row, = 4 (mod 8) so the DMMA fragment loads are bank-conflict-free, >= m.  (Pitch 28 with three
+// stages, the copy issued two sets ahead, measured 1% slower at config 4: 8.74 against 8.63 ms; the copy is hidden one set ahead.)
+template <int OUTER, bool CLAMP, bool TMAP>
 __global__ void __launch_bounds__(PW_THREADS, 2) grad_projected_dmma_kernel(const double* __restrict__ Ainv, int ld,
                                                                            const double* __restrict__ alpha,
                                                                            const double* __restrict__ F,
                                                                            const double* __restrict__ Nrm, int n, int m, int P,
                                                                            OuterHyp hyp, double* __restrict__ partial,
                                                                            const __grid_constant__ CUtensorMap tmap) {
-    constexpr int STAGES = (BULK && PITCH <= 28) ? 3 : 2;
-    constexpr int G2_STAGE_DOUBLES = 2 * PW_TILE * PITCH + 2 * PW_TILE;
+    constexpr int STAGES = G2_STAGES, PITCH = G2_PITCH;
     extern __shared__ __align__(128) double g2_smem[];
     __shared__ double s_red[2][PW_THREADS / 32];
-    __shared__ __align__(8) unsigned long long s_bar[3];
+    __shared__ __align__(8) unsigned long long s_bar[STAGES];
     int bi, bj;
     tile_from_index(blockIdx.x, bi, bj);
     const int row0 = bi * PW_TILE, col0 = bj * PW_TILE;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int wr = warp >> 1, wc = warp & 1, g = lane >> 2, t = lane & 3;
     const int ksteps = (m + 3) >> 2;
-    if (BULK) {
-        if (threadIdx.x == 0) { mbar_init(&s_bar[0], 1); mbar_init(&s_bar[1], 1); mbar_init(&s_bar[2], 1); mbar_fence_init(); }
+    if (TMAP) {
+        if (threadIdx.x == 0) { mbar_init(&s_bar[0], 1); mbar_init(&s_bar[1], 1); mbar_fence_init(); }
         __syncthreads();
     }
     const double gam = (OUTER == DQGP_OUTER_GAUSSIAN) ? hyp.a * DQGP_EXP_S32 : 1.0;      // Gaussian: argument in units of ln2/32
@@ -218,19 +128,14 @@ __global__ void __launch_bounds__(PW_THREADS, 2) grad_projected_dmma_kernel(cons
 
     const size_t set_stride = (size_t)n * m;
     const int T = 2 * P;
-    if (TMAP) g2_stage_tmap<PITCH>(g2_smem, &tmap, 1, Nrm + n, row0, col0, n, &s_bar[0]);
-    else if (BULK) g2_stage_bulk<PITCH>(g2_smem, F + set_stride, Nrm + n, row0, col0, n, m, &s_bar[0]);
-    else g2_stage<VEC, PITCH>(g2_smem, F + set_stride, Nrm + n, row0, col0, n, m);
+    if (TMAP) g2_stage_tmap(g2_smem, &tmap, 1, Nrm + n, row0, col0, n, &s_bar[0]);
+    else g2_stage(g2_smem, F + set_stride, Nrm + n, row0, col0, n, m);
     cp_async_commit();
-    if (STAGES == 3) {
-        if (T > 1) g2_stage_bulk<PITCH>(g2_smem + G2_STAGE_DOUBLES, F + 2 * set_stride, Nrm + 2 * (size_t)n, row0, col0, n, m, &s_bar[1]);
-        cp_async_commit();
-    }
     double pplus = 0.0, pminus = 0.0;
     for (int tt = 0; tt < T; ++tt) {
         const int cur = tt % STAGES;
-        if (STAGES == 3) cp_async_wait<1>(); else cp_async_wait<0>();
-        if (BULK) mbar_wait(&s_bar[cur], (tt / STAGES) & 1);
+        cp_async_wait<0>();
+        if (TMAP) mbar_wait(&s_bar[cur], (tt / STAGES) & 1);
         __syncthreads();
         if (tt >= 2 && (tt & 1) == 0 && threadIdx.x == 0) {
             const int i = (tt >> 1) - 1;
@@ -243,9 +148,8 @@ __global__ void __launch_bounds__(PW_THREADS, 2) grad_projected_dmma_kernel(cons
             const int nx = tt + STAGES - 1;          // the set whose copy is issued now; its stage was last read at iteration tt - 1
             if (nx < T) {
                 const int ns = nx % STAGES;
-                if (TMAP) g2_stage_tmap<PITCH>(g2_smem + ns * G2_STAGE_DOUBLES, &tmap, nx + 1, Nrm + (size_t)(nx + 1) * n, row0, col0, n, &s_bar[ns]);
-                else if (BULK) g2_stage_bulk<PITCH>(g2_smem + ns * G2_STAGE_DOUBLES, F + (size_t)(nx + 1) * set_stride, Nrm + (size_t)(nx + 1) * n, row0, col0, n, m, &s_bar[ns]);
-                else g2_stage<VEC, PITCH>(g2_smem + ns * G2_STAGE_DOUBLES, F + (size_t)(nx + 1) * set_stride, Nrm + (size_t)(nx + 1) * n, row0, col0, n, m);
+                if (TMAP) g2_stage_tmap(g2_smem + ns * G2_STAGE_DOUBLES, &tmap, nx + 1, Nrm + (size_t)(nx + 1) * n, row0, col0, n, &s_bar[ns]);
+                else g2_stage(g2_smem + ns * G2_STAGE_DOUBLES, F + (size_t)(nx + 1) * set_stride, Nrm + (size_t)(nx + 1) * n, row0, col0, n, m);
             }
         }
         cp_async_commit();
@@ -312,75 +216,6 @@ __global__ void feature_norms_kernel(const double* __restrict__ F, long long row
     double acc = 0.0;
     for (int k = 0; k < m; ++k) acc = fma(f[k], f[k], acc);
     Nrm[row] = scale * acc;
-}
-
-constexpr int FID_KC_G = 16;
-constexpr int FID_PITCH_G = 65;
-
-__global__ void __launch_bounds__(PW_THREADS) grad_fidelity_kernel(const double* __restrict__ Ainv, int ld,
-                                                                   const double* __restrict__ alpha,
-                                                                   const double2* __restrict__ Psi, int n, int dim, int P,
-                                                                   double* __restrict__ partial) {
-    __shared__ __align__(16) double2 ArT[FID_KC_G * FID_PITCH_G];
-    __shared__ __align__(16) double2 AcT[FID_KC_G * FID_PITCH_G];
-    __shared__ double s_red[PW_THREADS / 32];
-    int bi, bj;
-    tile_from_index(blockIdx.x, bi, bj);
-    const int row0 = bi * PW_TILE, col0 = bj * PW_TILE;
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    double b[4][4];
-    load_bracket(Ainv, ld, alpha, n, row0, col0, ty, tx, bi == bj ? 1.0 : 2.0, b);
-    const size_t set_stride = (size_t)n * dim;
-    const int vr = min(PW_TILE, n - row0), vc = min(PW_TILE, n - col0);
-    for (int i = 0; i < P; ++i) {
-        double acc = 0.0;
-#pragma unroll 1
-        for (int sg = 0; sg < 2; ++sg) {
-            const double2* Ps = Psi + (size_t)(1 + 2 * i + sg) * set_stride;
-            double re[4][4], im[4][4];
-#pragma unroll
-            for (int r = 0; r < 4; ++r)
-#pragma unroll
-                for (int c = 0; c < 4; ++c) re[r][c] = im[r][c] = 0.0;
-            for (int k0 = 0; k0 < dim; k0 += FID_KC_G) {
-                __syncthreads();
-                for (int e = threadIdx.x; e < PW_TILE * FID_KC_G; e += PW_THREADS) {
-                    const int r = e / FID_KC_G, kk = e % FID_KC_G;
-                    const bool kin = (k0 + kk) < dim;
-                    ArT[kk * FID_PITCH_G + r] = (r < vr && kin) ? Ps[(size_t)(row0 + r) * dim + k0 + kk] : make_double2(0.0, 0.0);
-                    AcT[kk * FID_PITCH_G + r] = (r < vc && kin) ? Ps[(size_t)(col0 + r) * dim + k0 + kk] : make_double2(0.0, 0.0);
-                }
-                __syncthreads();
-#pragma unroll 4
-                for (int kk = 0; kk < FID_KC_G; ++kk) {
-                    double2 a[4], bb[4];
-#pragma unroll
-                    for (int r = 0; r < 4; ++r) a[r] = ArT[kk * FID_PITCH_G + ty + 16 * r];
-#pragma unroll
-                    for (int jj = 0; jj < 2; ++jj) {
-                        bb[2 * jj] = AcT[kk * FID_PITCH_G + 2 * tx + 32 * jj];
-                        bb[2 * jj + 1] = AcT[kk * FID_PITCH_G + 2 * tx + 32 * jj + 1];
-                    }
-#pragma unroll
-                    for (int r = 0; r < 4; ++r)
-#pragma unroll
-                        for (int c = 0; c < 4; ++c) {
-                            re[r][c] = fma(a[r].x, bb[c].x, re[r][c]);
-                            re[r][c] = fma(a[r].y, bb[c].y, re[r][c]);
-                            im[r][c] = fma(a[r].y, bb[c].x, im[r][c]);
-                            im[r][c] = fma(-a[r].x, bb[c].y, im[r][c]);
-                        }
-                }
-            }
-            double part = 0.0;
-#pragma unroll
-            for (int r = 0; r < 4; ++r)
-#pragma unroll
-                for (int c = 0; c < 4; ++c) part = fma(b[r][c], re[r][c] * re[r][c] + im[r][c] * im[r][c], part);
-            acc += sg ? -part : part;
-        }
-        block_commit(acc, s_red, partial + (size_t)blockIdx.x * P + i);
-    }
 }
 
 // grad[i] = scale * sum_tiles partial[tile][i], fixed summation order (strided per thread, then a fixed tree)
@@ -550,35 +385,23 @@ int dqgp_grad_projected(int outer, const double* h_hyp, const double* d_Ainv, in
     cudaStream_t st = as_stream(stream);
     double* partial = static_cast<double*>(d_work);
     double* norms = partial + (size_t)tiles * P;
-    static const bool use_direct = getenv("DQGP_GRAD_DIRECT") != nullptr;   // v1 direct-difference kernel, kept for A/B checks
-    if (use_direct) {
-        switch (outer) {
-            case DQGP_OUTER_GAUSSIAN: grad_projected_kernel<DQGP_OUTER_GAUSSIAN><<<tiles, PW_THREADS, 0, st>>>(d_Ainv, ld, d_alpha, d_F, n, m, P, hyp, partial); break;
-            case DQGP_OUTER_MATERN15: grad_projected_kernel<DQGP_OUTER_MATERN15><<<tiles, PW_THREADS, 0, st>>>(d_Ainv, ld, d_alpha, d_F, n, m, P, hyp, partial); break;
-            default: grad_projected_kernel<DQGP_OUTER_EXPSINE2><<<tiles, PW_THREADS, 0, st>>>(d_Ainv, ld, d_alpha, d_F, n, m, P, hyp, partial); break;
-        }
-    } else {
-        const long long rows = (long long)(2 * P + 1) * n;
-        // the norms arrive pre-multiplied by -gamma_eff (and, Gaussian, by 32/ln2: the exponent's argument then leaves the DMMA in the
-        // units its range reduction wants): the kernel only adds them
-        const double gam_eff = (outer == DQGP_OUTER_GAUSSIAN) ? hyp.a * DQGP_EXP_S32 : 1.0;
-        feature_norms_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(d_F, rows, m, -gam_eff, norms);
-        // Pauli features lie in [-1, 1]: gamma d^2 <= 4 m gamma, so the exponent guard is only needed for large gamma
-        // the exponent's argument is bounded below by -gamma 4m (Gaussian), -sqrt(3) 2 sqrt(m) / l (Matern), -2 / l^2 (ExpSineSquared)
-        const double worst = outer == DQGP_OUTER_GAUSSIAN ? 4.0 * m * hyp.a
-                             : outer == DQGP_OUTER_MATERN15 ? 1.7320508075688772 * 2.0 * sqrt((double)m) * hyp.a : 2.0 * hyp.a * hyp.a;
-        const bool no_clamp = hyp.a > 0.0 && worst < 650.0;
-        // feature tiles through the bulk-copy (TMA) engine unless DQGP_GRAD_NO_BULK is set (A/B runs against per-thread cp.async)
-        const bool use_bulk = getenv("DQGP_GRAD_NO_BULK") == nullptr;
-        // pitch 28 + three stages (copy issued two sets ahead) measured 1% SLOWER than pitch 36 + two stages at config 4 (8.74 against
-        // 8.63 ms): the copy is already hidden one set ahead; kept as an opt-in for A/B runs
-        const bool use_p28 = getenv("DQGP_GRAD_P28") != nullptr;
-        // ... and as two boxes of a 3-D tensor map per parameter set (one thread issues them) unless DQGP_GRAD_NO_TMAP is set or the
-        // driver refuses the map (then the per-row bulk copies above)
-        CUtensorMap tmap;
-        memset(&tmap, 0, sizeof(tmap));
-        const bool have_tmap = use_bulk && !use_p28 && getenv("DQGP_GRAD_NO_TMAP") == nullptr && (m & 1) == 0 && m <= G2_PITCH &&
-                               (reinterpret_cast<uintptr_t>(d_F) & 15) == 0 && make_rows_tensor_map(&tmap, d_F, m, n, 2 * P + 1, G2_PITCH, PW_TILE);
+    const long long rows = (long long)(2 * P + 1) * n;
+    // the norms arrive pre-multiplied by -gamma_eff (and, Gaussian, by 32/ln2: the exponent's argument then leaves the DMMA in the
+    // units its range reduction wants): the kernel only adds them
+    const double gam_eff = (outer == DQGP_OUTER_GAUSSIAN) ? hyp.a * DQGP_EXP_S32 : 1.0;
+    feature_norms_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(d_F, rows, m, -gam_eff, norms);
+    // Pauli features lie in [-1, 1]: gamma d^2 <= 4 m gamma, so the exponent guard is only needed for large gamma
+    // the exponent's argument is bounded below by -gamma 4m (Gaussian), -sqrt(3) 2 sqrt(m) / l (Matern), -2 / l^2 (ExpSineSquared)
+    const double worst = outer == DQGP_OUTER_GAUSSIAN ? 4.0 * m * hyp.a
+                         : outer == DQGP_OUTER_MATERN15 ? 1.7320508075688772 * 2.0 * sqrt((double)m) * hyp.a : 2.0 * hyp.a * hyp.a;
+    const bool no_clamp = hyp.a > 0.0 && worst < 650.0;
+    // feature tiles as two boxes of a 3-D tensor map per parameter set (one thread issues them); odd m (rows not 16-byte multiples),
+    // a misaligned d_F or a map the driver refuses take the per-thread cp.async kernel, with the exponent guard (CLAMP only changes
+    // results below -700, where no_clamp is never set, so both kernels give the same gradient)
+    CUtensorMap tmap;
+    memset(&tmap, 0, sizeof(tmap));
+    const bool have_tmap = (m & 1) == 0 && (reinterpret_cast<uintptr_t>(d_F) & 15) == 0 &&
+                           make_rows_tensor_map(&tmap, d_F, m, n, 2 * P + 1, G2_PITCH, PW_TILE);
 #define DQGP_G2(OUT)                                                                                                         \
     do {                                                                                                                     \
         static bool attr_done_dev[64] = {false};        /* the attribute is per DEVICE (as gemm_init's flags) */            \
@@ -586,37 +409,22 @@ int dqgp_grad_projected(int outer, const double* h_hyp, const double* d_Ainv, in
         cudaGetDevice(&dev_);                                                                                                \
         bool& attr_done = attr_done_dev[(dev_ >= 0 && dev_ < 64) ? dev_ : 0];                                                \
         if (!attr_done) {                                                                                                    \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, 2, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, 2, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, 2, false, true, 28>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM_P28)); \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, 2, false, true, G2_PITCH, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, 2, true, true, G2_PITCH, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
+            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
+            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
+            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
             attr_done = true;                                                                                                \
         }                                                                                                                    \
-        if ((m & 1) == 0 && (reinterpret_cast<uintptr_t>(d_F) & 15) == 0) {                                                  \
-            if (use_bulk && have_tmap) {                                                                                     \
-                if (no_clamp) grad_projected_dmma_kernel<OUT, 2, false, true, G2_PITCH, true><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-                else grad_projected_dmma_kernel<OUT, 2, true, true, G2_PITCH, true><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-            } else if (use_bulk) {                                                                                           \
-                if (no_clamp && m <= 28 && use_p28) grad_projected_dmma_kernel<OUT, 2, false, true, 28><<<tiles, PW_THREADS, G2_SMEM_P28, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-                else if (no_clamp) grad_projected_dmma_kernel<OUT, 2, false, true><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-                else grad_projected_dmma_kernel<OUT, 2, true, true><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-            } else if (no_clamp) grad_projected_dmma_kernel<OUT, 2, false><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-            else grad_projected_dmma_kernel<OUT, 2><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-        } else                                                                                                               \
-            grad_projected_dmma_kernel<OUT, 1><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
+        if (have_tmap && no_clamp) grad_projected_dmma_kernel<OUT, false, true><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
+        else if (have_tmap) grad_projected_dmma_kernel<OUT, true, true><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
+        else grad_projected_dmma_kernel<OUT, true, false><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
     } while (0)
-        switch (outer) {
-            case DQGP_OUTER_GAUSSIAN: DQGP_G2(DQGP_OUTER_GAUSSIAN); break;
-            case DQGP_OUTER_MATERN15: DQGP_G2(DQGP_OUTER_MATERN15); break;
-            default: DQGP_G2(DQGP_OUTER_EXPSINE2); break;
-        }
-#undef DQGP_G2
+    switch (outer) {
+        case DQGP_OUTER_GAUSSIAN: DQGP_G2(DQGP_OUTER_GAUSSIAN); break;
+        case DQGP_OUTER_MATERN15: DQGP_G2(DQGP_OUTER_MATERN15); break;
+        default: DQGP_G2(DQGP_OUTER_EXPSINE2); break;
     }
-    DQGP_LAUNCH_CHECK("grad_projected_kernel");
+#undef DQGP_G2
+    DQGP_LAUNCH_CHECK("grad_projected_dmma_kernel");
     grad_reduce_kernel<<<P, 256, 0, st>>>(partial, tiles, P, 0.5 / (2.0 * h), d_grad);
     DQGP_LAUNCH_CHECK("grad_reduce_kernel");
     return 0;
@@ -695,18 +503,15 @@ int dqgp_grad_fidelity(const double* d_Ainv, int ld, const double* d_alpha, cons
                        double* d_grad, void* d_work, void* stream) {
     using namespace dqgp;
     DQGP_REQUIRE(d_Ainv && d_alpha && d_Psi && d_grad && d_work, "dqgp_grad_fidelity: NULL argument");
-    DQGP_REQUIRE(n >= 1 && ld >= n && P >= 1 && dim >= 1 && h != 0.0, "dqgp_grad_fidelity: bad shape / shift");
+    DQGP_REQUIRE(n >= 1 && ld >= n && P >= 1 && h != 0.0, "dqgp_grad_fidelity: bad shape / shift");
+    DQGP_REQUIRE(dim >= 2 && dim <= (1 << MAX_QUBITS) && (dim & (dim - 1)) == 0,
+                 "dqgp_grad_fidelity: dim %d is not 2^q amplitudes with 1 <= q <= %d", dim, MAX_QUBITS);
+    DQGP_REQUIRE((reinterpret_cast<uintptr_t>(d_Psi) & 15) == 0, "dqgp_grad_fidelity: the state array must be 16-byte aligned");
     const int tiles = grad_tiles(n);
     cudaStream_t st = as_stream(stream);
     double* partial = static_cast<double*>(d_work);
-    static const bool use_simt = getenv("DQGP_FID_SIMT") != nullptr;      // v1 SIMT kernel, kept for A/B checks
-    if (!use_simt && dim >= 2 && (reinterpret_cast<uintptr_t>(d_Psi) & 15) == 0) {
-        int rc = fidelity_grad_dmma(d_Ainv, ld, d_alpha, d_Psi, n, dim, P, partial, tiles, st);
-        if (rc) return rc;
-    } else {
-        grad_fidelity_kernel<<<tiles, PW_THREADS, 0, st>>>(d_Ainv, ld, d_alpha, reinterpret_cast<const double2*>(d_Psi), n, dim, P, partial);
-        DQGP_LAUNCH_CHECK("grad_fidelity_kernel");
-    }
+    int rc = fidelity_grad_dmma(d_Ainv, ld, d_alpha, d_Psi, n, dim, P, partial, tiles, st);
+    if (rc) return rc;
     grad_reduce_kernel<<<P, 256, 0, st>>>(partial, tiles, P, 0.5 / (2.0 * h), d_grad);
     DQGP_LAUNCH_CHECK("grad_reduce_kernel");
     return 0;

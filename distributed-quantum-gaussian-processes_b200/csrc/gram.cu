@@ -2,51 +2,16 @@
 // Replace ProjectedQuantumKernel.evaluate / FidelityKernel.evaluate (reference main.py:118-137, call
 // sites main.py:245,1420-1430, agent_riemannian.py:118).  One 64x64 tile of K per CTA; the only HBM
 // traffic besides the (tiny) feature tiles is the 8 B/entry store of K, issued as 128-bit stores.
-#include <cstdlib>
 #include "pairwise.cuh"
 
 namespace dqgp {
-
-template <int OUTER>
-__global__ void __launch_bounds__(PW_THREADS) gram_projected_kernel(const double* __restrict__ F1, int n1,
-                                                                    const double* __restrict__ F2, int n2, int m,
-                                                                    OuterHyp hyp, double* __restrict__ K, int ldk) {
-    __shared__ __align__(16) double FrT[PW_MAX_M * PW_PITCH];
-    __shared__ __align__(16) double FcT[PW_MAX_M * PW_PITCH];
-    const int row0 = blockIdx.y * PW_TILE, col0 = blockIdx.x * PW_TILE;
-    stage_features_T(FrT, F1, row0, n1, m);
-    stage_features_T(FcT, F2, col0, n2, m);
-    __syncthreads();
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    double d2[4][4];
-    micro_sqdist(FrT, FcT, m, ty, tx, d2);
-    const bool vec_ok = ((ldk & 1) == 0) && ((reinterpret_cast<uintptr_t>(K) & 15) == 0);
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int r = row0 + ty + 16 * i;
-        if (r >= n1) continue;
-#pragma unroll
-        for (int jj = 0; jj < 2; ++jj) {
-            const int c = col0 + 2 * tx + 32 * jj;
-            const double v0 = outer_eval<OUTER>(d2[i][2 * jj], hyp);
-            const double v1 = outer_eval<OUTER>(d2[i][2 * jj + 1], hyp);
-            double* dst = K + (size_t)r * ldk + c;
-            if (vec_ok && c + 1 < n2) {
-                *reinterpret_cast<double2*>(dst) = make_double2(v0, v1);
-            } else {
-                if (c < n2) dst[0] = v0;
-                if (c + 1 < n2) dst[1] = v1;
-            }
-        }
-    }
-}
 
 // ---- DMMA formulation of the projected Gram (same machinery as the fused gradient, grad.cu): -gamma*d^2 from the
 // Gram identity on DMMA.8x8x4, 11-instruction table exp, 16-byte stores.  SYM: only lower 64x64 tiles are computed
 // and each is stored twice (K and K^T; the transposed stores still fill whole 32-byte sectors), the diagonal is
 // exactly outer(0).  d^2 below 4e-15*(|f|^2+|g|^2) snaps to 0 so exact duplicates give exactly outer(0) = 1, as
-// the direct-difference form (kept below as gram_projected_kernel for odd cases) and SciPy's cdist do.
-// v1 (direct differences, libm exp) ran at 22% of the HBM write roofline: 72 FP64 instructions per entry.
+// direct differences and SciPy's cdist do.
+// v1 (direct differences, libm exp; since removed) ran at 22% of the HBM write roofline: 72 FP64 instructions per entry.
 template <int OUTER, int SYM>   // 0 rectangular, 1 lower tiles + mirror, 2 lower tiles only (what the factorisation reads)
 __global__ void __launch_bounds__(PW_THREADS) gram_projected_dmma_kernel(const double* __restrict__ F1, int n1,
                                                                          const double* __restrict__ F2, int n2, int m,
@@ -143,77 +108,6 @@ __global__ void __launch_bounds__(PW_THREADS) gram_projected_dmma_kernel(const d
     }
 }
 
-// Fidelity Gram: K[j][k] = |sum_i conj(psi2_k[i]) psi1_j[i]|^2, complex tile contraction over the 2^q
-// amplitudes in chunks of FID_KC, 4x4 complex accumulators per thread.
-constexpr int FID_KC = 16;
-constexpr int FID_PITCH = 65;   // double2 units
-
-__device__ __forceinline__ void stage_states_T(double2* dst, const double2* __restrict__ Psi, int row0, int n, int dim, int k0) {
-    // dst[kk*FID_PITCH + r] = Psi[(row0+r)*dim + k0+kk]
-    const int valid = min(PW_TILE, n - row0);
-    for (int e = threadIdx.x; e < PW_TILE * FID_KC; e += PW_THREADS) {
-        const int r = e / FID_KC, kk = e % FID_KC;
-        double2 v = make_double2(0.0, 0.0);
-        if (r < valid && k0 + kk < dim) v = Psi[(size_t)(row0 + r) * dim + k0 + kk];
-        dst[kk * FID_PITCH + r] = v;
-    }
-}
-
-__device__ __forceinline__ void micro_overlap(const double2* __restrict__ ArT, const double2* __restrict__ AcT, int ty, int tx,
-                                              double (&re)[4][4], double (&im)[4][4]) {
-#pragma unroll 4
-    for (int kk = 0; kk < FID_KC; ++kk) {
-        double2 a[4], b[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) a[i] = ArT[kk * FID_PITCH + ty + 16 * i];
-#pragma unroll
-        for (int jj = 0; jj < 2; ++jj) {
-            b[2 * jj] = AcT[kk * FID_PITCH + 2 * tx + 32 * jj];
-            b[2 * jj + 1] = AcT[kk * FID_PITCH + 2 * tx + 32 * jj + 1];
-        }
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                re[i][j] = fma(a[i].x, b[j].x, re[i][j]);
-                re[i][j] = fma(a[i].y, b[j].y, re[i][j]);
-                im[i][j] = fma(a[i].y, b[j].x, im[i][j]);
-                im[i][j] = fma(-a[i].x, b[j].y, im[i][j]);
-            }
-    }
-}
-
-__global__ void __launch_bounds__(PW_THREADS) gram_fidelity_kernel(const double2* __restrict__ Psi1, int n1,
-                                                                   const double2* __restrict__ Psi2, int n2, int dim,
-                                                                   double* __restrict__ K, int ldk) {
-    __shared__ __align__(16) double2 ArT[FID_KC * FID_PITCH];
-    __shared__ __align__(16) double2 AcT[FID_KC * FID_PITCH];
-    const int row0 = blockIdx.y * PW_TILE, col0 = blockIdx.x * PW_TILE;
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    double re[4][4], im[4][4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) re[i][j] = im[i][j] = 0.0;
-    for (int k0 = 0; k0 < dim; k0 += FID_KC) {
-        __syncthreads();
-        stage_states_T(ArT, Psi1, row0, n1, dim, k0);
-        stage_states_T(AcT, Psi2, col0, n2, dim, k0);
-        __syncthreads();
-        micro_overlap(ArT, AcT, ty, tx, re, im);
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int r = row0 + ty + 16 * i;
-        if (r >= n1) continue;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const int c = col0 + 2 * tx + 32 * (j >> 1) + (j & 1);
-            if (c < n2) K[(size_t)r * ldk + c] = re[i][j] * re[i][j] + im[i][j] * im[i][j];
-        }
-    }
-}
-
 __global__ void add_diagonal_kernel(double* A, int n, int lda, double v) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) A[(size_t)i * lda + i] += v;
@@ -235,13 +129,11 @@ int dqgp_gram_projected(int outer, const double* h_hyp, const double* d_F1, int 
     if (n1 == 0 || n2 == 0) return 0;
     dim3 grid((n2 + PW_TILE - 1) / PW_TILE, (n1 + PW_TILE - 1) / PW_TILE);
     cudaStream_t st = as_stream(stream);
-    static const bool use_direct = getenv("DQGP_GRAM_DIRECT") != nullptr;   // v1 direct-difference kernel, kept for A/B checks
     const bool sym = same && d_F1 == d_F2 && n1 == n2;
     const int tsym = grid.y * (grid.y + 1) / 2;
 #define DQGP_GRAM(OUT)                                                                                                     \
     do {                                                                                                                   \
-        if (use_direct) gram_projected_kernel<OUT><<<grid, PW_THREADS, 0, st>>>(d_F1, n1, d_F2, n2, m, hyp, d_K, ldk);      \
-        else if (sym && same == 2) gram_projected_dmma_kernel<OUT, 2><<<tsym, PW_THREADS, 0, st>>>(d_F1, n1, d_F2, n2, m, hyp, d_K, ldk); \
+        if (sym && same == 2) gram_projected_dmma_kernel<OUT, 2><<<tsym, PW_THREADS, 0, st>>>(d_F1, n1, d_F2, n2, m, hyp, d_K, ldk); \
         else if (sym) gram_projected_dmma_kernel<OUT, 1><<<tsym, PW_THREADS, 0, st>>>(d_F1, n1, d_F2, n2, m, hyp, d_K, ldk); \
         else gram_projected_dmma_kernel<OUT, 0><<<grid, PW_THREADS, 0, st>>>(d_F1, n1, d_F2, n2, m, hyp, d_K, ldk);        \
     } while (0)
@@ -251,7 +143,7 @@ int dqgp_gram_projected(int outer, const double* h_hyp, const double* d_F1, int 
         default: DQGP_GRAM(DQGP_OUTER_EXPSINE2); break;
     }
 #undef DQGP_GRAM
-    DQGP_LAUNCH_CHECK("gram_projected_kernel");
+    DQGP_LAUNCH_CHECK("gram_projected_dmma_kernel");
     return 0;
 }
 
@@ -261,16 +153,13 @@ int dqgp_gram_fidelity(const double* d_Psi1, int n1, const double* d_Psi2, int n
     (void)same;
     if (n1 == 0 || n2 == 0) return 0;
     DQGP_REQUIRE(d_Psi1 && d_Psi2 && d_K, "dqgp_gram_fidelity: NULL argument");
-    DQGP_REQUIRE(dim >= 1 && n1 >= 0 && n2 >= 0 && ldk >= n2, "dqgp_gram_fidelity: bad shape");
+    DQGP_REQUIRE(n1 >= 0 && n2 >= 0 && ldk >= n2, "dqgp_gram_fidelity: bad shape");
+    DQGP_REQUIRE(dim >= 2 && dim <= (1 << MAX_QUBITS) && (dim & (dim - 1)) == 0,
+                 "dqgp_gram_fidelity: dim %d is not 2^q amplitudes with 1 <= q <= %d", dim, MAX_QUBITS);
+    DQGP_REQUIRE(((reinterpret_cast<uintptr_t>(d_Psi1) | reinterpret_cast<uintptr_t>(d_Psi2)) & 15) == 0,
+                 "dqgp_gram_fidelity: state arrays must be 16-byte aligned");
     if (n1 == 0 || n2 == 0) return 0;
-    static const bool use_simt = getenv("DQGP_FID_SIMT") != nullptr;      // v1 SIMT kernel, kept for A/B checks
-    if (!use_simt && dim >= 2 && ((reinterpret_cast<uintptr_t>(d_Psi1) | reinterpret_cast<uintptr_t>(d_Psi2)) & 15) == 0)
-        return fidelity_gram_dmma(d_Psi1, n1, d_Psi2, n2, dim, d_K, ldk, as_stream(stream));
-    dim3 grid((n2 + PW_TILE - 1) / PW_TILE, (n1 + PW_TILE - 1) / PW_TILE);
-    gram_fidelity_kernel<<<grid, PW_THREADS, 0, as_stream(stream)>>>(reinterpret_cast<const double2*>(d_Psi1), n1,
-                                                                    reinterpret_cast<const double2*>(d_Psi2), n2, dim, d_K, ldk);
-    DQGP_LAUNCH_CHECK("gram_fidelity_kernel");
-    return 0;
+    return fidelity_gram_dmma(d_Psi1, n1, d_Psi2, n2, dim, d_K, ldk, as_stream(stream));
 }
 
 int dqgp_add_diagonal(double* d_A, int n, int lda, double value, void* stream) {

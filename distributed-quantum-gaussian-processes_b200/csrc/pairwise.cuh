@@ -1,10 +1,7 @@
 // Pairwise tile machinery shared by the Gram kernels (gram.cu) and the fused gradient kernels (grad.cu).
 //
-// A CTA of 256 threads owns a 64x64 tile of (row sample j, column sample k) pairs.  Thread (ty,tx) =
-// (tid>>4, tid&15) owns the 4x4 micro-tile rows {ty+16i} x cols {2tx+32jj+e}: a warp then touches two
-// tile rows and 64 contiguous columns, so K / A^-1 accesses are full 128-byte-line, 128-bit per lane.
-// Feature tiles live in shared memory transposed ([feature][sample], pitch 66) so a lane's two adjacent
-// columns are one LDS.128 and the row operand is a broadcast.
+// A CTA of 256 threads owns a 64x64 tile of (row sample j, column sample k) pairs; its 8 warps (4x2) each own a
+// 16x32 sub-tile as 2x4 DMMA 8x8 blocks.  Sample rows live in shared memory [sample][feature] with pitch G2_PITCH.
 #pragma once
 #include "common.cuh"
 #include "fastmath.cuh"
@@ -12,7 +9,6 @@
 namespace dqgp {
 
 constexpr int PW_TILE = 64;
-constexpr int PW_PITCH = 66;      // doubles; even (16-byte LDS.128 alignment), != multiple of 32
 constexpr int PW_THREADS = 256;
 constexpr int PW_MAX_M = 3 * MAX_QUBITS;
 
@@ -20,21 +16,6 @@ struct OuterHyp {
     double a;   // gaussian: gamma        | matern: 1/length_scale | expsine2: 1/length_scale
     double b;   //                                                  | expsine2: pi/periodicity
 };
-
-// Outer kernels with scikit-learn's formulas (sklearn/gaussian_process/kernels.py RBF / Matern(nu=1.5) /
-// ExpSineSquared, as used by squlearn's ProjectedQuantumKernel; reference main.py:130-137).
-template <int OUTER>
-__device__ __forceinline__ double outer_eval(double d2, const OuterHyp& h) {
-    if (OUTER == DQGP_OUTER_GAUSSIAN) {
-        return exp(-h.a * d2);
-    } else if (OUTER == DQGP_OUTER_MATERN15) {
-        const double k = sqrt(d2) * h.a * 1.7320508075688772;   // sqrt(3) * d / l
-        return (1.0 + k) * exp(-k);
-    } else {
-        const double s = sin(sqrt(d2) * h.b) * h.a;             // sin(pi d / p) / l
-        return exp(-2.0 * (s * s));
-    }
-}
 
 static inline int make_outer_hyp(int outer, const double* h_hyp, OuterHyp* out) {
     const double pi = 3.14159265358979323846;
@@ -60,45 +41,10 @@ static inline int make_outer_hyp(int outer, const double* h_hyp, OuterHyp* out) 
     return -1;
 }
 
-// Stage a (<=64 rows) x m feature tile into shared memory, transposed: dst[k*PW_PITCH + r] = F[(row0+r)*m + k].
-// Rows past n are zero-filled.  Global reads are fully coalesced (the tile is one contiguous span).
-__device__ __forceinline__ void stage_features_T(double* dst, const double* __restrict__ F, int row0, int n, int m) {
-    const int valid = min(PW_TILE, n - row0);
-    const double* src = F + (size_t)row0 * m;
-    for (int e = threadIdx.x; e < PW_TILE * m; e += PW_THREADS) {
-        const int r = e / m, k = e - r * m;
-        dst[k * PW_PITCH + r] = (r < valid) ? src[e] : 0.0;
-    }
-}
-
-// squared distances of the thread's 4x4 micro-tile by direct differences (what SciPy cdist does; exact 0
-// on identical inputs, no cancellation for near-duplicates — SURVEY §7.3.3)
-__device__ __forceinline__ void micro_sqdist(const double* __restrict__ FrT, const double* __restrict__ FcT, int m, int ty,
-                                             int tx, double (&d2)[4][4]) {
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) d2[i][j] = 0.0;
-#pragma unroll 2
-    for (int k = 0; k < m; ++k) {
-        double a[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) a[i] = FrT[k * PW_PITCH + ty + 16 * i];
-        const double2 b0 = *reinterpret_cast<const double2*>(&FcT[k * PW_PITCH + 2 * tx]);
-        const double2 b1 = *reinterpret_cast<const double2*>(&FcT[k * PW_PITCH + 2 * tx + 32]);
-        const double b[4] = {b0.x, b0.y, b1.x, b1.y};
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const double df = a[i] - b[j];
-                d2[i][j] = fma(df, df, d2[i][j]);
-            }
-    }
-}
-
 // Outer kernel from v = -gamma_eff * d^2 (gamma_eff = gamma for the Gaussian, 1 otherwise), as left in a DMMA
-// accumulator by the Gram identity.  Warp-collective: fast_exp_tab shuffles its table.
+// accumulator by the Gram identity, with scikit-learn's formulas (sklearn/gaussian_process/kernels.py RBF /
+// Matern(nu=1.5) / ExpSineSquared, as used by squlearn's ProjectedQuantumKernel; reference main.py:130-137).
+// Warp-collective: fast_exp_tab shuffles its table.
 template <int OUTER>
 __device__ __forceinline__ double outer_from_neg_gd2(double v, const OuterHyp& h, double tab) {
     // v = -gamma_eff * d^2 (gamma_eff = gamma for the Gaussian, 1 otherwise); warp-collective (table shuffle)

@@ -15,7 +15,6 @@
 // __syncwarp separates passes.  The epilogue reduces <X_k>,<Y_k>,<Z_k> three qubits at a time from registers
 // with group-local shuffles, or streams the state to HBM for the fidelity kernel.
 #include <cstdlib>
-#include <type_traits>
 #include "common.cuh"
 
 namespace dqgp {
@@ -901,7 +900,7 @@ __global__ void __launch_bounds__(SvTeam<Q>::THREADS) statevec_lc_kernel(
 // ---- lc2: the linear-combination form, rebuilt around what ncu showed in round 2 (profiles/r02_sv_q10_before.txt: FP64 pipe
 // 33%, issue slots 52%, 68% of all instructions are not FP64) -------------------------------------------------------------------
 // For circuits whose parameters ALL enter through one RX / RY / RZ (yz_cx, kyriienko: BASELINE configs 4 and 5), features only.
-//  * TWO forks advance together through every pass (run_pass2<B, 2>): the op decode, control predicates, address arithmetic and
+//  * TWO forks advance together through every pass (run_pass3<Q, B, 2>): the op decode, address arithmetic and
 //    fused-matrix loads of a pass are paid once for two states, and every thread carries two independent FP64 chains;
 //  * the first pass of a fork reads the base state and writes the fork's scratch (no copy);
 //  * ONE epilogue sweep per fork gives <phi|O|phi> and Re<psi|O|phi> together (each scratch amplitude is loaded once per qubit
@@ -911,98 +910,6 @@ __global__ void __launch_bounds__(SvTeam<Q>::THREADS) statevec_lc_kernel(
 //  * the gate program is read from global memory (uniform, L1-resident) instead of being copied into every CTA's shared memory.
 // __noinline__: one copy of each instantiation for all call sites (the inlined version stalled 14% of the time on instruction
 // fetch, profiles/r02_sv_q10_lc2_v1.txt).
-template <int B, int NS, bool ALT>
-__device__ __noinline__ void run_pass2(const double2* __restrict__ src0, const double2* __restrict__ src1, double2* __restrict__ dst0,
-                                       double2* __restrict__ dst1, const SvPass* __restrict__ pass, const SvOp* __restrict__ ops,
-                                       const double2* __restrict__ mats, const double2* __restrict__ trig, int lig, int lps, int groups,
-                                       int alt_mat0, const double2* __restrict__ alt_u0, int alt_mat1, const double2* __restrict__ alt_u1) {
-    constexpr int N = 1 << B;
-    const SvPass ps = *pass;
-    const int q0 = ps.q[0], q1 = ps.q[1], q2 = ps.q[2];
-    int off[N];
-#pragma unroll
-    for (int j = 0; j < N; ++j) off[j] = ((j & 1) ? (1 << q0) : 0) + ((B > 1 && (j & 2)) ? (1 << q1) : 0) + ((B > 2 && (j & 4)) ? (1 << q2) : 0);
-    for (int gi = lig; gi < groups; gi += lps) {
-        int base = insert_zero_bit(gi, q0);
-        if (B > 1) base = insert_zero_bit(base, q1);
-        if (B > 2) base = insert_zero_bit(base, q2);
-        // CX gates with an outside control at the head / tail of the pass: flip the target bit of the load / store address
-        int xl = 0, xs = 0;
-        for (int o = ps.op_begin; o < ps.lead_end; ++o) {
-            const SvOp op = ops[o];
-            if ((base >> op.cq) & 1) xl ^= 1 << (op.lbit == 0 ? q0 : (op.lbit == 1 ? q1 : q2));
-        }
-        for (int o = ps.trail_begin; o < ps.op_end; ++o) {
-            const SvOp op = ops[o];
-            if ((base >> op.cq) & 1) xs ^= 1 << (op.lbit == 0 ? q0 : (op.lbit == 1 ? q1 : q2));
-        }
-        int addr[N];
-        double2 r0[N], r1[N];      // r1 is dead code for NS == 1
-#pragma unroll
-        for (int j = 0; j < N; ++j) {
-            addr[j] = base + off[j];
-            const int a = sv_phys(addr[j] ^ xl);
-            r0[j] = src0[a];
-            if (NS == 2) r1[j] = src1[a];
-        }
-        SvOp nxt = ops[ps.lead_end < ps.trail_begin ? ps.lead_end : ps.op_begin];
-#pragma unroll 1
-        for (int o = ps.lead_end; o < ps.trail_begin; ++o) {
-            const SvOp op = nxt;
-            if (o + 1 < ps.trail_begin) nxt = ops[o + 1];          // the next op's fetch overlaps this op's arithmetic
-            if (op.kind == SV_U2) {
-                const double2* u0 = mats + 4 * op.idx;
-                const double2* u1 = u0;
-                if (ALT) {
-                    if (op.idx == alt_mat0) u0 = alt_u0;
-                    if (NS == 2 && op.idx == alt_mat1) u1 = alt_u1;
-                }
-                double2 a = u0[0], b = u0[1], c = u0[2], d = u0[3];
-                if (op.lbit == 0) apply_u2<N, 0>(r0, a, b, c, d);
-                else if (B > 1 && op.lbit == 1) apply_u2<N, (B > 1 ? 1 : 0)>(r0, a, b, c, d);
-                else if (B > 2) apply_u2<N, (B > 2 ? 2 : 0)>(r0, a, b, c, d);
-                if (NS == 2) {
-                    if (ALT && u1 != u0) { a = u1[0]; b = u1[1]; c = u1[2]; d = u1[3]; }
-                    if (op.lbit == 0) apply_u2<N, 0>(r1, a, b, c, d);
-                    else if (B > 1 && op.lbit == 1) apply_u2<N, (B > 1 ? 1 : 0)>(r1, a, b, c, d);
-                    else if (B > 2) apply_u2<N, (B > 2 ? 2 : 0)>(r1, a, b, c, d);
-                }
-            } else {
-                const bool ext = (op.cq >= 0) ? (((base >> op.cq) & 1) != 0) : false;
-                const double2 cs = (op.kind == SV_CRZ) ? trig[op.idx] : make_double2(1.0, 0.0);
-                if (op.lbit == 0) {
-                    apply_controlled<N, 0>(r0, op.kind, op.cloc, ext, cs.x, cs.y);
-                    if (NS == 2) apply_controlled<N, 0>(r1, op.kind, op.cloc, ext, cs.x, cs.y);
-                } else if (B > 1 && op.lbit == 1) {
-                    apply_controlled<N, (B > 1 ? 1 : 0)>(r0, op.kind, op.cloc, ext, cs.x, cs.y);
-                    if (NS == 2) apply_controlled<N, (B > 1 ? 1 : 0)>(r1, op.kind, op.cloc, ext, cs.x, cs.y);
-                } else if (B > 2) {
-                    apply_controlled<N, (B > 2 ? 2 : 0)>(r0, op.kind, op.cloc, ext, cs.x, cs.y);
-                    if (NS == 2) apply_controlled<N, (B > 2 ? 2 : 0)>(r1, op.kind, op.cloc, ext, cs.x, cs.y);
-                }
-            }
-        }
-#pragma unroll
-        for (int j = 0; j < N; ++j) {
-            const int a = sv_phys(addr[j] ^ xs);
-            dst0[a] = r0[j];
-            if (NS == 2) dst1[a] = r1[j];
-        }
-    }
-}
-
-template <int Q, int NS, bool ALT>
-__device__ __forceinline__ void sv_pass2(const double2* src0, const double2* src1, double2* dst0, double2* dst1, const SvPass* ps_ptr,
-                                         const SvOp* __restrict__ ops, const double2* __restrict__ u2, const double2* __restrict__ trig, int lig,
-                                         int am0, const double2* au0, int am1, const double2* au1) {
-    using T = SvTeam<Q>;
-    const int nq = ps_ptr->nq;
-    if (nq == 3) run_pass2<(Q >= 3 ? 3 : 1), NS, ALT>(src0, src1, dst0, dst1, ps_ptr, ops, u2, trig, lig, T::SIZE, T::DIM >> 3, am0, au0, am1, au1);
-    else if (nq == 2) run_pass2<(Q >= 2 ? 2 : 1), NS, ALT>(src0, src1, dst0, dst1, ps_ptr, ops, u2, trig, lig, T::SIZE, T::DIM >> 2, am0, au0, am1, au1);
-    else run_pass2<1, NS, ALT>(src0, src1, dst0, dst1, ps_ptr, ops, u2, trig, lig, T::SIZE, T::DIM >> 1, am0, au0, am1, au1);
-    T::sync();
-}
-
 // ---- CX-free passes (SvPass3): the coset a thread owns is selected by the bits of its index through the pass's rest masks; register j
 // holds the amplitude whose logical block bits are j.  Only fused 2x2 unitaries are executed: CX gates live in the index map.
 template <int NREST>
@@ -1110,10 +1017,10 @@ struct TeamReduceLeft { static constexpr int value = (N / W) > 1 ? (N / W) : 1; 
 
 // value ids of one fork in the reduction buffer: [Bx | By | Bz | Cx | Cy | Cz] x Q, B = <phi|O|phi> (X, Y without their factor 2),
 // C = Re<psi|O|phi>; red[id * NW + warp]
-// MAPPED: positions through the final index map of the CX-free plan (`grp`: the group's block / rest masks)
-template <int Q, int B, bool MAPPED = false>
+// positions through the final index map of the CX-free plan (`grp`: the group's block / rest masks)
+template <int Q, int B>
 __device__ __forceinline__ void lc2_group_xy(const double2* __restrict__ fin, const double2* __restrict__ scr, int k0, int lig, int warp,
-                                             double* __restrict__ red, const SvPass3* __restrict__ grp = nullptr) {
+                                             double* __restrict__ red, const SvPass3* __restrict__ grp) {
     using T = SvTeam<Q>;
     constexpr int N = 1 << B, NV = 16, W = T::SIZE < 32 ? T::SIZE : 32, NW = T::BLOCK ? T::SIZE / 32 : 1;
     const int groups = T::DIM >> B;
@@ -1121,25 +1028,14 @@ __device__ __forceinline__ void lc2_group_xy(const double2* __restrict__ fin, co
 #pragma unroll
     for (int i = 0; i < NV; ++i) v[i] = 0.0;
     int comb[N];
-    if (MAPPED) {
 #pragma unroll
-        for (int j = 0; j < N; ++j) comb[j] = ((j & 1) ? grp->bm[0] : 0) ^ ((B > 1 && (j & 2)) ? grp->bm[1] : 0) ^ ((B > 2 && (j & 4)) ? grp->bm[2] : 0);
-    }
+    for (int j = 0; j < N; ++j) comb[j] = ((j & 1) ? grp->bm[0] : 0) ^ ((B > 1 && (j & 2)) ? grp->bm[1] : 0) ^ ((B > 2 && (j & 4)) ? grp->bm[2] : 0);
     for (int gi = lig; gi < groups; gi += T::SIZE) {
-        int base = gi;
-        if (MAPPED) {
-            base = coset_base<Q - B>(grp->rest, gi);
-        } else {
-#pragma unroll
-            for (int l = 0; l < B; ++l) base = insert_zero_bit(base, k0 + l);
-        }
+        const int base = coset_base<Q - B>(grp->rest, gi);
         double2 p[N], s[N];
 #pragma unroll
         for (int j = 0; j < N; ++j) {
-            int o = 0;
-#pragma unroll
-            for (int l = 0; l < B; ++l) o += ((j >> l) & 1) << (k0 + l);
-            const int a = MAPPED ? sv_phys(base ^ comb[j]) : sv_phys(base + o);
+            const int a = sv_phys(base ^ comb[j]);
             p[j] = fin[a];
             s[j] = scr[a];
         }
@@ -1173,25 +1069,23 @@ __device__ __forceinline__ void lc2_group_xy(const double2* __restrict__ fin, co
 }
 
 // Z observables of a fork from ONE layout (block qubits 0, 1, 2): <phi|Z_k|phi> = sum_a (+-)|phi_a|^2, Re<psi|Z_k|phi> likewise
-template <int Q, bool MAPPED = false>
+template <int Q>
 __device__ __forceinline__ void lc2_group_z(const double2* __restrict__ fin, const double2* __restrict__ scr, int lig, int warp,
-                                            double* __restrict__ red, const SvPass3* __restrict__ grp = nullptr) {
+                                            double* __restrict__ red, const SvPass3* __restrict__ grp) {
     using T = SvTeam<Q>;
     constexpr int NZ = (2 * Q <= 16) ? 16 : 32, W = T::SIZE < 32 ? T::SIZE : 32, NW = T::BLOCK ? T::SIZE / 32 : 1;
     double v[NZ];
 #pragma unroll
     for (int i = 0; i < NZ; ++i) v[i] = 0.0;
     int comb[8];
-    if (MAPPED) {
 #pragma unroll
-        for (int j = 0; j < 8; ++j) comb[j] = ((j & 1) ? grp->bm[0] : 0) ^ ((j & 2) ? grp->bm[1] : 0) ^ ((j & 4) ? grp->bm[2] : 0);
-    }
+    for (int j = 0; j < 8; ++j) comb[j] = ((j & 1) ? grp->bm[0] : 0) ^ ((j & 2) ? grp->bm[1] : 0) ^ ((j & 4) ? grp->bm[2] : 0);
     for (int gi = lig; gi < (T::DIM >> 3); gi += T::SIZE) {
-        const int base = MAPPED ? coset_base<(Q >= 3 ? Q - 3 : 0)>(grp->rest, gi) : (gi << 3);
+        const int base = coset_base<(Q >= 3 ? Q - 3 : 0)>(grp->rest, gi);
         double pp[8], ww[8];
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
-            const int a = MAPPED ? sv_phys(base ^ comb[j]) : sv_phys(base + j);
+            const int a = sv_phys(base ^ comb[j]);
             const double2 ps = fin[a], ph = scr[a];
             pp[j] = fma(ph.x, ph.x, ph.y * ph.y);
             ww[j] = fma(ps.x, ph.x, ps.y * ph.y);
@@ -1231,27 +1125,27 @@ __device__ __forceinline__ void lc2_group_z(const double2* __restrict__ fin, con
 }
 
 // one fork's epilogue: both central-difference sets of parameter i from A = <psi|O|psi> (featA), B, C
-// all partial sums of one fork into `red` (no synchronisation); `grps`: the epilogue groups of the CX-free plan (MAPPED)
-template <int Q, bool MAPPED>
+// all partial sums of one fork into `red` (no synchronisation); `grps`: the epilogue groups of the CX-free plan
+template <int Q>
 __device__ __forceinline__ void lc2_collect(const double2* __restrict__ fin, const double2* __restrict__ scr, double* __restrict__ red, int lig,
                                             const SvPass3* __restrict__ grps) {
     using T = SvTeam<Q>;
     constexpr int FULL = Q / 3, REM = Q % 3;
     const int warp = T::BLOCK ? (lig >> 5) : 0;
-    lc2_group_z<Q, MAPPED>(fin, scr, lig, warp, red, grps);
+    lc2_group_z<Q>(fin, scr, lig, warp, red, grps);
 #pragma unroll 1
-    for (int b = 0; b < FULL; ++b) lc2_group_xy<Q, 3, MAPPED>(fin, scr, 3 * b, lig, warp, red, MAPPED ? grps + b : nullptr);
-    if (REM == 2) lc2_group_xy<Q, 2, MAPPED>(fin, scr, 3 * FULL, lig, warp, red, MAPPED ? grps + FULL : nullptr);
-    if (REM == 1) lc2_group_xy<Q, 1, MAPPED>(fin, scr, 3 * FULL, lig, warp, red, MAPPED ? grps + FULL : nullptr);
+    for (int b = 0; b < FULL; ++b) lc2_group_xy<Q, 3>(fin, scr, 3 * b, lig, warp, red, grps + b);
+    if (REM == 2) lc2_group_xy<Q, 2>(fin, scr, 3 * FULL, lig, warp, red, grps + FULL);
+    if (REM == 1) lc2_group_xy<Q, 1>(fin, scr, 3 * FULL, lig, warp, red, grps + FULL);
 }
 
-template <int Q, bool MAPPED = false>
+template <int Q>
 __device__ __forceinline__ void lc2_emit(const double2* __restrict__ fin, const double2* __restrict__ scr, const double* __restrict__ featA,
                                          double* __restrict__ red, int lig, bool live, double c0, double s0, double c1, double s1,
-                                         double* __restrict__ out_plus, double* __restrict__ out_minus, const SvPass3* __restrict__ grps = nullptr) {
+                                         double* __restrict__ out_plus, double* __restrict__ out_minus, const SvPass3* __restrict__ grps) {
     using T = SvTeam<Q>;
     constexpr int NW = T::BLOCK ? T::SIZE / 32 : 1, M3 = 3 * Q;
-    lc2_collect<Q, MAPPED>(fin, scr, red, lig, grps);
+    lc2_collect<Q>(fin, scr, red, lig, grps);
     T::sync();
     if (live) {
         for (int k = lig; k < M3; k += T::SIZE) {
@@ -1267,56 +1161,37 @@ __device__ __forceinline__ void lc2_emit(const double2* __restrict__ fin, const 
     T::sync();
 }
 
-template <int Q, int NS, bool ALT, bool MAPPED, typename PassT>
-__device__ __forceinline__ void lc2_pass(const double2* src0, const double2* src1, double2* dst0, double2* dst1, const PassT* ps,
-                                         const SvOp* __restrict__ ops, const double2* __restrict__ u2, const double2* __restrict__ trig, int lig,
-                                         int am0, const double2* au0, int am1, const double2* au1) {
-    if constexpr (MAPPED) sv_pass3<Q, NS, ALT>(src0, src1, dst0, dst1, ps, ops, u2, lig, am0, au0, am1, au1);
-    else sv_pass2<Q, NS, ALT>(src0, src1, dst0, dst1, ps, ops, u2, trig, lig, am0, au0, am1, au1);
-}
-
-// PAIR = false: one fork at a time and three state copies (no second scratch): the variant for one-state-per-warp teams (q <= 8)
-// MAPPED = true: the CX-free plan (SvPass3 passes; CX gates absorbed into the logical -> physical index map, Pauli features read
-// through the final map)
-// Resident CTAs the register allocation must allow: lane-group teams (q <= 8) 4 x 128 threads; CTA-per-state teams up to q = 10 three
-// CTAs with pairing (four state copies, 73 KB), four without (three copies and the plan read from global memory: 56 KB per CTA at
-// q = 10 - measured 37.3 ms against 36.3 ms for the paired variant at config 5, so pairing stays the default; DQGP_SV_UNPAIRED for A/B).
-// Without the bound the paired q = 10 kernel takes 174 registers and drops to two CTAs per SM (39.8 ms).
-template <int Q, bool PAIR>
-struct Lc2Bounds { static constexpr int MIN_BLOCKS = !SvTeam<Q>::BLOCK ? (PAIR ? 3 : 0) : (Q > 10 ? 0 : (PAIR ? 3 : 4)); };   // 0 = unspecified
-template <int Q, bool PAIR, bool MAPPED>
-__global__ void __launch_bounds__(SvTeam<Q>::THREADS, Lc2Bounds<Q, PAIR>::MIN_BLOCKS) statevec_lc2_kernel(
-    const dqgp_gate* __restrict__ g_gates, int n_gates, const typename std::conditional<MAPPED, SvPass3, SvPass>::type* __restrict__ g_passes,
-    int n_passes, const SvOp* __restrict__ g_ops,
+// Runs the CX-free plan (SvPass3 passes; CX gates absorbed into the logical -> physical index map, Pauli features read through the
+// final map).  PAIR: where a CTA owns the state (q >= 9) two forks advance together through every pass (four state copies); a
+// lane-group team (q <= 8) takes one fork at a time with three state copies (no second scratch).
+// Resident CTAs the register allocation must allow: CTA-per-state teams up to q = 10 three CTAs (73 KB each).  Without the bound the
+// q = 10 kernel takes 174 registers and drops to two CTAs per SM (39.8 ms at config 5 against 36.3 ms).  (An unpaired CTA-per-state
+// variant - three copies, the plan read from global memory, four CTAs per SM - measured 37.3 ms there and was removed.)
+template <int Q>
+constexpr int LC2_MIN_BLOCKS = (SvTeam<Q>::BLOCK && Q <= 10) ? 3 : 0;      // 0 = unspecified
+template <int Q>
+__global__ void __launch_bounds__(SvTeam<Q>::THREADS, LC2_MIN_BLOCKS<Q>) statevec_lc2_kernel(
+    const dqgp_gate* __restrict__ g_gates, int n_gates, const SvPass3* __restrict__ g_passes, int n_passes, const SvOp* __restrict__ g_ops,
     const SvMat* __restrict__ g_mats, int n_mats, const int* __restrict__ g_mat_gates, const int* __restrict__ g_share, int d, int P,
-    int uses_acos, int pair_forks, const double* __restrict__ X, int n, const double* __restrict__ Pm, double* __restrict__ out) {
+    int uses_acos, const double* __restrict__ X, int n, const double* __restrict__ Pm, double* __restrict__ out) {
     using T = SvTeam<Q>;
-    using PassT = typename std::conditional<MAPPED, SvPass3, SvPass>::type;
+    using PassT = SvPass3;
+    constexpr bool PAIR = T::BLOCK;
     constexpr int M3 = 3 * Q, M3P = (M3 + 1) & ~1, NW = T::BLOCK ? T::SIZE / 32 : 1;
-    constexpr int N_EPI = MAPPED ? (Q + 2) / 3 : 0;        // epilogue group entries stored after the real passes
+    constexpr int N_EPI = (Q + 2) / 3;        // epilogue group entries stored after the real passes
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int* par_gate = g_share;
     const int* par_mat = g_share + P;
     const int* pass_par_begin = g_share + 2 * P;
     const int* pass_params = g_share + 2 * P + n_passes + 1;
     // per CTA: the op list and the pass table (read in every pass; the rest of the gate program stays in global memory)
-    constexpr bool STAGE_PLAN = !(T::BLOCK && !PAIR);      // the unpaired CTA-per-state variant spends its shared memory on a fourth CTA
-    const size_t op_bytes = STAGE_PLAN ? ((sizeof(SvOp) * n_gates + 15) & ~size_t(15)) : 0;
-    const size_t pass_bytes = STAGE_PLAN ? ((sizeof(PassT) * (n_passes + N_EPI) + 15) & ~size_t(15)) : 0;
-    const SvOp* s_ops;
-    const PassT* s_passes;
-    if constexpr (STAGE_PLAN) {          // (if constexpr: one address space per instantiation, so the staged reads stay LDS)
-        SvOp* so = reinterpret_cast<SvOp*>(smem_raw);
-        PassT* sp = reinterpret_cast<PassT*>(smem_raw + op_bytes);
-        for (int i = threadIdx.x; i < n_gates; i += blockDim.x) so[i] = g_ops[i];        // #ops <= #gates
-        for (int i = threadIdx.x; i < n_passes + N_EPI; i += blockDim.x) sp[i] = g_passes[i];
-        s_ops = so;
-        s_passes = sp;
-    } else {
-        s_ops = g_ops;
-        s_passes = g_passes;
-    }
-    const SvPass3* epi = reinterpret_cast<const SvPass3*>(s_passes + n_passes);        // MAPPED only
+    const size_t op_bytes = (sizeof(SvOp) * n_gates + 15) & ~size_t(15);
+    const size_t pass_bytes = (sizeof(PassT) * (n_passes + N_EPI) + 15) & ~size_t(15);
+    SvOp* s_ops = reinterpret_cast<SvOp*>(smem_raw);
+    PassT* s_passes = reinterpret_cast<PassT*>(smem_raw + op_bytes);
+    for (int i = threadIdx.x; i < n_gates; i += blockDim.x) s_ops[i] = g_ops[i];        // #ops <= #gates
+    for (int i = threadIdx.x; i < n_passes + N_EPI; i += blockDim.x) s_passes[i] = g_passes[i];
+    const SvPass3* epi = s_passes + n_passes;
     __syncthreads();
     // per-team storage: base | scratch 0 | scratch 1 | final base state | cos/sin table | fused matrices | 2 fork matrices | acos | red | A
     const size_t team_bytes = sizeof(double2) * ((PAIR ? 4 : 3) * T::DIM + n_gates + 4 * n_mats + 8) + sizeof(double) * (((d + 1) & ~1) + 2 * M3 * NW + M3P + 8);
@@ -1360,39 +1235,28 @@ __global__ void __launch_bounds__(SvTeam<Q>::THREADS, Lc2Bounds<Q, PAIR>::MIN_BL
         T::sync();
 
         // sweep 1: the final base state (kept for the cross terms) and the base set's features A
-        for (int ip = 0; ip < n_passes; ++ip) lc2_pass<Q, 1, false, MAPPED>(fin, fin, fin, fin, s_passes + ip, s_ops, u2, trig, lig, -1, nullptr, -1, nullptr);
-        if (MAPPED) {
-            // A = <psi|O|psi> through the final index map: the fork epilogue's own sums with phi = psi
-            lc2_collect<Q, MAPPED>(fin, fin, red, lig, epi);
-            T::sync();
-            for (int k = lig; k < M3; k += T::SIZE) {
-                double Bv = 0.0;
+        for (int ip = 0; ip < n_passes; ++ip) sv_pass3<Q, 1, false>(fin, fin, fin, fin, s_passes + ip, s_ops, u2, lig, -1, nullptr, -1, nullptr);
+        // A = <psi|O|psi> through the final index map: the fork epilogue's own sums with phi = psi
+        lc2_collect<Q>(fin, fin, red, lig, epi);
+        T::sync();
+        for (int k = lig; k < M3; k += T::SIZE) {
+            double Bv = 0.0;
 #pragma unroll
-                for (int w = 0; w < NW; ++w) Bv += red[k * NW + w];
-                featA[k] = (k < 2 * Q) ? 2.0 * Bv : Bv;
-            }
-            T::sync();
-            if (live)
-                for (int k = lig; k < M3; k += T::SIZE) out[(size_t)j * M3 + k] = featA[k];
-        } else {
-            constexpr int FULL = Q / 3, REM = Q % 3;
-#pragma unroll 1
-            for (int b = 0; b < FULL; ++b) features_block<(Q >= 3 ? 3 : 1), Q>(fin, 3 * b, lig, T::SIZE, true, featA, red);
-            if (REM == 2) features_block<(Q >= 2 ? 2 : 1), Q>(fin, 3 * FULL, lig, T::SIZE, true, featA, red);
-            if (REM == 1) features_block<1, Q>(fin, 3 * FULL, lig, T::SIZE, true, featA, red);
-            T::sync();
-            if (live)
-                for (int k = lig; k < M3; k += T::SIZE) out[(size_t)j * M3 + k] = featA[k];
+            for (int w = 0; w < NW; ++w) Bv += red[k * NW + w];
+            featA[k] = (k < 2 * Q) ? 2.0 * Bv : Bv;
         }
+        T::sync();
+        if (live)
+            for (int k = lig; k < M3; k += T::SIZE) out[(size_t)j * M3 + k] = featA[k];
         T::sync();
 
         // sweep 2: advance the base pass by pass; before pass ip runs, fork every parameter whose rotation lives in it
         for (int ip = 0; ip < n_passes; ++ip) {
             const int pb = pass_par_begin[ip], pe = pass_par_begin[ip + 1];
             const PassT* ps0 = s_passes + ip;
-            for (int f0 = pb; f0 < pe; f0 += ((PAIR && pair_forks) ? 2 : 1)) {
+            for (int f0 = pb; f0 < pe; f0 += (PAIR ? 2 : 1)) {
                 const int i0 = pass_params[f0];
-                const int i1 = (PAIR && pair_forks && f0 + 1 < pe) ? pass_params[f0 + 1] : -1;
+                const int i1 = (PAIR && f0 + 1 < pe) ? pass_params[f0 + 1] : -1;
                 // fork matrices: the parameter's rotation with its angle advanced by pi: (cos, sin)(theta/2 + pi/2) = (-sin, cos)(theta/2)
                 // and the linear-combination coefficients cos / sin of half the two angle differences (once per fork, not per thread)
                 for (int e = lig; e < 2; e += T::SIZE) {
@@ -1408,41 +1272,41 @@ __global__ void __launch_bounds__(SvTeam<Q>::THREADS, Lc2Bounds<Q, PAIR>::MIN_BL
                 }
                 T::sync();
                 if (PAIR && i1 >= 0) {
-                    lc2_pass<Q, (PAIR ? 2 : 1), true, MAPPED>(base, base, scr0, scr1, ps0, s_ops, u2, trig, lig, par_mat[i0], altm, par_mat[i1], altm + 4);
+                    sv_pass3<Q, (PAIR ? 2 : 1), true>(base, base, scr0, scr1, ps0, s_ops, u2, lig, par_mat[i0], altm, par_mat[i1], altm + 4);
                     for (int kp = ip + 1; kp < n_passes; ++kp)
-                        lc2_pass<Q, (PAIR ? 2 : 1), false, MAPPED>(scr0, scr1, scr0, scr1, s_passes + kp, s_ops, u2, trig, lig, -1, nullptr, -1, nullptr);
+                        sv_pass3<Q, (PAIR ? 2 : 1), false>(scr0, scr1, scr0, scr1, s_passes + kp, s_ops, u2, lig, -1, nullptr, -1, nullptr);
                 } else {
-                    lc2_pass<Q, 1, true, MAPPED>(base, base, scr0, scr0, ps0, s_ops, u2, trig, lig, par_mat[i0], altm, -1, nullptr);
+                    sv_pass3<Q, 1, true>(base, base, scr0, scr0, ps0, s_ops, u2, lig, par_mat[i0], altm, -1, nullptr);
                     for (int kp = ip + 1; kp < n_passes; ++kp)
-                        lc2_pass<Q, 1, false, MAPPED>(scr0, scr0, scr0, scr0, s_passes + kp, s_ops, u2, trig, lig, -1, nullptr, -1, nullptr);
+                        sv_pass3<Q, 1, false>(scr0, scr0, scr0, scr0, s_passes + kp, s_ops, u2, lig, -1, nullptr, -1, nullptr);
                 }
 #pragma unroll 1
                 for (int e = 0; e < 2; ++e) {
                     const int i = e == 0 ? i0 : i1;
                     if (i < 0) break;
-                    lc2_emit<Q, MAPPED>(fin, e == 0 ? scr0 : scr1, featA, red, lig, live, coef[4 * e], coef[4 * e + 1], coef[4 * e + 2], coef[4 * e + 3],
+                    lc2_emit<Q>(fin, e == 0 ? scr0 : scr1, featA, red, lig, live, coef[4 * e], coef[4 * e + 1], coef[4 * e + 2], coef[4 * e + 3],
                                         out + ((size_t)(1 + 2 * i) * n + j) * M3, out + ((size_t)(2 + 2 * i) * n + j) * M3, epi);
                 }
             }
-            lc2_pass<Q, 1, false, MAPPED>(base, base, base, base, ps0, s_ops, u2, trig, lig, -1, nullptr, -1, nullptr);
+            sv_pass3<Q, 1, false>(base, base, base, base, ps0, s_ops, u2, lig, -1, nullptr, -1, nullptr);
         }
         T::sync();
     }
 }
 
-template <int Q, bool MAPPED, bool PAIR>
-static int launch_sv_lc2_impl(const dqgp_circuit* c, const double* X, int n, const double* Pm, double* out, cudaStream_t st) {
+template <int Q>
+static int launch_sv_lc2(const dqgp_circuit* c, const double* X, int n, const double* Pm, double* out, cudaStream_t st) {
     using T = SvTeam<Q>;
-    using PassT = typename std::conditional<MAPPED, SvPass3, SvPass>::type;
+    constexpr bool PAIR = T::BLOCK;
     const int n_gates = (int)c->gates.size();
-    const int n_passes = MAPPED ? c->n_passes3 : (int)c->passes.size(), n_mats = (int)(MAPPED ? c->mats3.size() : c->mats.size());
-    const int n_epi = MAPPED ? (Q + 2) / 3 : 0;
+    const int n_passes = c->n_passes3, n_mats = (int)c->mats3.size();
+    const int n_epi = (Q + 2) / 3;
     constexpr int M3 = 3 * Q, M3P = (M3 + 1) & ~1, NW = T::BLOCK ? T::SIZE / 32 : 1;
     const size_t team_bytes = sizeof(double2) * ((PAIR ? 4 : 3) * T::DIM + n_gates + 4 * n_mats + 8) + sizeof(double) * (((c->d + 1) & ~1) + 2 * M3 * NW + M3P + 8);
-    const size_t fixed = (T::BLOCK && !PAIR) ? 0 : ((sizeof(SvOp) * n_gates + 15) & ~size_t(15)) + ((sizeof(PassT) * (n_passes + n_epi) + 15) & ~size_t(15));
+    const size_t fixed = ((sizeof(SvOp) * n_gates + 15) & ~size_t(15)) + ((sizeof(SvPass3) * (n_passes + n_epi) + 15) & ~size_t(15));
     int warps = T::BLOCK ? T::SIZE / 32 : 4;
     if (!T::BLOCK) {
-        // CTA size that keeps the most warps resident under the shared-memory limit (four state copies per team)
+        // CTA size that keeps the most warps resident under the shared-memory limit
         int best = 0;
         for (int w = 4; w >= 1; --w) {
             const size_t bytes = fixed + team_bytes * w * T::PER_WARP + 1024;
@@ -1453,7 +1317,7 @@ static int launch_sv_lc2_impl(const dqgp_circuit* c, const double* X, int n, con
     const int teams = T::BLOCK ? 1 : warps * T::PER_WARP;
     const size_t smem = fixed + team_bytes * teams;
     if (smem > 227 * 1024) return 1;          // caller falls back to the one-fork kernel
-    auto kern = statevec_lc2_kernel<Q, PAIR, MAPPED>;
+    auto kern = statevec_lc2_kernel<Q>;
     DQGP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
     DQGP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, warps * 32, smem));
@@ -1462,27 +1326,10 @@ static int launch_sv_lc2_impl(const dqgp_circuit* c, const double* X, int n, con
     const long long cap = (long long)sm_count() * per_sm;
     if (blocks > cap) blocks = cap;
     if (blocks < 1) return 0;
-    const int pair_forks = getenv("DQGP_SV_NO_PAIR") == nullptr;
-    if constexpr (MAPPED)
-        kern<<<(unsigned)blocks, warps * 32, smem, st>>>(c->d_gates, n_gates, c->d_passes3, n_passes, c->d_ops3, c->d_mats3, n_mats, c->d_mat_gates3,
-                                                        c->d_share3, c->d, c->P, c->uses_acos ? 1 : 0, pair_forks, X, n, Pm, out);
-    else
-        kern<<<(unsigned)blocks, warps * 32, smem, st>>>(c->d_gates, n_gates, c->d_passes, n_passes, c->d_ops, c->d_mats, n_mats, c->d_mat_gates,
-                                                        c->d_share, c->d, c->P, c->uses_acos ? 1 : 0, pair_forks, X, n, Pm, out);
+    kern<<<(unsigned)blocks, warps * 32, smem, st>>>(c->d_gates, n_gates, c->d_passes3, n_passes, c->d_ops3, c->d_mats3, n_mats, c->d_mat_gates3,
+                                                    c->d_share3, c->d, c->P, c->uses_acos ? 1 : 0, X, n, Pm, out);
     DQGP_LAUNCH_CHECK("statevec_lc2_kernel");
     return 0;
-}
-
-template <int Q, bool MAPPED>
-static int launch_sv_lc2(const dqgp_circuit* c, const double* X, int n, const double* Pm, double* out, cudaStream_t st) {
-    if constexpr (SvTeam<Q>::BLOCK) {
-        // CTA per state: two forks per pass and three CTAs per SM, or (DQGP_SV_UNPAIRED, A/B) one fork and four CTAs per SM
-        if (getenv("DQGP_SV_UNPAIRED") != nullptr) return launch_sv_lc2_impl<Q, MAPPED, false>(c, X, n, Pm, out, st);
-        return launch_sv_lc2_impl<Q, MAPPED, true>(c, X, n, Pm, out, st);
-    } else {
-        if (getenv("DQGP_SV_PAIRED_SMALL") != nullptr) return launch_sv_lc2_impl<Q, MAPPED, true>(c, X, n, Pm, out, st);   // A/B only
-        return launch_sv_lc2_impl<Q, MAPPED, false>(c, X, n, Pm, out, st);
-    }
 }
 
 template <int Q, bool WANT_STATES>
@@ -1494,23 +1341,15 @@ static int launch_sv_shared(const dqgp_circuit* c, const double* X, int n, const
     const size_t fixed = ((sizeof(dqgp_gate) * n_gates + 15) & ~size_t(15)) + ((sizeof(SvPass) * n_passes + 15) & ~size_t(15)) +
                          ((sizeof(SvOp) * n_gates + 15) & ~size_t(15)) + ((sizeof(SvMat) * n_mats + sizeof(int) * n_mat_gates + 15) & ~size_t(15)) +
                          ((sizeof(int) * n_share + 15) & ~size_t(15));
-    // linear-combination form (statevec_lc_kernel) unless DQGP_SV_NO_LC is set (A/B checks against the two-fork kernel) or its
-    // third copy of the state does not fit in shared memory (q = 12 with a long gate list)
+    // linear-combination form (statevec_lc_kernel) unless its third copy of the state does not fit in shared memory (q = 12 with a long
+    // gate list) or DQGP_SV_NO_LC is set: a test hook, the only way to reach the two-fork kernel (statevec_shared_kernel) at small q
     bool use_lc = getenv("DQGP_SV_NO_LC") == nullptr;
-    // lc2 (fused epilogue, halving reductions; two forks per pass where a CTA owns the state) for circuits whose parameters all sit on
-    // rotations.  With the CX-free plan (no CRZ in the circuit: yz_cx, kyriienko) it is the default for every q: config 5's shard
-    // 60 -> 36 ms, config 4's 3.9 -> 3.1 ms.  Without that plan its larger code only pays for q >= 9 (one state per warp: instruction-fetch
-    // bound, 4.3 ms against 3.9), so the one-fork kernel below stays the default there (DQGP_SV_FORCE_LC2 overrides, for tests / A-B)
-    if (!WANT_STATES && Q >= 3 && use_lc && getenv("DQGP_SV_NO_LC2") == nullptr &&
-        (T::BLOCK || getenv("DQGP_SV_FORCE_LC2") != nullptr || (c->has_plan3 && getenv("DQGP_SV_NO_MAPPED") == nullptr))) {
-        bool all_rot = true;
-        for (int i = 0; i < c->P; ++i) all_rot = all_rot && c->par_mat[i] >= 0;
-        if (all_rot) {
-            // the CX-free plan when the circuit has one (no CRZ): CX gates cost nothing and the pass loop shrinks to fused 2x2 unitaries
-            const bool mapped = c->has_plan3 && getenv("DQGP_SV_NO_MAPPED") == nullptr;
-            const int rc = mapped ? launch_sv_lc2<(Q >= 3 ? Q : 3), true>(c, X, n, Pm, out, st) : launch_sv_lc2<(Q >= 3 ? Q : 3), false>(c, X, n, Pm, out, st);
-            if (rc <= 0) return rc;          // 1 = does not fit in shared memory: the one-fork kernel below
-        }
+    // lc2 (fused epilogue, halving reductions; two forks per pass where a CTA owns the state) for circuits with the CX-free plan (no CRZ
+    // in the circuit, so every parameter sits on a rotation: yz_cx, kyriienko): CX gates cost nothing and the pass loop shrinks to fused
+    // 2x2 unitaries.  Config 5's shard 60 -> 36 ms, config 4's 3.9 -> 3.1 ms.  Circuits with a CRZ take statevec_lc_kernel below.
+    if (!WANT_STATES && Q >= 3 && use_lc && c->has_plan3) {
+        const int rc = launch_sv_lc2<(Q >= 3 ? Q : 3)>(c, X, n, Pm, out, st);
+        if (rc <= 0) return rc;          // 1 = does not fit in shared memory: the one-fork kernel below
     }
     auto team_size = [&](bool lc) {
         return sizeof(double2) * ((lc ? 3 : 2) * T::DIM + n_gates + 4 * n_mats + 4 * T::SLOTS) +
@@ -1665,7 +1504,7 @@ static int dispatch_sv_shared(const dqgp_circuit* c, const double* X, int n, con
     // prefix sharing parallelises over samples only: with few samples (or a parameter feeding several gates) the
     // per-set kernel, which parallelises over samples x sets, fills the machine better
     const long long teams = c->q >= 9 ? n : (long long)n * (c->q > 3 ? (1 << (c->q - 3)) : 1) / 32;
-    // DQGP_SV_FORCE_SHARED: tests exercise the sharing kernels at small n
+    // DQGP_SV_FORCE_SHARED: a test hook that reaches the prefix-sharing kernels at small n
     if (!c->shareable || (teams < (c->q >= 9 ? 600 : 1200) && getenv("DQGP_SV_FORCE_SHARED") == nullptr))
         return WANT_STATES ? dqgp_states(c, X, n, Pm, 2 * P + 1, out, stream) : dqgp_features(c, X, n, Pm, 2 * P + 1, out, stream);
     int rc = circuit_on_device(c);

@@ -7,7 +7,7 @@ namespace dqgp {
 
 // A = [sets][n][inner] doubles (row stride inner * 8 bytes, a multiple of 16) as a 3-D tensor map whose box is (1, box_rows, box_inner).
 // box_inner may exceed `inner` and a box may hang over the last row: what lies outside the tensor arrives as zeros.
-// false when the driver entry point is missing or refuses the map (callers then keep their per-row bulk copies).
+// false when the driver entry point is missing or refuses the map.
 static inline bool make_rows_tensor_map(CUtensorMap* out, const double* base, int inner, int n, int sets, int box_inner, int box_rows) {
     typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
                                  const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);

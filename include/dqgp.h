@@ -13,8 +13,8 @@
  *   - return value: 0 = ok, <0 = error (dqgp_last_error() gives a thread-local message); nothing throws;
  *   - no global mutable state; handles are immutable after creation and may be shared by streams,
  *     except dqgp_solver (owns scratch and internal streams: one in-flight use at a time);
- *   - diagnostics read from the environment at call time: DQGP_POTRF_TRACE (time stamps of the Cholesky's leaf chain),
- *     DQGP_SV_NO_LC / DQGP_SV_FORCE_SHARED (simulator kernel selection), DQGP_GRAM_DIRECT, DQGP_FID_SIMT (v1 kernels);
+ *   - read from the environment at call time: DQGP_POTRF_TRACE (diagnostic: time stamps of the Cholesky's leaf chain);
+ *     DQGP_SV_NO_LC / DQGP_SV_FORCE_SHARED (test hooks: reach the two-fork / prefix-sharing simulator kernels at small sizes);
  *   - there is no CPU fallback anywhere in this library.
  */
 #ifndef DQGP_H
@@ -89,7 +89,8 @@ int dqgp_states_shifted(const dqgp_circuit* c, const double* d_X, int n, const d
  *      (FidelityKernel.evaluate, main.py:118-124). `same` != 0 promises the two operands are the same
  *      array so the diagonal is exactly outer(0) / the mirror is exact; `same` == 2 (projected kernel) writes
  *      only the 64x64 tiles that intersect the lower triangle - all dqgp_potrf_solve_inv reads - and leaves
- *      the rest of d_K untouched. */
+ *      the rest of d_K untouched.  Fidelity: dim = 2^q amplitudes with 1 <= q <= 12, and d_Psi1 / d_Psi2
+ *      16-byte aligned (anything else returns < 0). */
 int dqgp_gram_projected(int outer, const double* h_hyp, const double* d_F1, int n1, const double* d_F2, int n2, int m,
                         double* d_K, int ldk, int same, void* stream);
 int dqgp_gram_fidelity(const double* d_Psi1, int n1, const double* d_Psi2, int n2, int dim, double* d_K, int ldk,
@@ -176,7 +177,8 @@ int dqgp_shift_parameter_sets(const double* d_z, int P, double h, double period,
 /* ---- fused gradient: grad_i = 1/2 sum_jk (A^-1 - alpha alpha^T)_jk (K(p+h e_i) - K(p-h e_i))_kj / (2h)
  *      (agent_riemannian.py:270-275 and :431-436) without materialising any shifted Gram.
  *      d_F: (2P+1, n, m) features / d_Psi: (2P+1, n, dim) states of the sets in dqgp_shift_parameter_sets
- *      order; d_Ainv (n, ld).  d_work: dqgp_grad_workspace_bytes(n, P) bytes.  d_grad[P] is UNROUNDED. */
+ *      order; d_Ainv (n, ld).  d_work: dqgp_grad_workspace_bytes(n, P) bytes.  d_grad[P] is UNROUNDED.
+ *      Fidelity: dim = 2^q amplitudes with 1 <= q <= 12, and d_Psi 16-byte aligned (anything else returns < 0). */
 size_t dqgp_grad_workspace_bytes(int n, int P);
 int dqgp_grad_projected(int outer, const double* h_hyp, const double* d_Ainv, int ld, const double* d_alpha,
                         const double* d_F, int n, int m, int P, double h, double* d_grad, void* d_work, void* stream);

@@ -91,21 +91,9 @@ def test_shared_prefix_simulation_matches_per_set_kernels(d, enc, q, dd, layers,
             assert (F - F_ref).abs().max().item() < 2e-14
             assert (S - S_ref).abs().max().item() < 2e-14
             assert torch.equal(S[0], S_ref[0])                       # the base set is simulated directly
-            # ... and so are its features; the CX-free kernel (q >= 9 default) sums them through the final index map in another order
+            # ... and so are its features; the CX-free lc2 kernel (yz_cx, kyriienko: every q) sums them through the final index map
+            # in another order
             assert (F[0] - F_ref[0]).abs().max().item() < 5e-15
-    # statevec_lc2_kernel (two forks per pass, fused epilogue, CX gates folded into the load / store addresses): the default
-    # for q >= 9 when every parameter sits on a rotation; forced here for every q, with and without fork pairing
-    # and with / without the CX-free plan (CX gates absorbed into the logical -> physical index map, yz_cx and kyriienko)
-    for env in ({"DQGP_SV_FORCE_LC2": "1"}, {"DQGP_SV_FORCE_LC2": "1", "DQGP_SV_NO_PAIR": "1"}, {"DQGP_SV_FORCE_LC2": "1", "DQGP_SV_NO_MAPPED": "1"},
-                {"DQGP_SV_FORCE_LC2": "1", "DQGP_SV_NO_MAPPED": "1", "DQGP_SV_NO_PAIR": "1"}, {"DQGP_SV_NO_LC2": "1"}):
-        for k in ("DQGP_SV_FORCE_LC2", "DQGP_SV_NO_PAIR", "DQGP_SV_NO_LC2", "DQGP_SV_NO_MAPPED"):
-            monkeypatch.delenv(k, raising=False)
-        for k, v in env.items():
-            monkeypatch.setenv(k, v)
-        F = torch.full_like(F_ref, float("nan"))
-        assert lib.dqgp_features_shifted(ec.handle, dx.data_ptr(), n, dpm.data_ptr(), P, F.data_ptr(), _sp()) == 0, lib.dqgp_last_error()
-        torch.cuda.synchronize()
-        assert (F - F_ref).abs().max().item() < 2e-14, env
 
 
 def test_features_empty_and_single(d):
@@ -188,6 +176,29 @@ def test_dgemm_rejects_bad_shapes(d):
     lib = d.load()
     assert lib.dqgp_dgemm(1, 1, 100, 128, 16, 1.0, t.data_ptr(), 16, t.data_ptr(), 16, 0.0, t.data_ptr(), 128, _sp()) < 0
     assert b"multiples" in lib.dqgp_last_error()
+
+
+@pytest.mark.parametrize("dim,offset,message", [(3, 0, b"2^q"), (24, 0, b"2^q"), (8, 1, b"16-byte aligned")])
+def test_fidelity_entry_points_reject_unsupported_states(d, dim, offset, message):
+    """dqgp_gram_fidelity / dqgp_grad_fidelity take 2^q amplitudes (q >= 1) per state and 16-byte aligned state arrays: the DMMA
+    kernel splits every state into chunks of 4k doubles and copies them with the TMA engine.  Anything else is refused before a
+    launch, with a message."""
+    n, P = 5, 1
+    lib = d.load()
+    buf = torch.zeros((2 * P + 1) * n * 2 * dim + 1, dtype=torch.float64, device="cuda")
+    psi = buf[offset:offset + (2 * P + 1) * n * 2 * dim]
+    assert psi.data_ptr() % 16 == 8 * offset
+    K = torch.zeros((n, n), dtype=torch.float64, device="cuda")
+    ainv = torch.eye(n, dtype=torch.float64, device="cuda")
+    alpha = torch.zeros(n, dtype=torch.float64, device="cuda")
+    grad = torch.zeros(P, dtype=torch.float64, device="cuda")
+    work = torch.zeros(max(1, lib.dqgp_grad_workspace_bytes(n, P) // 8), dtype=torch.float64, device="cuda")
+    assert lib.dqgp_gram_fidelity(psi.data_ptr(), n, psi.data_ptr(), n, dim, K.data_ptr(), n, 1, _sp()) < 0
+    assert message in lib.dqgp_last_error()
+    assert lib.dqgp_grad_fidelity(ainv.data_ptr(), n, alpha.data_ptr(), psi.data_ptr(), n, dim, P, 0.1, grad.data_ptr(),
+                                  work.data_ptr(), _sp()) < 0
+    assert message in lib.dqgp_last_error()
+    torch.cuda.synchronize()
 
 
 @pytest.mark.parametrize("n", [1, 5, 127, 128, 129, 300, 640, 1100])
@@ -446,10 +457,12 @@ def test_fused_gradient_honoured_outer_kernels_match_oracle(d, outer, enc, q, dd
 @pytest.mark.parametrize("enc,ktype,q,dd,layers,n,outer", [("yz_cx", "projected", 8, 4, 3, 333, "gaussian"), ("kyriienko", "projected", 10, 6, 2, 200, "matern"),
                                                           ("yz_cx", "projected", 5, 3, 2, 64, "expsinesquared"), ("hubregtsen", "fidelity", 5, 2, 2, 333, "gaussian"),
                                                           ("chebyshev", "fidelity", 2, 2, 1, 97, "gaussian")])
-def test_gradient_staging_paths_agree_bit_for_bit(d, monkeypatch, enc, ktype, q, dd, layers, n, outer):
-    """The fused gradients stage their tiles through a 3-D tensor map (TMA, the default), through one bulk copy per row
-    (DQGP_*_NO_TMAP) or through per-thread cp.async (DQGP_GRAD_NO_BULK): same arithmetic on the same operands, so the gradients must
-    be identical to the last bit - at ragged n, where the tensor map zero-fills the rows past n and the other paths clamp them."""
+def test_gradient_staging_paths_agree_bit_for_bit(d, enc, ktype, q, dd, layers, n, outer):
+    """The fused projected gradient stages its feature tiles through a 3-D tensor map (TMA: even m, 16-byte aligned features) or
+    through per-thread cp.async (any other features): same arithmetic on the same operands, so the gradients must be identical to the
+    last bit - at ragged n, where the tensor map zero-fills the rows past n and cp.async clamps them.  The fused fidelity gradient has
+    one staging path (the tensor map); it is checked against the central difference assembled from the per-set Grams, whose tiles
+    arrive as one bulk copy per row."""
     x, y = d.synthetic_dataset(n, dd, enc, seed=3)
     eng = d.AgentEngine(x, y, encoding_type=enc, kernel_type=ktype, num_qubits=q, num_layers=layers, noise_std=0.1, rho=100.0, L=100.0,
                         outer_kernel=outer, training_ignores_outer_kernel=False)
@@ -457,22 +470,37 @@ def test_gradient_staging_paths_agree_bit_for_bit(d, monkeypatch, enc, ktype, q,
     eng.simulate(z); eng.gram(full=True)
     rs = np.random.RandomState(2)                       # any symmetric "inverse" and alpha will do: the contraction is what is compared
     b = rs.randn(n, n)
-    eng.solver.inverse()[:n, :n].copy_(torch.from_numpy(b + b.T).cuda())
-    eng.d_alpha.copy_(torch.from_numpy(rs.randn(n)).cuda())
-    grads = {}
-    for name, env in (("tensor map", {}), ("bulk rows", {"DQGP_GRAD_NO_TMAP": "1", "DQGP_FID_NO_TMAP": "1"}),
-                      ("cp.async", {"DQGP_GRAD_NO_TMAP": "1", "DQGP_FID_NO_TMAP": "1", "DQGP_GRAD_NO_BULK": "1"})):
-        for k in ("DQGP_GRAD_NO_TMAP", "DQGP_FID_NO_TMAP", "DQGP_GRAD_NO_BULK"):
-            monkeypatch.delenv(k, raising=False)
-        for k, v in env.items():
-            monkeypatch.setenv(k, v)
-        eng.d_grad.zero_()
-        eng.gradient()
+    ainv, alpha = b + b.T, rs.randn(n)
+    eng.solver.inverse()[:n, :n].copy_(torch.from_numpy(ainv).cuda())
+    eng.d_alpha.copy_(torch.from_numpy(alpha).cuda())
+    eng.d_grad.zero_()
+    eng.gradient()
+    torch.cuda.synchronize()
+    got = eng.d_grad.cpu().numpy().copy()
+    assert np.all(np.isfinite(got)) and np.abs(got).max() > 0
+    lib, s = d.load(), eng.solver
+    if ktype == "projected":
+        # the same features at an 8-byte offset: not 16-byte aligned, so the cp.async kernel
+        buf = torch.empty(eng.d_feat.numel() + 1, dtype=torch.float64, device="cuda")
+        feat = buf[1:].view(eng.d_feat.shape)
+        feat.copy_(eng.d_feat)
+        assert feat.data_ptr() % 16 == 8
+        grad = torch.zeros_like(eng.d_grad)
+        assert lib.dqgp_grad_projected(eng._outer_id, eng._hyp, s.inverse_ptr, s.ld, eng.d_alpha.data_ptr(), feat.data_ptr(), n, eng.m,
+                                       eng.P, eng.h, grad.data_ptr(), eng.d_work.data_ptr(), _sp()) == 0, lib.dqgp_last_error()
         torch.cuda.synchronize()
-        grads[name] = eng.d_grad.cpu().numpy().copy()
-    assert np.all(np.isfinite(grads["tensor map"])) and np.abs(grads["tensor map"]).max() > 0
-    assert np.array_equal(grads["tensor map"], grads["bulk rows"])
-    assert np.array_equal(grads["tensor map"], grads["cp.async"])
+        assert np.array_equal(got, grad.cpu().numpy())
+    else:
+        dim = 1 << q
+        K = torch.empty((eng.S, n, n), dtype=torch.float64, device="cuda")
+        for st in range(eng.S):
+            f = eng.d_feat[st].data_ptr()
+            assert lib.dqgp_gram_fidelity(f, n, f, n, dim, K[st].data_ptr(), n, 1, _sp()) == 0, lib.dqgp_last_error()
+        torch.cuda.synchronize()
+        K = K.cpu().numpy()
+        bracket = ainv - np.outer(alpha, alpha)
+        ref = np.array([0.5 * np.sum(bracket * (K[1 + 2 * i] - K[2 + 2 * i])) / (2.0 * eng.h) for i in range(eng.P)])
+        assert np.max(np.abs(got - ref)) <= 1e-12 * np.abs(ref).max()
 
 
 @pytest.mark.parametrize("n", [1, 5, 33, 64, 100, 257, 700])

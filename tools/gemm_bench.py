@@ -1,7 +1,7 @@
 """Throughput of the DMMA GEMM building block (dqgp_dgemm) against the measured FP64 peak.  Usage: python tools/gemm_bench.py
 
 The test utility builds and frees the two tensor maps of its one task on every call (cudaMalloc / cudaFree): at K = 8192 that is
-noise, at K <= 256 it dominates - use DQGP_GEMM_NO_TMAP=1 for kernel rates of the small-K shapes, or time a factorisation
+noise, at K <= 256 it dominates - for kernel rates of the small-K shapes, time a factorisation
 (tools/factor_breakdown.py), where the maps are built once per solver."""
 import ctypes as C
 import os
