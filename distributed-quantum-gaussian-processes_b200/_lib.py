@@ -22,7 +22,8 @@ class Gate(C.Structure):
 
 
 ENCODINGS = {"chebyshev": 0, "hubregtsen": 1, "yz_cx": 2, "kyriienko": 3}
-OUTER_KERNELS = {"gaussian": 0, "matern": 1, "expsinesquared": 2}
+# pairwisekernel = PairwiseKernel(metric="linear") = f.g, the dot product with sigma_0 = 0 (kernels.outer_hyp)
+OUTER_KERNELS = {"gaussian": 0, "matern": 1, "expsinesquared": 2, "rationalquadratic": 3, "dotproduct": 4, "pairwisekernel": 4}
 
 _vp, _i, _d, _sz = C.c_void_p, C.c_int, C.c_double, C.c_size_t
 _dp = C.POINTER(C.c_double)
@@ -46,6 +47,7 @@ SIGNATURES = {
     "dqgp_states_shifted": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp]),
     "dqgp_gram_projected": (_i, [_i, _dp, _vp, _i, _vp, _i, _i, _vp, _i, _i, _vp]),
     "dqgp_gram_fidelity": (_i, [_vp, _i, _vp, _i, _i, _vp, _i, _i, _vp]),
+    "dqgp_projected_self_kernel": (_i, [_i, _dp, _vp, _i, _i, _vp, _vp]),
     "dqgp_solver_create": (_i, [_i, C.POINTER(_vp)]),
     "dqgp_solver_create_ex": (_i, [_i, _i, C.POINTER(_vp)]),
     "dqgp_solver_create_lean": (_i, [_i, _i, C.POINTER(_vp)]),

@@ -98,8 +98,9 @@ __global__ void __launch_bounds__(PW_THREADS, 2) grad_projected_dmma_kernel(cons
         if (threadIdx.x == 0) { mbar_init(&s_bar[0], 1); mbar_init(&s_bar[1], 1); mbar_fence_init(); }
         __syncthreads();
     }
+    constexpr bool STAT = outer_is_stationary(OUTER);
     const double gam = (OUTER == DQGP_OUTER_GAUSSIAN) ? hyp.a * DQGP_EXP_S32 : 1.0;      // Gaussian: argument in units of ln2/32
-    const double a_scale = 2.0 * gam;
+    const double a_scale = STAT ? 2.0 * gam : 1.0;                                      // dot product: sigma_0^2 + f.g
     const double tab = exp_table_entry();
 
     // zero the k-padding columns of both stages once (cp.async never writes them; the tensor map's boxes bring their own zeros)
@@ -110,7 +111,8 @@ __global__ void __launch_bounds__(PW_THREADS, 2) grad_projected_dmma_kernel(cons
         g2_smem[stage * G2_STAGE_DOUBLES + rr * PITCH + k] = 0.0;
     }
 
-    // B = weight * (A^-1 - alpha alpha^T) for this lane's 16 entries; zero outside the matrix and on the diagonal
+    // B = weight * (A^-1 - alpha alpha^T) for this lane's 16 entries; zero outside the matrix, and on the diagonal where k(f, f) = 1
+    // does not depend on the parameters (the dot product's sigma_0^2 + |f|^2 does)
     double br[2][4][2];
     const double weight = (bi == bj) ? 1.0 : 2.0;
 #pragma unroll
@@ -122,7 +124,7 @@ __global__ void __launch_bounds__(PW_THREADS, 2) grad_projected_dmma_kernel(cons
             const int c = col0 + wc * 32 + cb * 8 + 2 * t;
 #pragma unroll
             for (int e = 0; e < 2; ++e)
-                br[rb][cb][e] = (r < n && c + e < n && r != c + e) ? weight * (Ainv[(size_t)r * ld + c + e] - ar * alpha[c + e]) : 0.0;
+                br[rb][cb][e] = (r < n && c + e < n && (!STAT || r != c + e)) ? weight * (Ainv[(size_t)r * ld + c + e] - ar * alpha[c + e]) : 0.0;
         }
     }
 
@@ -159,7 +161,7 @@ __global__ void __launch_bounds__(PW_THREADS, 2) grad_projected_dmma_kernel(cons
         const double* nr = buf + 2 * PW_TILE * PITCH;
         double c[2][4][2];
         {
-            const double n0 = nr[wr * 16 + g], n1 = nr[wr * 16 + 8 + g];            // already -gamma_eff |f|^2
+            const double n0 = nr[wr * 16 + g], n1 = nr[wr * 16 + 8 + g];            // already -gamma_eff |f|^2 (dot product: sigma_0^2 / 2)
 #pragma unroll
             for (int cb = 0; cb < 4; ++cb) {
                 const double2 nc = *reinterpret_cast<const double2*>(&nr[PW_TILE + wc * 32 + cb * 8 + 2 * t]);
@@ -387,9 +389,11 @@ int dqgp_grad_projected(int outer, const double* h_hyp, const double* d_Ainv, in
     double* norms = partial + (size_t)tiles * P;
     const long long rows = (long long)(2 * P + 1) * n;
     // the norms arrive pre-multiplied by -gamma_eff (and, Gaussian, by 32/ln2: the exponent's argument then leaves the DMMA in the
-    // units its range reduction wants): the kernel only adds them
+    // units its range reduction wants): the kernel only adds them.  The dot product's "norms" are sigma_0^2 / 2 each, so the
+    // accumulator starts at exactly sigma_0^2.
     const double gam_eff = (outer == DQGP_OUTER_GAUSSIAN) ? hyp.a * DQGP_EXP_S32 : 1.0;
-    feature_norms_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(d_F, rows, m, -gam_eff, norms);
+    if (outer_is_stationary(outer)) feature_norms_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(d_F, rows, m, -gam_eff, norms);
+    else launch_self_kernel(nullptr, rows, m, 0.5 * hyp.a, false, norms, st);
     // Pauli features lie in [-1, 1]: gamma d^2 <= 4 m gamma, so the exponent guard is only needed for large gamma
     // the exponent's argument is bounded below by -gamma 4m (Gaussian), -sqrt(3) 2 sqrt(m) / l (Matern), -2 / l^2 (ExpSineSquared)
     const double worst = outer == DQGP_OUTER_GAUSSIAN ? 4.0 * m * hyp.a
@@ -418,11 +422,29 @@ int dqgp_grad_projected(int outer, const double* h_hyp, const double* d_Ainv, in
         else if (have_tmap) grad_projected_dmma_kernel<OUT, true, true><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
         else grad_projected_dmma_kernel<OUT, true, false><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
     } while (0)
+    // RationalQuadratic and DotProduct have no exponent to guard: only their CLAMP = false kernels exist, one per staging path
+#define DQGP_G2_NOEXP(OUT)                                                                                                   \
+    do {                                                                                                                     \
+        static bool attr_done_dev[64] = {false};                                                                             \
+        int dev_ = 0;                                                                                                        \
+        cudaGetDevice(&dev_);                                                                                                \
+        bool& attr_done = attr_done_dev[(dev_ >= 0 && dev_ < 64) ? dev_ : 0];                                                \
+        if (!attr_done) {                                                                                                    \
+            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
+            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
+            attr_done = true;                                                                                                \
+        }                                                                                                                    \
+        if (have_tmap) grad_projected_dmma_kernel<OUT, false, true><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
+        else grad_projected_dmma_kernel<OUT, false, false><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
+    } while (0)
     switch (outer) {
         case DQGP_OUTER_GAUSSIAN: DQGP_G2(DQGP_OUTER_GAUSSIAN); break;
         case DQGP_OUTER_MATERN15: DQGP_G2(DQGP_OUTER_MATERN15); break;
+        case DQGP_OUTER_RATQUAD: DQGP_G2_NOEXP(DQGP_OUTER_RATQUAD); break;
+        case DQGP_OUTER_DOTPRODUCT: DQGP_G2_NOEXP(DQGP_OUTER_DOTPRODUCT); break;
         default: DQGP_G2(DQGP_OUTER_EXPSINE2); break;
     }
+#undef DQGP_G2_NOEXP
 #undef DQGP_G2
     DQGP_LAUNCH_CHECK("grad_projected_dmma_kernel");
     grad_reduce_kernel<<<P, 256, 0, st>>>(partial, tiles, P, 0.5 / (2.0 * h), d_grad);

@@ -10,7 +10,8 @@ namespace dqgp {
 // Gram identity on DMMA.8x8x4, 11-instruction table exp, 16-byte stores.  SYM: only lower 64x64 tiles are computed
 // and each is stored twice (K and K^T; the transposed stores still fill whole 32-byte sectors), the diagonal is
 // exactly outer(0).  d^2 below 4e-15*(|f|^2+|g|^2) snaps to 0 so exact duplicates give exactly outer(0) = 1, as
-// direct differences and SciPy's cdist do.
+// direct differences and SciPy's cdist do.  The dot product (not stationary) starts the accumulator at sigma_0^2 and stores
+// sigma_0^2 + f.g as it leaves the DMMA: no snap, and its diagonal is sigma_0^2 + |f|^2.
 // v1 (direct differences, libm exp; since removed) ran at 22% of the HBM write roofline: 72 FP64 instructions per entry.
 template <int OUTER, int SYM>   // 0 rectangular, 1 lower tiles + mirror, 2 lower tiles only (what the factorisation reads)
 __global__ void __launch_bounds__(PW_THREADS) gram_projected_dmma_kernel(const double* __restrict__ F1, int n1,
@@ -48,8 +49,9 @@ __global__ void __launch_bounds__(PW_THREADS) gram_projected_dmma_kernel(const d
     __syncthreads();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int wr = warp >> 1, wc = warp & 1, g = lane >> 2, t = lane & 3;
+    constexpr bool STAT = outer_is_stationary(OUTER);
     const double gam = (OUTER == DQGP_OUTER_GAUSSIAN) ? hyp.a : 1.0;
-    const double a_scale = 2.0 * gam;
+    const double a_scale = STAT ? 2.0 * gam : 1.0;                          // dot product: f.g, unscaled
     const double tab = exp_table_entry();
     const double* fr = Fr + (wr * 16 + g) * G2_PITCH + t;
     const double* fc = Fc + (wc * 32 + g) * G2_PITCH + t;
@@ -59,8 +61,12 @@ __global__ void __launch_bounds__(PW_THREADS) gram_projected_dmma_kernel(const d
 #pragma unroll
         for (int cb = 0; cb < 4; ++cb) {
             const double2 nc = *reinterpret_cast<const double2*>(&nr[PW_TILE + wc * 32 + cb * 8 + 2 * t]);
-            c[0][cb][0] = -gam * (n0 + nc.x); c[0][cb][1] = -gam * (n0 + nc.y);
-            c[1][cb][0] = -gam * (n1s + nc.x); c[1][cb][1] = -gam * (n1s + nc.y);
+            if (STAT) {
+                c[0][cb][0] = -gam * (n0 + nc.x); c[0][cb][1] = -gam * (n0 + nc.y);
+                c[1][cb][0] = -gam * (n1s + nc.x); c[1][cb][1] = -gam * (n1s + nc.y);
+            } else {                                                          // sigma_0^2 + f.g
+                c[0][cb][0] = c[0][cb][1] = c[1][cb][0] = c[1][cb][1] = hyp.a;
+            }
 #pragma unroll
             for (int rb = 0; rb < 2; ++rb)
 #pragma unroll
@@ -89,11 +95,14 @@ __global__ void __launch_bounds__(PW_THREADS) gram_projected_dmma_kernel(const d
 #pragma unroll
             for (int e = 0; e < 2; ++e) {
                 double x = c[rb][cb][e];
-                x = (x > snap[rb][cb][e]) ? 0.0 : x;                 // |gamma d^2| below rounding level (or negative d^2) -> 0
-                if (SYM && r == cc + e) x = 0.0;
+                if (STAT) {
+                    x = (x > snap[rb][cb][e]) ? 0.0 : x;             // |gamma d^2| below rounding level (or negative d^2) -> 0
+                    if (SYM && r == cc + e) x = 0.0;
+                }
                 v[e] = outer_from_neg_gd2<OUTER>(x, hyp, tab);
-                // NaN features (arccos outside [-1,1]) must propagate as in NumPy: the clamps above would swallow them
-                if (snap[rb][cb][e] != snap[rb][cb][e]) v[e] = snap[rb][cb][e];
+                // NaN features (arccos outside [-1,1]) must propagate as in NumPy: the clamps above would swallow them (the dot
+                // product has none: a NaN feature makes the DMMA sum NaN)
+                if (STAT && snap[rb][cb][e] != snap[rb][cb][e]) v[e] = snap[rb][cb][e];
             }
             if (r < n1) {
                 double* dst = K + (size_t)r * ldk + cc;
@@ -106,6 +115,22 @@ __global__ void __launch_bounds__(PW_THREADS) gram_projected_dmma_kernel(const d
             }
         }
     }
+}
+
+// out[row] = add (+ |f_row|^2 when with_norm): the projected kernel's k(f, f), and the dot product's norm buffer of the fused gradient
+__global__ void self_kernel_kernel(const double* __restrict__ F, long long rows, int m, double add, int with_norm, double* __restrict__ out) {
+    const long long row = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= rows) return;
+    double acc = 0.0;
+    if (with_norm) {
+        const double* f = F + row * m;
+        for (int k = 0; k < m; ++k) acc = fma(f[k], f[k], acc);
+    }
+    out[row] = with_norm ? acc + add : add;
+}
+
+void launch_self_kernel(const double* F, long long rows, int m, double add, bool with_norm, double* out, cudaStream_t st) {
+    self_kernel_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(F, rows, m, add, with_norm ? 1 : 0, out);
 }
 
 __global__ void add_diagonal_kernel(double* A, int n, int lda, double v) {
@@ -140,10 +165,25 @@ int dqgp_gram_projected(int outer, const double* h_hyp, const double* d_F1, int 
     switch (outer) {
         case DQGP_OUTER_GAUSSIAN: DQGP_GRAM(DQGP_OUTER_GAUSSIAN); break;
         case DQGP_OUTER_MATERN15: DQGP_GRAM(DQGP_OUTER_MATERN15); break;
+        case DQGP_OUTER_RATQUAD: DQGP_GRAM(DQGP_OUTER_RATQUAD); break;
+        case DQGP_OUTER_DOTPRODUCT: DQGP_GRAM(DQGP_OUTER_DOTPRODUCT); break;
         default: DQGP_GRAM(DQGP_OUTER_EXPSINE2); break;
     }
 #undef DQGP_GRAM
     DQGP_LAUNCH_CHECK("gram_projected_dmma_kernel");
+    return 0;
+}
+
+int dqgp_projected_self_kernel(int outer, const double* h_hyp, const double* d_F, int n, int m, double* d_out, void* stream) {
+    using namespace dqgp;
+    DQGP_REQUIRE(n >= 0 && m >= 1 && m <= PW_MAX_M, "dqgp_projected_self_kernel: bad shape (%d, %d)", n, m);
+    OuterHyp hyp;
+    if (make_outer_hyp(outer, h_hyp, &hyp)) return -1;
+    if (n == 0) return 0;
+    const bool dot = !outer_is_stationary(outer);
+    DQGP_REQUIRE(d_out && (d_F || !dot), "dqgp_projected_self_kernel: NULL argument");
+    launch_self_kernel(d_F, n, m, dot ? hyp.a : 1.0, dot, d_out, as_stream(stream));
+    DQGP_LAUNCH_CHECK("self_kernel_kernel");
     return 0;
 }
 

@@ -13,9 +13,12 @@ constexpr int PW_THREADS = 256;
 constexpr int PW_MAX_M = 3 * MAX_QUBITS;
 
 struct OuterHyp {
-    double a;   // gaussian: gamma        | matern: 1/length_scale | expsine2: 1/length_scale
-    double b;   //                                                  | expsine2: pi/periodicity
+    double a;   // gaussian: gamma        | matern: 1/length_scale | expsine2: 1/length_scale   | ratquad: 1/(2 alpha l^2) | dot: sigma_0^2
+    double b;   //                                                  | expsine2: pi/periodicity   | ratquad: alpha
 };
+
+// the dot product is the one outer kernel that is not a function of f - g: no snap to zero, no diagonal override, B keeps its diagonal
+__host__ __device__ constexpr bool outer_is_stationary(int outer) { return outer != DQGP_OUTER_DOTPRODUCT; }
 
 static inline int make_outer_hyp(int outer, const double* h_hyp, OuterHyp* out) {
     const double pi = 3.14159265358979323846;
@@ -36,14 +39,43 @@ static inline int make_outer_hyp(int outer, const double* h_hyp, OuterHyp* out) 
             out->a = 1.0 / l; out->b = pi / per;
             return 0;
         }
+        case DQGP_OUTER_RATQUAD: {
+            const double l = h_hyp ? h_hyp[0] : 1.0, alpha = h_hyp ? h_hyp[1] : 1.0;
+            DQGP_REQUIRE(l > 0 && alpha > 0, "rationalquadratic outer kernel: length_scale and alpha must be > 0");
+            out->a = 1.0 / (2.0 * alpha * l * l); out->b = alpha;
+            return 0;
+        }
+        case DQGP_OUTER_DOTPRODUCT: {
+            const double s0 = h_hyp ? h_hyp[0] : 1.0;
+            DQGP_REQUIRE(s0 >= 0, "dotproduct outer kernel: sigma_0 must be >= 0");
+            out->a = s0 * s0; out->b = 0.0;
+            return 0;
+        }
     }
-    set_error("unknown outer kernel id %d (hot path covers gaussian, matern, expsinesquared)", outer);
+    set_error("unknown outer kernel id %d (hot path covers gaussian, matern, expsinesquared, rationalquadratic, dotproduct)", outer);
     return -1;
+}
+
+// 1/x from the MUFU.RCP64H seed and one cubic Newton step y (1 + e + e^2), e = 1 - x y: 3 DFMA, no range branch.  Meant for
+// x >= 1 (the rational quadratic's base): the seed's ~20 bits become ~60 before rounding, and x = 1 gives exactly 1.
+__device__ __forceinline__ double fast_rcp_ge1(double x) {
+    double y;
+    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(x));
+    const double e = fma(-x, y, 1.0);
+    return fma(y, fma(e, e, e), y);
+}
+
+// RationalQuadratic (1 + d^2 / (2 alpha l^2))^-alpha from v = -d^2: a reciprocal at alpha = 1 (the only value the reference
+// reaches, Q2), exp(-alpha log(base)) otherwise (uniform branch on a kernel argument)
+__device__ __forceinline__ double ratquad_from_neg_d2(double v, const OuterHyp& h) {
+    const double base = fma(-v, h.a, 1.0);
+    return h.b == 1.0 ? fast_rcp_ge1(base) : exp(-h.b * log(base));
 }
 
 // Outer kernel from v = -gamma_eff * d^2 (gamma_eff = gamma for the Gaussian, 1 otherwise), as left in a DMMA
 // accumulator by the Gram identity, with scikit-learn's formulas (sklearn/gaussian_process/kernels.py RBF /
-// Matern(nu=1.5) / ExpSineSquared, as used by squlearn's ProjectedQuantumKernel; reference main.py:130-137).
+// Matern(nu=1.5) / ExpSineSquared / RationalQuadratic, as used by squlearn's ProjectedQuantumKernel; reference main.py:130-137).
+// The dot product's accumulator already holds sigma_0^2 + f.g, which passes through.
 // Warp-collective: fast_exp_tab shuffles its table.
 template <int OUTER>
 __device__ __forceinline__ double outer_from_neg_gd2(double v, const OuterHyp& h, double tab) {
@@ -53,6 +85,10 @@ __device__ __forceinline__ double outer_from_neg_gd2(double v, const OuterHyp& h
     } else if (OUTER == DQGP_OUTER_MATERN15) {
         const double k = sqrt(fmax(-v, 0.0)) * h.a * 1.7320508075688772;
         return (1.0 + k) * fast_exp_tab(fmax(-k, -700.0), tab);
+    } else if (OUTER == DQGP_OUTER_RATQUAD) {
+        return ratquad_from_neg_d2(v, h);
+    } else if (OUTER == DQGP_OUTER_DOTPRODUCT) {
+        return v;
     } else {
         const double sn = sin(sqrt(fmax(-v, 0.0)) * h.b) * h.a;
         return fast_exp_tab(fmax(-2.0 * (sn * sn), -700.0), tab);
@@ -79,6 +115,7 @@ __device__ __forceinline__ double fast_sqrt_guarded(double x) {
 // The fused gradient's outer kernel from v = -gamma_eff d^2: same formulas as outer_from_neg_gd2, built for the FP64 pipe that
 // bounds grad_projected_dmma_kernel: branch-free sqrt (above), degree-5 table exp (10 instructions), (1 + k) e^-k as one FMA,
 // and no exponent clamp when the host has shown the argument cannot go below -700 (CLAMP = false; features lie in [-1, 1]).
+// RationalQuadratic and DotProduct have no exponent (CLAMP is always false for them).
 template <int OUTER, bool CLAMP>
 __device__ __forceinline__ double outer_grad_from_neg_gd2(double v, const OuterHyp& h, double tab) {
     if (OUTER == DQGP_OUTER_GAUSSIAN) {
@@ -88,12 +125,19 @@ __device__ __forceinline__ double outer_grad_from_neg_gd2(double v, const OuterH
         const double nk = fast_sqrt_guarded(-v) * (-1.7320508075688772 * h.a);      // -sqrt(3) d / l
         const double e = fast_exp_tab5(CLAMP ? fmax(nk, -700.0) : nk, tab);
         return fma(-nk, e, e);
+    } else if (OUTER == DQGP_OUTER_RATQUAD) {
+        return ratquad_from_neg_d2(v, h);
+    } else if (OUTER == DQGP_OUTER_DOTPRODUCT) {
+        return v;
     } else {
         const double sn = sin(fast_sqrt_guarded(-v) * h.b) * h.a;
         const double x = -2.0 * (sn * sn);
         return fast_exp_tab5(CLAMP ? fmax(x, -700.0) : x, tab);
     }
 }
+
+// out[row] = add (+ |F[row]|^2 when with_norm), rows of m features (gram.cu)
+void launch_self_kernel(const double* F, long long rows, int m, double add, bool with_norm, double* out, cudaStream_t st);
 
 // DMMA fidelity kernels (fid.cu)
 int fidelity_gram_dmma(const double* Psi1, int n1, const double* Psi2, int n2, int dim, double* K, int ldk, cudaStream_t st);

@@ -88,7 +88,9 @@ class Executor:
 
 def outer_hyp(outer_kernel, params=None):
     """Host hyper-parameter vector of an outer kernel: gaussian {gamma}; matern {length_scale} (nu = 1.5);
-    expsinesquared {length_scale, periodicity}.  Defaults = the only values the reference reaches (Q2)."""
+    expsinesquared {length_scale, periodicity}; rationalquadratic {length_scale, alpha}; dotproduct {sigma_0};
+    pairwisekernel {0.0}: scikit-learn's PairwiseKernel(metric="linear") is f.g, the dot product with sigma_0 = 0 (its
+    gamma is accepted and ignored, as filter_params=True does).  Defaults = the only values the reference reaches (Q2)."""
     params = dict(params or {})
     if outer_kernel == "gaussian":
         return [float(params.get("gamma", 1.0))]
@@ -98,6 +100,14 @@ def outer_hyp(outer_kernel, params=None):
         return [float(params.get("length_scale", 1.0))]
     if outer_kernel == "expsinesquared":
         return [float(params.get("length_scale", 1.0)), float(params.get("periodicity", 1.0))]
+    if outer_kernel == "rationalquadratic":
+        return [float(params.get("length_scale", 1.0)), float(params.get("alpha", 1.0))]
+    if outer_kernel == "dotproduct":
+        return [float(params.get("sigma_0", 1.0))]
+    if outer_kernel == "pairwisekernel":
+        if params.get("metric", "linear") != "linear":
+            raise ValueError(f"only PairwiseKernel metric='linear' is on the hot path (got {params['metric']!r})")
+        return [0.0]
     raise ValueError(f"outer kernel {outer_kernel!r} is outside the hot path (supported: {sorted(OUTER_KERNELS)})")
 
 

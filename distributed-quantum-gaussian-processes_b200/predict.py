@@ -120,10 +120,17 @@ predict_quantum_gp.used_lu_fallback = False
 
 
 def _self_kernel_diag(qk, d_x, d_p):
-    """k(x_i, x_i) for every row: exactly outer(0) = 1 for the projected kernels; |<psi|psi>|^2 for fidelity."""
+    """k(x_i, x_i) for every row: outer(f_i, f_i) for the projected kernels (exactly 1 for the stationary ones, sigma_0^2 + |f_i|^2
+    for the dot product); |<psi|psi>|^2 for fidelity."""
     nt = d_x.shape[0]
     if hasattr(qk, "outer_kernel"):
-        return torch.ones(nt, dtype=torch.float64, device=d_x.device)
+        out = torch.empty(nt, dtype=torch.float64, device=d_x.device)
+        outer_id, m = _lib.OUTER_KERNELS[qk.outer_kernel], 3 * qk.encoding_circuit.num_qubits
+        # only the dot product reads the features (the stationary kernels' k(f, f) is 1 whatever f is)
+        f = qk.encoding_circuit.features(d_x, d_p) if outer_id == _lib.OUTER_KERNELS["dotproduct"] else None     # (1, nt, 3q)
+        check(_lib.load().dqgp_projected_self_kernel(outer_id, _lib.hyp_array(qk._hyp), f.data_ptr() if f is not None else None, nt, m,
+                                                     out.data_ptr(), stream_ptr()), "dqgp_projected_self_kernel")
+        return out
     s = qk.encoding_circuit.states(d_x, d_p)[0]           # (nt, dim, 2)
     nrm = (s * s).sum(dim=(1, 2))
     return nrm * nrm

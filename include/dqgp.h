@@ -31,8 +31,9 @@ extern "C" {
 
 /* encoding circuits (reference ctor sites main.py:68-83, agent_riemannian.py:51-66) */
 enum { DQGP_CHEBYSHEV = 0, DQGP_HUBREGTSEN = 1, DQGP_YZ_CX = 2, DQGP_KYRIIENKO = 3 };
-/* outer kernels of the projected kernel (main.py:130-137; sklearn RBF / Matern(1.5) / ExpSineSquared) */
-enum { DQGP_OUTER_GAUSSIAN = 0, DQGP_OUTER_MATERN15 = 1, DQGP_OUTER_EXPSINE2 = 2 };
+/* outer kernels of the projected kernel (main.py:130-137, --outer-kernel main.py:1996-2013; sklearn RBF / Matern(1.5) /
+ * ExpSineSquared / RationalQuadratic / DotProduct).  PairwiseKernel(metric="linear") is DOTPRODUCT with sigma_0 = 0. */
+enum { DQGP_OUTER_GAUSSIAN = 0, DQGP_OUTER_MATERN15 = 1, DQGP_OUTER_EXPSINE2 = 2, DQGP_OUTER_RATQUAD = 3, DQGP_OUTER_DOTPRODUCT = 4 };
 /* gate kinds / angle forms of the gate program (dqgp_circuit_describe) */
 enum { DQGP_G_H = 0, DQGP_G_RX = 1, DQGP_G_RY = 2, DQGP_G_RZ = 3, DQGP_G_CX = 4, DQGP_G_CRZ = 5 };
 enum { DQGP_A_NONE = 0, DQGP_A_P = 1, DQGP_A_X = 2, DQGP_A_P_PLUS_CX = 3, DQGP_A_P_TIMES_ACOS = 4, DQGP_A_C_TIMES_ACOS = 5 };
@@ -84,10 +85,11 @@ int dqgp_features_shifted(const dqgp_circuit* c, const double* d_X, int n, const
 int dqgp_states_shifted(const dqgp_circuit* c, const double* d_X, int n, const double* d_Pm, int P, double* d_Psi, void* stream);
 
 /* ---- Gram matrices.  d_K (n1,n2) with leading dimension ldk (>= n2).
- *      projected: K = outer(f1_j, f2_k); hyp = {gamma} | {length_scale} | {length_scale, periodicity}
- *      (ProjectedQuantumKernel.evaluate, main.py:130-137);  fidelity: K = |<psi2_k|psi1_j>|^2
- *      (FidelityKernel.evaluate, main.py:118-124). `same` != 0 promises the two operands are the same
- *      array so the diagonal is exactly outer(0) / the mirror is exact; `same` == 2 (projected kernel) writes
+ *      projected: K = outer(f1_j, f2_k); hyp = {gamma} | {length_scale} | {length_scale, periodicity} |
+ *      {length_scale, alpha} | {sigma_0} (NULL = all 1; ids as DQGP_OUTER_*) (ProjectedQuantumKernel.evaluate, main.py:130-137);
+ *      fidelity: K = |<psi2_k|psi1_j>|^2 (FidelityKernel.evaluate, main.py:118-124). `same` != 0 promises the two operands are
+ *      the same array so the diagonal of a stationary outer kernel is exactly outer(0) = 1 (the dot product's is
+ *      sigma_0^2 + |f|^2, not overridden) and the mirror is exact; `same` == 2 (projected kernel) writes
  *      only the 64x64 tiles that intersect the lower triangle - all dqgp_potrf_solve_inv reads - and leaves
  *      the rest of d_K untouched.  Fidelity: dim = 2^q amplitudes with 1 <= q <= 12, and d_Psi1 / d_Psi2
  *      16-byte aligned (anything else returns < 0). */
@@ -95,6 +97,10 @@ int dqgp_gram_projected(int outer, const double* h_hyp, const double* d_F1, int 
                         double* d_K, int ldk, int same, void* stream);
 int dqgp_gram_fidelity(const double* d_Psi1, int n1, const double* d_Psi2, int n2, int dim, double* d_K, int ldk,
                        int same, void* stream);
+/*      k(f_i, f_i) of the projected kernel for every row of d_F (n, m) -> d_out[n] (the predictive variance's prior term,
+ *      main.py:1463): 1 for the stationary outer kernels (d_F is not read and may be NULL), sigma_0^2 + |f_i|^2 for the dot
+ *      product (DotProduct.diag). */
+int dqgp_projected_self_kernel(int outer, const double* h_hyp, const double* d_F, int n, int m, double* d_out, void* stream);
 
 /* ---- fp64 Cholesky / solve / inverse (agent_riemannian.py:410-418, :442): for the SPD matrix
  *      A = K + sigma^2 I held in the solver (dqgp_solver_matrix, leading dimension dqgp_solver_ld):
@@ -178,6 +184,7 @@ int dqgp_shift_parameter_sets(const double* d_z, int P, double h, double period,
  *      (agent_riemannian.py:270-275 and :431-436) without materialising any shifted Gram.
  *      d_F: (2P+1, n, m) features / d_Psi: (2P+1, n, dim) states of the sets in dqgp_shift_parameter_sets
  *      order; d_Ainv (n, ld).  d_work: dqgp_grad_workspace_bytes(n, P) bytes.  d_grad[P] is UNROUNDED.
+ *      Every outer kernel; the dot product's diagonal k(f_j, f_j) depends on the parameters and enters the sum.
  *      Fidelity: dim = 2^q amplitudes with 1 <= q <= 12, and d_Psi 16-byte aligned (anything else returns < 0). */
 size_t dqgp_grad_workspace_bytes(int n, int P);
 int dqgp_grad_projected(int outer, const double* h_hyp, const double* d_Ainv, int ld, const double* d_alpha,
