@@ -237,21 +237,27 @@ __global__ void __launch_bounds__(256) grad_reduce_kernel(const double* __restri
 }
 
 // ---- analytic gradient (opt-in; SURVEY 8(f) row 3: NOT the reference's central difference, Q3) -------------------------------
-// For the Gaussian outer kernel K_jk = exp(-gamma |f_j - f_k|^2) and B = A^-1 - alpha alpha^T,
-//   grad_i = 1/2 sum_jk B_jk dK_jk/dp_i = -2 gamma sum_j < df_j/dp_i , G_j >,   G_j = sum_k (B o K)_jk (f_j - f_k),
-// so ONE pass over the n x n entries (one exp per entry instead of 2P) gives G (n x m), and the P parameters only enter
-// through the feature Jacobian (dqgp_features_jacobian) in an O(P n m) contraction.
+// With B = A^-1 - alpha alpha^T (symmetric) and a stationary outer kernel K_jk = kappa(|f_j - f_k|^2),
+//   grad_i = 1/2 sum_jk B_jk dK_jk/dp_i = 2 sum_j < df_j/dp_i , G_j >,   G_j = sum_k B_jk kappa'(s_jk) (f_j - f_k),
+// so ONE pass over the n x n entries (one outer-kernel derivative per entry instead of 2P kernels) gives G (n x m), and the P
+// parameters only enter through the feature Jacobian (dqgp_features_jacobian) in an O(P n m) contraction.  The per-pair weight
+// is outer_analytic_weight (pairwise.cuh); the Gaussian's weight is e^{-gamma s} and its contraction scale -2 gamma.  The dot
+// product K_jk = sigma_0^2 + f_j.f_k gives grad_i = sum_j < df_j/dp_i , (B F)_j >: G_j = sum_k B_jk f_k, diagonal included,
+// contraction scale 1.
 // grad_analytic_rows_kernel: thread = row r of a column segment; f_r and the running G_r live in registers (M = 3q at compile
 // time), the segment's f_c stream through shared memory 64 columns at a time, A^-1 is read through its symmetric image
 // A^-1[c][r] so consecutive threads read consecutive addresses.  Fixed summation order: bit-reproducible.
+// hyp_a, hyp_b: the OuterHyp fields (hyp_a is the Gaussian's gamma; hyp_b is last so the parameter offsets before it are those
+// of a kernel without it).  ALPHA1: see outer_analytic_weight.
 constexpr int GA_ROWS = 128, GA_CHUNK = 64, GA_SEGMENTS = 16;
 
-template <int M>
+template <int OUTER, int M, bool ALPHA1>
 __global__ void __launch_bounds__(GA_ROWS) grad_analytic_rows_kernel(const double* __restrict__ Ainv, int ld, const double* __restrict__ alpha,
-                                                                    const double* __restrict__ F, int n, double gamma, int seg_cols,
-                                                                    double* __restrict__ Gpart) {
+                                                                    const double* __restrict__ F, int n, double hyp_a, int seg_cols,
+                                                                    double* __restrict__ Gpart, double hyp_b) {
     __shared__ double Fc[GA_CHUNK * M];
     __shared__ double ac[GA_CHUNK];
+    const OuterHyp hyp{hyp_a, hyp_b};
     const int r = blockIdx.x * GA_ROWS + threadIdx.x;
     const int c_begin = blockIdx.y * seg_cols, c_end = min(n, c_begin + seg_cols);
     const bool live = r < n;
@@ -268,10 +274,16 @@ __global__ void __launch_bounds__(GA_ROWS) grad_analytic_rows_kernel(const doubl
         if (!live) continue;
         for (int cc = 0; cc < cnt; ++cc) {
             const double* fc = Fc + cc * M;
+            if (OUTER == DQGP_OUTER_DOTPRODUCT) {
+                const double b = Ainv[(size_t)(c0 + cc) * ld + r] - ar * ac[cc];
+#pragma unroll
+                for (int k = 0; k < M; ++k) h[k] = fma(b, fc[k], h[k]);
+                continue;
+            }
             double df[M], d2 = 0.0;
 #pragma unroll
             for (int k = 0; k < M; ++k) { df[k] = fr[k] - fc[k]; d2 = fma(df[k], df[k], d2); }
-            const double q = (Ainv[(size_t)(c0 + cc) * ld + r] - ar * ac[cc]) * fast_exp(-gamma * d2);
+            const double q = (Ainv[(size_t)(c0 + cc) * ld + r] - ar * ac[cc]) * outer_analytic_weight<OUTER, ALPHA1>(d2, hyp);
 #pragma unroll
             for (int k = 0; k < M; ++k) h[k] = fma(q, df[k], h[k]);
         }
@@ -364,6 +376,16 @@ __global__ void __launch_bounds__(GF_ROWS) grad_fid_analytic_rows_kernel(const d
 static inline int grad_tiles(int n) {
     const int t = (n + PW_TILE - 1) / PW_TILE;
     return t * (t + 1) / 2;
+}
+
+template <int OUTER, bool ALPHA1>
+static void launch_grad_analytic_rows(int m, dim3 grid, cudaStream_t st, const double* Ainv, int ld, const double* alpha, const double* F,
+                                      int n, const OuterHyp& hyp, int seg_cols, double* Gpart) {
+    switch (m / 3) {
+#define DQGP_GA(QQ) case QQ: grad_analytic_rows_kernel<OUTER, 3 * QQ, ALPHA1><<<grid, GA_ROWS, 0, st>>>(Ainv, ld, alpha, F, n, hyp.a, seg_cols, Gpart, hyp.b); break;
+        DQGP_GA(1) DQGP_GA(2) DQGP_GA(3) DQGP_GA(4) DQGP_GA(5) DQGP_GA(6) DQGP_GA(7) DQGP_GA(8) DQGP_GA(9) DQGP_GA(10) DQGP_GA(11) DQGP_GA(12)
+#undef DQGP_GA
+    }
 }
 
 }  // namespace dqgp
@@ -461,7 +483,6 @@ int dqgp_grad_projected_analytic(int outer, const double* h_hyp, const double* d
                                  const double* d_J, int n, int m, int P, double* d_grad, void* d_work, void* stream) {
     using namespace dqgp;
     DQGP_REQUIRE(d_Ainv && d_alpha && d_F && d_J && d_grad && d_work && h_hyp, "dqgp_grad_projected_analytic: NULL argument");
-    DQGP_REQUIRE(outer == DQGP_OUTER_GAUSSIAN, "dqgp_grad_projected_analytic: only the Gaussian outer kernel (what the reference trains with, Q1)");
     DQGP_REQUIRE(n >= 1 && ld >= n && P >= 1 && m >= 3 && m <= 36 && m % 3 == 0, "dqgp_grad_projected_analytic: bad shape (m = 3q, q <= 12)");
     OuterHyp hyp;
     if (make_outer_hyp(outer, h_hyp, &hyp)) return -1;
@@ -471,15 +492,27 @@ int dqgp_grad_projected_analytic(int outer, const double* h_hyp, const double* d
     const int seg_cols = ((n + GA_SEGMENTS - 1) / GA_SEGMENTS + GA_CHUNK - 1) / GA_CHUNK * GA_CHUNK;
     const int segments = (n + seg_cols - 1) / seg_cols;
     dim3 grid((n + GA_ROWS - 1) / GA_ROWS, segments);
-    switch (m / 3) {
-#define DQGP_GA(QQ) case QQ: grad_analytic_rows_kernel<3 * QQ><<<grid, GA_ROWS, 0, st>>>(d_Ainv, ld, d_alpha, d_F, n, hyp.a, seg_cols, Gpart); break;
-        DQGP_GA(1) DQGP_GA(2) DQGP_GA(3) DQGP_GA(4) DQGP_GA(5) DQGP_GA(6) DQGP_GA(7) DQGP_GA(8) DQGP_GA(9) DQGP_GA(10) DQGP_GA(11) DQGP_GA(12)
-#undef DQGP_GA
+    double scale = 2.0;                        // stationary: 2 sum_j <J_j, G_j>
+    switch (outer) {
+        case DQGP_OUTER_GAUSSIAN:
+            launch_grad_analytic_rows<DQGP_OUTER_GAUSSIAN, false>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart);
+            scale = -2.0 * hyp.a;              // the weight is e^{-gamma s}: kappa' = -gamma e^{-gamma s}
+            break;
+        case DQGP_OUTER_MATERN15: launch_grad_analytic_rows<DQGP_OUTER_MATERN15, false>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart); break;
+        case DQGP_OUTER_EXPSINE2: launch_grad_analytic_rows<DQGP_OUTER_EXPSINE2, false>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart); break;
+        case DQGP_OUTER_RATQUAD:
+            if (hyp.b == 1.0) launch_grad_analytic_rows<DQGP_OUTER_RATQUAD, true>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart);
+            else launch_grad_analytic_rows<DQGP_OUTER_RATQUAD, false>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart);
+            break;
+        default:                               // DQGP_OUTER_DOTPRODUCT: make_outer_hyp refused every other id
+            launch_grad_analytic_rows<DQGP_OUTER_DOTPRODUCT, false>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart);
+            scale = 1.0;                       // sum_j <J_j, (B F)_j>
+            break;
     }
     DQGP_LAUNCH_CHECK("grad_analytic_rows_kernel");
     const size_t count = (size_t)n * m;
     grad_analytic_sum_kernel<<<(unsigned)((count + 255) / 256), 256, 0, st>>>(Gpart, count, segments, G);
-    grad_analytic_contract_kernel<<<P, 256, 0, st>>>(d_J, G, count, -2.0 * hyp.a, d_grad);
+    grad_analytic_contract_kernel<<<P, 256, 0, st>>>(d_J, G, count, scale, d_grad);
     DQGP_LAUNCH_CHECK("grad_analytic kernels");
     return 0;
 }

@@ -136,6 +136,40 @@ __device__ __forceinline__ double outer_grad_from_neg_gd2(double v, const OuterH
     }
 }
 
+// The analytic gradient's per-pair weight (grad_analytic_rows_kernel) from s = |f_j - f_k|^2, for a stationary outer kernel
+// K = kappa(s): kappa'(s), with d = sqrt(s), a and b as in OuterHyp.  The Gaussian returns e^{-gamma s} and leaves -gamma to the
+// contraction's scale.
+//   Matern 1.5:        -(3/2) a^2 e^{-sqrt(3) a d}
+//   ExpSineSquared:    -a^2 b (sin(2 b d) / d) kappa, kappa = e^{-2 a^2 sin^2(b d)}
+//   RationalQuadratic: -alpha a base^{-alpha-1}, base = 1 + a s (alpha = 1: -a / base^2)
+// A duplicate sample (s = 0) gets a finite weight: fast_sqrt_guarded never returns 0, and sin(b d) / d is then b exactly.  Matern,
+// ExpSineSquared and RationalQuadratic clamp their exponents at -700 (a tiny length scale reaches it); the Gaussian's -gamma s is
+// not clamped and stays inside fast_exp's range while gamma 4m < 708.  NaN features reach the gradient through f_j - f_k whatever
+// the weight.  Not warp-collective: rows past n leave the column loop, so the table exp cannot be used.
+// ALPHA1 (RationalQuadratic only): alpha = 1, chosen by the host per launch, so the pair loop carries no branch on alpha.
+template <int OUTER, bool ALPHA1>
+__device__ __forceinline__ double outer_analytic_weight(double s, const OuterHyp& h) {
+    if (OUTER == DQGP_OUTER_GAUSSIAN) {
+        return fast_exp(-h.a * s);
+    } else if (OUTER == DQGP_OUTER_MATERN15) {
+        const double nk = fast_sqrt_guarded(s) * (-1.7320508075688772 * h.a);      // -sqrt(3) d / l
+        return (-1.5 * h.a * h.a) * fast_exp(fmax(nk, -700.0));
+    } else if (OUTER == DQGP_OUTER_RATQUAD) {
+        const double base = fma(s, h.a, 1.0);
+        if (ALPHA1) {
+            const double r = fast_rcp_ge1(base);
+            return -h.a * (r * r);
+        }
+        return (-h.b * h.a) * fast_exp(fmax(-(h.b + 1.0) * log(base), -700.0));
+    } else {
+        const double d = fast_sqrt_guarded(s);
+        double sn, cs;
+        sincos(h.b * d, &sn, &cs);
+        const double k = fast_exp(fmax(-2.0 * (h.a * h.a) * (sn * sn), -700.0));
+        return (-2.0 * h.a * h.a * h.b) * (sn * cs / d) * k;
+    }
+}
+
 // out[row] = add (+ |F[row]|^2 when with_norm), rows of m features (gram.cu)
 void launch_self_kernel(const double* F, long long rows, int m, double add, bool with_norm, double* out, cudaStream_t st);
 

@@ -75,8 +75,8 @@ class AgentEngine:
         """``gradient``: "central_difference" = the reference's rule (dK_i = (K(p + h e_i) - K(p - h e_i)) / 2h, h = pi/8,
         agent_riemannian.py:275) - the parity path; "analytic" (opt-in, SURVEY 8(f) row 3) = the exact derivative of the NLL:
         feature Jacobian from one extra suffix simulation per parameter and ONE pass over the n^2 Gram entries.  The analytic
-        mode does NOT reproduce the reference's trajectories (its h = pi/8 difference is far from the derivative); it needs the
-        Gaussian outer kernel (projected) or at most 6 qubits (fidelity)."""
+        mode does NOT reproduce the reference's trajectories (its h = pi/8 difference is far from the derivative).  It takes
+        every outer kernel of the projected kernel, and at most 6 qubits for the fidelity kernel."""
         _require_cuda()
         self._lib = _lib.load()
         X = np.asarray(X, dtype=np.float64)
@@ -102,8 +102,6 @@ class AgentEngine:
         if gradient not in ("central_difference", "analytic"):
             raise ValueError(f"Unknown gradient mode: {gradient}")
         self.gradient_mode = gradient
-        if gradient == "analytic" and kernel_type == "projected" and self.outer_kernel != "gaussian":
-            raise ValueError("gradient='analytic' needs the Gaussian outer kernel for the projected kernel")
         if gradient == "analytic" and kernel_type == "fidelity" and self.q > 6:
             raise ValueError("gradient='analytic' supports the fidelity kernel up to 6 qubits")
         self.d_Pm = torch.empty((self.S, self.P), **f64)

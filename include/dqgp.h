@@ -196,8 +196,16 @@ int dqgp_grad_fidelity(const double* d_Ainv, int ld, const double* d_alpha, cons
  *      h = pi/8 - trajectories differ from the reference's; replaces the dead evaluate_derivatives branch,
  *      agent_riemannian.py:402-404).  dqgp_features_jacobian: d_F (n,3q) features at d_p (P) and d_J (P,n,3q) their exact
  *      derivatives, one extra suffix simulation per parameter (every parameter must feed exactly one gate).
- *      dqgp_grad_projected_analytic: Gaussian outer kernel, d_Ainv the FULL symmetric A^-1 (want_inverse = 2), one pass
- *      over the n^2 entries (one exp per entry instead of 2P).  d_work: dqgp_grad_analytic_workspace_bytes(n, m). */
+ *      dqgp_grad_projected_analytic: every outer id (DQGP_OUTER_*), h_hyp as for dqgp_grad_projected ({gamma} | {length_scale} |
+ *      {length_scale, periodicity} | {length_scale, alpha} | {sigma_0}); d_Ainv the FULL symmetric A^-1 (want_inverse = 2);
+ *      m = 3q, q <= 12.  With B = A^-1 - alpha alpha^T, s = |f_j - f_k|^2 and d = sqrt(s), one pass over the n^2 entries
+ *      (one outer-kernel derivative per entry instead of 2P kernels) gives
+ *        stationary K = kappa(s): grad_i = 2 sum_j <J_i,j, G_j>, G_j = sum_k B_jk kappa'(s_jk) (f_j - f_k), with kappa'(s) =
+ *          gaussian -gamma e^{-gamma s}; matern -(3/2) e^{-sqrt(3) d / l} / l^2;
+ *          expsinesquared -(pi / (p l^2)) (sin(2 pi d / p) / d) K (limit -2 pi^2 / (p l)^2 at d = 0);
+ *          rationalquadratic -(1 / (2 l^2)) (1 + s / (2 alpha l^2))^(-alpha-1);
+ *        dotproduct K = sigma_0^2 + f_j.f_k: grad_i = sum_j <J_i,j, (B F)_j> (diagonal included; sigma_0 drops out).
+ *      d_work: dqgp_grad_analytic_workspace_bytes(n, m). */
 int dqgp_features_jacobian(const dqgp_circuit* c, const double* d_X, int n, const double* d_p, double* d_F, double* d_J, void* stream);
 /* fidelity kernel: d_Psi (n,2^q) states at d_p and d_D (P,n,2^q) their derivatives d psi / dp_i (complex128);
  * dqgp_grad_fidelity_analytic: grad_i = 2 Re sum_j <G_j | d_i psi_j>, G_j = sum_k (A^-1 - alpha alpha^T)_jk <psi_k|psi_j> psi_k; q <= 6. */

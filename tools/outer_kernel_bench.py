@@ -1,11 +1,13 @@
-"""Time the projected Gram (dqgp_gram_projected, same = 2: the lower tiles the factorisation reads) and the fused central-difference
-gradient (dqgp_grad_projected) for every outer kernel at the shard shapes of BASELINE configs 4 and 5, with CUDA events.
+"""Time the projected Gram (dqgp_gram_projected, same = 2: the lower tiles the factorisation reads), the fused central-difference
+gradient (dqgp_grad_projected) and the analytic gradient (dqgp_grad_projected_analytic, `grad_analytic_ms`) for every outer kernel at
+the shard shapes of BASELINE configs 4 and 5, with CUDA events.
 
     python tools/outer_kernel_bench.py [--reps 5] [--rounds 3]
 
-Inputs are seeded and synthetic: features uniform in [-1, 1] (where Pauli expectations lie), a random symmetric A^-1 and alpha
-(the gradient's cost does not depend on their values).  The outer kernels are timed in turn, `rounds` times over, and each
-figure is the median of the rounds' mean times.  Prints one JSON line with the card's name and power limit."""
+Inputs are seeded and synthetic: features uniform in [-1, 1] (where Pauli expectations lie), a random symmetric A^-1 and alpha,
+and for the analytic gradient a random feature Jacobian (the gradients' cost does not depend on these values).  The outer
+kernels are timed in turn, `rounds` times over, and each figure is the median of the rounds' mean times.  Prints one JSON line
+with the card's name and power limit."""
 import argparse
 import ctypes as C
 import json
@@ -66,7 +68,9 @@ def main():
         K = torch.zeros((n, n), dtype=torch.float64, device="cuda")
         grad = torch.zeros(P, dtype=torch.float64, device="cuda")
         work = torch.empty(lib.dqgp_grad_workspace_bytes(n, P) // 8 + 1, dtype=torch.float64, device="cuda")
-        samples = {o: {"gram_ms": [], "grad_ms": []} for o in OUTERS}
+        J = torch.randn((P, n, m), dtype=torch.float64, device="cuda", generator=g)
+        work_a = torch.empty(lib.dqgp_grad_analytic_workspace_bytes(n, m) // 8 + 1, dtype=torch.float64, device="cuda")
+        samples = {o: {"gram_ms": [], "grad_ms": [], "grad_analytic_ms": []} for o in OUTERS}
         for _ in range(args.rounds):
             for o in OUTERS:
                 oid, hyp = _lib.OUTER_KERNELS[o], _lib.hyp_array(d.kernels.outer_hyp(o))
@@ -79,12 +83,17 @@ def main():
                     assert lib.dqgp_grad_projected(oid, hyp, ainv.data_ptr(), n, alpha.data_ptr(), F.data_ptr(), n, m, P, 0.39269908169872414,
                                                    grad.data_ptr(), work.data_ptr(), st) == 0, lib.dqgp_last_error()
 
+                def gradient_analytic():
+                    assert lib.dqgp_grad_projected_analytic(oid, hyp, ainv.data_ptr(), n, alpha.data_ptr(), F.data_ptr(), J.data_ptr(), n,
+                                                            m, P, grad.data_ptr(), work_a.data_ptr(), st) == 0, lib.dqgp_last_error()
+
                 samples[o]["gram_ms"].append(timed(gram, 4 * args.reps))
                 samples[o]["grad_ms"].append(timed(gradient, args.reps))
+                samples[o]["grad_analytic_ms"].append(timed(gradient_analytic, 4 * args.reps))
         results[cname] = {"n": n, "q": c["q"], "m": m, "P": P,
                           **{o: {k: round(sorted(v)[len(v) // 2], 4) for k, v in s.items()} for o, s in samples.items()},
                           "spread_ms": {o: {k: round(max(v) - min(v), 4) for k, v in s.items()} for o, s in samples.items()}}
-        del F, ainv, K, work
+        del F, ainv, K, work, J, work_a
         torch.cuda.empty_cache()
     name, power = card()
     print(json.dumps({"tool": "outer_kernel_bench", "card": name, "power_limit_w": power, "reps": args.reps, "rounds": args.rounds,
