@@ -47,7 +47,7 @@ class RiemannianAgent:
         #   False, projected: `_manual_projected_kernel_derivatives_riemannian` (:279-312) - the same central difference, but
         #         through self.q_kernel, which was built with the REAL outer kernel -> training_ignores_outer_kernel=False;
         #   False, fidelity: `q_kernel.evaluate_derivatives(["K", "dKdp"])` (:402-404), the analytic derivative -> gradient="analytic"
-        #         (up to 6 qubits here; AgentEngine raises beyond that instead of silently substituting the finite difference).
+        #         (every qubit count up to 12, as the central difference).
         # Explicit `training_ignores_outer_kernel` / `gradient` arguments override the mapping.
         if training_ignores_outer_kernel is None:
             training_ignores_outer_kernel = bool(use_parameter_shift) or kernel_type != "projected"

@@ -5,8 +5,10 @@
 // row fragment read from the same shared-memory tile at index t^1 with a sign flip (no extra staging, no extra HBM).
 // MODE 0 writes the Gram (FidelityKernel.evaluate, reference main.py:118-124); MODE 1 is the fused central-difference
 // gradient over the 2P shifted state sets (agent_riemannian.py:270-275,431-436), lower tiles only, B = A^-1 - alpha
-// alpha^T in registers, deterministic two-stage reduction.  Operand chunks of 32 doubles stream through a
-// double-buffered ring filled by the TMA engine.
+// alpha^T in registers, deterministic two-stage reduction.  MODE 2 is the first stage of the analytic gradient for
+// 2^q >= 128 (grad.cu): over the lower tiles of one state set it writes W = B o S, S_jk = <psi_k|psi_j>, as the real
+// matrix [W_re | W_im] (row stride ldk = 2 n_pad) together with each off-diagonal tile's mirror (W_re symmetric, W_im
+// antisymmetric).  Operand chunks of 32 doubles stream through a double-buffered ring filled by the TMA engine.
 #include <cstring>
 #include "pairwise.cuh"
 #include "tensormap.cuh"
@@ -30,7 +32,7 @@ __device__ __forceinline__ void fd_stage_bulk(double* buf, const double* __restr
     }
 }
 
-// MODE 1 (one state array): the chunk as two boxes of a 3-D tensor map over Psi = [set][state][2 * 2^q doubles] (TMA proper, SASS UTMALDG), issued by one thread: box =
+// MODE 1 and 2 (one state array): the chunk as two boxes of a 3-D tensor map over Psi = [set][state][2 * 2^q doubles] (TMA proper, SASS UTMALDG), issued by one thread: box =
 // 64 states x FD_PITCH doubles starting at the chunk; the four doubles beyond the chunk land in the padding of the fragment layout (never
 // read), states beyond n arrive as zero rows (their bracket weights are zero).
 __device__ __forceinline__ void fd_stage_tmap(double* buf, const void* tmap, int set, int row0, int col0, int k0, unsigned long long* bar) {
@@ -56,7 +58,7 @@ __global__ void __launch_bounds__(PW_THREADS, 1) fidelity_dmma_kernel(const doub
     if (threadIdx.x == 0) { mbar_init(&s_bar[0], 1); mbar_init(&s_bar[1], 1); mbar_fence_init(); }
     __syncthreads();
     int bi, bj;
-    if (MODE == 1) {
+    if (MODE != 0) {
         bi = int((sqrt(8.0 * blockIdx.x + 1.0) - 1.0) * 0.5);
         while ((bi + 1) * (bi + 2) / 2 <= (int)blockIdx.x) ++bi;
         while (bi * (bi + 1) / 2 > (int)blockIdx.x) --bi;
@@ -72,8 +74,8 @@ __global__ void __launch_bounds__(PW_THREADS, 1) fidelity_dmma_kernel(const doub
     const double jsign = (t & 1) ? -1.0 : 1.0;
 
     double br[2][4][2];
-    if (MODE == 1) {
-        const double weight = (bi == bj) ? 1.0 : 2.0;
+    if (MODE != 0) {
+        const double weight = (MODE == 2 || bi == bj) ? 1.0 : 2.0;
 #pragma unroll
         for (int rb = 0; rb < 2; ++rb) {
             const int r = row0 + wr * 16 + rb * 8 + g;
@@ -91,7 +93,7 @@ __global__ void __launch_bounds__(PW_THREADS, 1) fidelity_dmma_kernel(const doub
     const size_t set_stride1 = (size_t)n1 * d2, set_stride2 = (size_t)n2 * d2;
     const int first_set = (MODE == 1) ? 1 : 0;
     const int total = n_sets * n_chunks;
-    if (MODE == 1) fd_stage_tmap(fd_smem, &tmap, first_set, row0, col0, 0, &s_bar[0]);
+    if (MODE != 0) fd_stage_tmap(fd_smem, &tmap, first_set, row0, col0, 0, &s_bar[0]);
     else fd_stage_bulk(fd_smem, Psi1 + first_set * set_stride1, Psi2 + first_set * set_stride2, row0, col0, n1, n2, d2, 0, kc, &s_bar[0]);
     double re[2][4][2], im[2][4][2];
     double pplus = 0.0;
@@ -108,7 +110,7 @@ __global__ void __launch_bounds__(PW_THREADS, 1) fidelity_dmma_kernel(const doub
         }
         if (it + 1 < total) {
             const int ns = (it + 1) / n_chunks, nch = (it + 1) - ns * n_chunks;
-            if (MODE == 1)
+            if (MODE != 0)
                 fd_stage_tmap(fd_smem + ((it + 1) & 1) * FD_STAGE, &tmap, first_set + ns, row0, col0, nch * kc, &s_bar[(it + 1) & 1]);
             else
                 fd_stage_bulk(fd_smem + ((it + 1) & 1) * FD_STAGE, Psi1 + (size_t)(first_set + ns) * set_stride1,
@@ -151,6 +153,28 @@ __global__ void __launch_bounds__(PW_THREADS, 1) fidelity_dmma_kernel(const doub
                                 K[(size_t)r * ldk + c + e] = fma(re[rb][cb][e], re[rb][cb][e], im[rb][cb][e] * im[rb][cb][e]);
                     }
                 }
+            } else if (MODE == 2) {
+                // every row and column below n_pad = ldk / 2 is written: states past n arrive as zero rows and B is zero there.
+                // A diagonal tile computes all its entries itself (no mirror: two writers of one entry would race).
+                const int npad = ldk >> 1;
+#pragma unroll
+                for (int rb = 0; rb < 2; ++rb) {
+                    const int r = row0 + wr * 16 + rb * 8 + g;
+#pragma unroll
+                    for (int cb = 0; cb < 4; ++cb) {
+                        const int c = col0 + wc * 32 + cb * 8 + 2 * t;
+                        const double2 wre = make_double2(br[rb][cb][0] * re[rb][cb][0], br[rb][cb][1] * re[rb][cb][1]);
+                        const double2 wim = make_double2(br[rb][cb][0] * im[rb][cb][0], br[rb][cb][1] * im[rb][cb][1]);
+                        *reinterpret_cast<double2*>(K + (size_t)r * ldk + c) = wre;
+                        *reinterpret_cast<double2*>(K + (size_t)r * ldk + npad + c) = wim;
+                        if (bi != bj) {
+                            K[(size_t)c * ldk + r] = wre.x;
+                            K[(size_t)(c + 1) * ldk + r] = wre.y;
+                            K[(size_t)c * ldk + npad + r] = -wim.x;
+                            K[(size_t)(c + 1) * ldk + npad + r] = -wim.y;
+                        }
+                    }
+                }
             } else {
                 double part = 0.0;
 #pragma unroll
@@ -189,6 +213,7 @@ static int fd_attr() {
     if (!done) {
         DQGP_CUDA(cudaFuncSetAttribute(fidelity_dmma_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FD_SMEM));
         DQGP_CUDA(cudaFuncSetAttribute(fidelity_dmma_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FD_SMEM));
+        DQGP_CUDA(cudaFuncSetAttribute(fidelity_dmma_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FD_SMEM));
         done = true;
     }
     return 0;
@@ -217,6 +242,21 @@ int fidelity_grad_dmma(const double* Ainv, int ld, const double* alpha, const do
                  "dqgp_grad_fidelity: the driver refused the tensor map of the states (n %d, dim %d, P %d)", n, dim, P);
     fidelity_dmma_kernel<1><<<tiles, PW_THREADS, FD_SMEM, st>>>(Psi, n, Psi, n, 2 * dim, 2 * P, nullptr, 0, Ainv, ld, alpha, P, partial, tmap);
     DQGP_LAUNCH_CHECK("fidelity_dmma_kernel<1>");
+    return 0;
+}
+
+int fidelity_weights_dmma(const double* Ainv, int ld, const double* alpha, const double* Psi, int n, int dim, double* W, int n_pad,
+                          cudaStream_t st) {
+    int rc = fd_attr();
+    if (rc) return rc;
+    CUtensorMap tmap;
+    memset(&tmap, 0, sizeof(tmap));
+    DQGP_REQUIRE(make_rows_tensor_map(&tmap, Psi, 2 * dim, n, 1, FD_PITCH, PW_TILE),
+                 "dqgp_grad_fidelity_analytic: the driver refused the tensor map of the states (n %d, dim %d)", n, dim);
+    const int t = n_pad / PW_TILE;
+    fidelity_dmma_kernel<2><<<t * (t + 1) / 2, PW_THREADS, FD_SMEM, st>>>(Psi, n, Psi, n, 2 * dim, 1, W, 2 * n_pad, Ainv, ld, alpha, 0,
+                                                                         nullptr, tmap);
+    DQGP_LAUNCH_CHECK("fidelity_dmma_kernel<2>");
     return 0;
 }
 

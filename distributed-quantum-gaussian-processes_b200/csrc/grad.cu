@@ -7,7 +7,9 @@
 // kernel and contracting on the fly.  Partial sums go to partial[tile][i]; a second kernel adds them in a
 // fixed order, so the result is bit-reproducible run to run (the reference rounds it to 4 decimals).
 // Bound: FP64 pipe (3m + outer-kernel flops per entry, SURVEY §8(d)); HBM traffic is one read of A^-1.
+#include <algorithm>
 #include <cstring>
+#include "gemm64.cuh"
 #include "pairwise.cuh"
 #include "tensormap.cuh"
 
@@ -373,6 +375,49 @@ __global__ void __launch_bounds__(GF_ROWS) grad_fid_analytic_rows_kernel(const d
     }
 }
 
+// Fidelity kernel, analytic gradient for 128 <= 2^q <= 4096 as two dense DMMA stages.  With R the states as a real n x 2 dim
+// matrix (re, im interleaved) and R~ = R with (re, im) -> (-im, re) per amplitude:
+//   1. W = B o S as [W_re | W_im] (fidelity_dmma_kernel<2>, fid.cu);
+//   2. G = W_re R + W_im R~ = [W_re | W_im] [R; R~], one real GEMM on the grouped DMMA engine (gemm64.cu);
+//   3. grad_i = 2 <D_i, G> over the first n rows, in slices (partial sums in the W region, free after the GEMM).
+// Workspace (doubles): the one-task GEMM table, W (n_pad x 2 n_pad), [R; R~] (2 n_pad x 2 dim), G (n_pad x 2 dim), with
+// n_pad = n rounded up to the GEMM's 128-row tile.
+constexpr int GFD_TABLE = 16;                   // doubles reserved for the GemmTask
+static_assert(sizeof(GemmTask) <= GFD_TABLE * sizeof(double), "the GEMM task must fit its workspace slot");
+static inline size_t gfd_npad(int n) { return ((size_t)n + GM_BM - 1) / GM_BM * GM_BM; }
+
+// [R; R~] with zero rows past n: row k < n_pad is psi_k, row n_pad + k is J psi_k
+__global__ void grad_fid_pack_kernel(const double2* __restrict__ Psi, int n, int dim, int n_pad, double2* __restrict__ RR) {
+    const size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= (size_t)n_pad * dim) return;
+    const size_t k = e / dim;
+    const double2 v = k < (size_t)n ? Psi[e] : make_double2(0.0, 0.0);
+    RR[e] = v;
+    RR[(size_t)n_pad * dim + e] = make_double2(-v.y, v.x);
+}
+// <D_i, G> in fixed slices of `count`, one CTA per (slice, parameter): P CTAs alone (40 at q = 10) cannot stream P n 2^(q+1) doubles
+// of d psi at HBM rate.  partial[slice][i]; grad_reduce_kernel adds the slices in a fixed order.
+constexpr int GFD_SLICES = 64;
+__global__ void __launch_bounds__(256) grad_fid_contract_kernel(const double* __restrict__ D, const double* __restrict__ G, size_t count, int P,
+                                                                double* __restrict__ partial) {
+    __shared__ double sred[256];
+    const size_t per = (count + gridDim.x - 1) / gridDim.x;
+    const size_t b = (size_t)blockIdx.x * per, e = min(count, b + per);
+    const double* Di = D + (size_t)blockIdx.y * count;
+    double acc = 0.0;
+#pragma unroll 4
+    for (size_t k = b + threadIdx.x; k < e; k += 256) acc = fma(Di[k], G[k], acc);
+    sred[threadIdx.x] = acc;
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {
+        if (threadIdx.x < o) sred[threadIdx.x] += sred[threadIdx.x + o];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) partial[(size_t)blockIdx.x * P + blockIdx.y] = sred[0];
+}
+// the task table is written on the device so the entry point stays capturable into a CUDA graph (a host copy would synchronise)
+__global__ void grad_fid_task_kernel(GemmTask t, GemmTask* __restrict__ dst) { *dst = t; }
+
 static inline int grad_tiles(int n) {
     const int t = (n + PW_TILE - 1) / PW_TILE;
     return t * (t + 1) / 2;
@@ -519,7 +564,9 @@ int dqgp_grad_projected_analytic(int outer, const double* h_hyp, const double* d
 
 size_t dqgp_grad_fidelity_analytic_workspace_bytes(int n, int dim) {
     if (n <= 0 || dim <= 0) return 0;
-    return sizeof(double) * 2 * (size_t)(dqgp::GA_SEGMENTS + 1) * (size_t)n * (size_t)dim;
+    if (dim <= 64) return sizeof(double) * 2 * (size_t)(dqgp::GA_SEGMENTS + 1) * (size_t)n * (size_t)dim;
+    const size_t npad = dqgp::gfd_npad(n);
+    return sizeof(double) * (dqgp::GFD_TABLE + 2 * npad * npad + 6 * npad * (size_t)dim);
 }
 
 int dqgp_grad_fidelity_analytic(const double* d_Ainv, int ld, const double* d_alpha, const double* d_Psi, const double* d_D, int n, int dim,
@@ -527,8 +574,42 @@ int dqgp_grad_fidelity_analytic(const double* d_Ainv, int ld, const double* d_al
     using namespace dqgp;
     DQGP_REQUIRE(d_Ainv && d_alpha && d_Psi && d_D && d_grad && d_work, "dqgp_grad_fidelity_analytic: NULL argument");
     DQGP_REQUIRE(n >= 1 && ld >= n && P >= 1, "dqgp_grad_fidelity_analytic: bad shape");
-    DQGP_REQUIRE(dim >= 2 && dim <= 64 && (dim & (dim - 1)) == 0, "dqgp_grad_fidelity_analytic: 2^q amplitudes with q <= 6 (got %d)", dim);
+    DQGP_REQUIRE(dim >= 2 && dim <= (1 << MAX_QUBITS) && (dim & (dim - 1)) == 0,
+                 "dqgp_grad_fidelity_analytic: dim %d is not 2^q amplitudes with 1 <= q <= %d", dim, MAX_QUBITS);
     cudaStream_t st = as_stream(stream);
+    if (dim > 64) {
+        DQGP_REQUIRE((reinterpret_cast<uintptr_t>(d_Psi) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_work) & 15) == 0,
+                     "dqgp_grad_fidelity_analytic: the state array and the workspace must be 16-byte aligned for 2^q >= 128");
+        const int npad = (int)gfd_npad(n), d2 = 2 * dim;
+        GemmTask* task = static_cast<GemmTask*>(d_work);
+        double* W = static_cast<double*>(d_work) + GFD_TABLE;
+        double* RR = W + (size_t)2 * npad * npad;
+        double* G = RR + (size_t)2 * npad * d2;
+        int rc = fidelity_weights_dmma(d_Ainv, ld, d_alpha, d_Psi, n, dim, W, npad, st);
+        if (rc) return rc;
+        const size_t pairs = (size_t)npad * dim;
+        grad_fid_pack_kernel<<<(unsigned)((pairs + 255) / 256), 256, 0, st>>>(reinterpret_cast<const double2*>(d_Psi), n, dim, npad,
+                                                                               reinterpret_cast<double2*>(RR));
+        GemmTask t;
+        memset(&t, 0, sizeof(t));
+        t.A = W; t.B = RR; t.C = G;
+        t.M = npad; t.N = d2; t.K = 2 * npad;
+        t.lda = 2 * npad; t.ldb = d2; t.ldc = d2;
+        t.a_k_contig = 1; t.b_k_contig = 0;
+        t.lower_tiles = 0; t.krule = GM_KRULE_ALL;
+        t.alpha = 1.0; t.beta = 0.0;
+        t.tile_begin = 0; t.tiles = gemm_task_tiles(t);
+        grad_fid_task_kernel<<<1, 1, 0, st>>>(t, task);
+        DQGP_LAUNCH_CHECK("grad_fid_pack_kernel / grad_fid_task_kernel");
+        rc = launch_gemm_group(task, 1, t.tiles, st);       // an unregistered table: the cp.async ring
+        if (rc) return rc;
+        const size_t count = (size_t)n * d2;
+        const int slices = (int)std::max<size_t>(1, std::min<size_t>(GFD_SLICES, (size_t)2 * npad * npad / P));
+        grad_fid_contract_kernel<<<dim3(slices, P), 256, 0, st>>>(d_D, G, count, P, W);
+        grad_reduce_kernel<<<P, 256, 0, st>>>(W, slices, P, 2.0, d_grad);
+        DQGP_LAUNCH_CHECK("grad_fid_contract_kernel");
+        return 0;
+    }
     double2* Gpart = static_cast<double2*>(d_work);
     double2* G = Gpart + (size_t)GA_SEGMENTS * n * dim;
     const int seg_cols = ((n + GA_SEGMENTS - 1) / GA_SEGMENTS + GF_CHUNK - 1) / GF_CHUNK * GF_CHUNK;

@@ -177,6 +177,9 @@ void launch_self_kernel(const double* F, long long rows, int m, double add, bool
 int fidelity_gram_dmma(const double* Psi1, int n1, const double* Psi2, int n2, int dim, double* K, int ldk, cudaStream_t st);
 int fidelity_grad_dmma(const double* Ainv, int ld, const double* alpha, const double* Psi, int n, int dim, int P, double* partial,
                        int tiles, cudaStream_t st);
+// W = [B o Re S | B o Im S] (n_pad x 2 n_pad, every entry written), S_jk = <psi_k|psi_j>, B = A^-1 - alpha alpha^T
+int fidelity_weights_dmma(const double* Ainv, int ld, const double* alpha, const double* Psi, int n, int dim, double* W, int n_pad,
+                          cudaStream_t st);
 
 constexpr int G2_PITCH = 36;   // doubles per staged sample row: = 4 (mod 16) -> conflict-free DMMA fragment loads
 

@@ -76,7 +76,9 @@ class AgentEngine:
         agent_riemannian.py:275) - the parity path; "analytic" (opt-in, SURVEY 8(f) row 3) = the exact derivative of the NLL:
         feature Jacobian from one extra suffix simulation per parameter and ONE pass over the n^2 Gram entries.  The analytic
         mode does NOT reproduce the reference's trajectories (its h = pi/8 difference is far from the derivative).  It takes
-        every outer kernel of the projected kernel, and at most 6 qubits for the fidelity kernel."""
+        every outer kernel of the projected kernel and the fidelity kernel up to 12 qubits.  It keeps the derivative of every
+        sample's state (fidelity) or features (projected) for every parameter resident: P * n * 2^q * 16 bytes for the fidelity
+        kernel, e.g. 5.4 GB at q = 10, n = 8192, P = 40, plus a workspace of about 16 n^2 bytes from 2^q = 128 on."""
         _require_cuda()
         self._lib = _lib.load()
         X = np.asarray(X, dtype=np.float64)
@@ -102,8 +104,6 @@ class AgentEngine:
         if gradient not in ("central_difference", "analytic"):
             raise ValueError(f"Unknown gradient mode: {gradient}")
         self.gradient_mode = gradient
-        if gradient == "analytic" and kernel_type == "fidelity" and self.q > 6:
-            raise ValueError("gradient='analytic' supports the fidelity kernel up to 6 qubits")
         self.d_Pm = torch.empty((self.S, self.P), **f64)
         if gradient == "analytic":
             self.d_feat = torch.empty((1, self.n, self.m), **f64)

@@ -208,7 +208,9 @@ int dqgp_grad_fidelity(const double* d_Ainv, int ld, const double* d_alpha, cons
  *      d_work: dqgp_grad_analytic_workspace_bytes(n, m). */
 int dqgp_features_jacobian(const dqgp_circuit* c, const double* d_X, int n, const double* d_p, double* d_F, double* d_J, void* stream);
 /* fidelity kernel: d_Psi (n,2^q) states at d_p and d_D (P,n,2^q) their derivatives d psi / dp_i (complex128);
- * dqgp_grad_fidelity_analytic: grad_i = 2 Re sum_j <G_j | d_i psi_j>, G_j = sum_k (A^-1 - alpha alpha^T)_jk <psi_k|psi_j> psi_k; q <= 6. */
+ * dqgp_grad_fidelity_analytic: grad_i = 2 Re sum_j <G_j | d_i psi_j>, G_j = sum_k (A^-1 - alpha alpha^T)_jk <psi_k|psi_j> psi_k; d_Ainv
+ *      the FULL symmetric A^-1 (want_inverse = 2); dim = 2^q, 1 <= q <= 12.  From dim = 128 on, d_Psi and d_work must be 16-byte
+ *      aligned; d_work: dqgp_grad_fidelity_analytic_workspace_bytes(n, dim).  Deterministic: a second call gives the same bits. */
 int dqgp_states_jacobian(const dqgp_circuit* c, const double* d_X, int n, const double* d_p, double* d_Psi, double* d_D, void* stream);
 size_t dqgp_grad_fidelity_analytic_workspace_bytes(int n, int dim);
 int dqgp_grad_fidelity_analytic(const double* d_Ainv, int ld, const double* d_alpha, const double* d_Psi, const double* d_D, int n,
