@@ -80,6 +80,9 @@ SIGNATURES = {
     "dqgp_grad_fidelity_analytic": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "dqgp_grad_analytic_workspace_bytes": (_sz, [_i, _i]),
     "dqgp_grad_projected_analytic": (_i, [_i, _dp, _vp, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
+    "dqgp_grad_outer_hyperparameters_workspace_bytes": (_sz, [_i]),
+    "dqgp_grad_outer_hyperparameters": (_i, [_i, _dp, _vp, _i, _vp, _vp, _i, _i, _vp, _vp, _vp]),
+    "dqgp_grad_noise_std": (_i, [_vp, _i, _vp, _i, _d, _vp, _vp]),
     "dqgp_nll_terms": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     "dqgp_admm_local": (_i, [_vp, _vp, _vp, _i, _d, _d, _d, _vp, _vp, _vp]),
     "dqgp_admm_consensus": (_i, [_vp, _vp, _i, _i, _d, _d, _vp, _vp]),

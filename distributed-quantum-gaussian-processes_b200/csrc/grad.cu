@@ -418,6 +418,124 @@ __global__ void __launch_bounds__(256) grad_fid_contract_kernel(const double* __
 // the task table is written on the device so the entry point stays capturable into a CUDA graph (a host copy would synchronise)
 __global__ void grad_fid_task_kernel(GemmTask t, GemmTask* __restrict__ dst) { *dst = t; }
 
+// ---- NLL gradient with respect to the outer kernel's hyper-parameters h: dNLL/dh = 1/2 sum_jk B_jk dK_jk/dh, B = A^-1 - alpha alpha^T.
+// One CTA per lower 64x64 tile, the Gram kernel's layout: both feature tiles staged once, -d^2 from the Gram identity on DMMA, then
+// the Gram's snap-to-zero and diagonal rules (so duplicates and the diagonal see the s = 0 of the K that was factored) and its NaN
+// restore.  Entries j > k weigh 2, j = k weighs 1, j < k is never read: A^-1 may be the lower tiles only (want_inverse = 1).
+// partial[tile][2] = {c0 sum B w0, c1 sum B w1} (outer_hyper_terms); grad_reduce_kernel adds the tiles in a fixed order.  The dot
+// product's terms do not depend on the features: its tiles skip the staging and the DMMA.
+template <int OUTER>
+__global__ void __launch_bounds__(PW_THREADS) grad_hyper_dmma_kernel(const double* __restrict__ Ainv, int ld, const double* __restrict__ alpha,
+                                                                     const double* __restrict__ F, int n, int m, OuterHyp hyp, double c0,
+                                                                     double c1, double* __restrict__ partial) {
+    __shared__ __align__(16) double Fr[PW_TILE * G2_PITCH];
+    __shared__ __align__(16) double Fc[PW_TILE * G2_PITCH];
+    __shared__ __align__(16) double nr[2 * PW_TILE];
+    __shared__ double s_red[2][PW_THREADS / 32];
+    constexpr bool STAT = outer_is_stationary(OUTER);
+    int bi, bj;
+    tile_from_index(blockIdx.x, bi, bj);
+    const int row0 = bi * PW_TILE, col0 = bj * PW_TILE;
+    const int mp = (m + 3) & ~3;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int wr = warp >> 1, wc = warp & 1, g = lane >> 2, t = lane & 3;
+    double c[2][4][2], snap[2][4][2];
+    if (STAT) {
+        {   // stage both tiles (zero padding in k and past the matrix edge) and their squared norms, as gram_projected_dmma_kernel
+            const int r = threadIdx.x >> 2, l4 = threadIdx.x & 3;
+            const bool vr = row0 + r < n, vc = col0 + r < n;
+            const double* sr = F + (size_t)min(row0 + r, n - 1) * m;
+            const double* sc = F + (size_t)min(col0 + r, n - 1) * m;
+            double pr = 0.0, pc = 0.0;
+            for (int k = l4; k < mp; k += 4) {
+                const double a = (k < m && vr) ? sr[k] : 0.0, b = (k < m && vc) ? sc[k] : 0.0;
+                Fr[r * G2_PITCH + k] = a; Fc[r * G2_PITCH + k] = b;
+                pr = fma(a, a, pr); pc = fma(b, b, pc);
+            }
+            pr += __shfl_xor_sync(0xffffffffu, pr, 1); pr += __shfl_xor_sync(0xffffffffu, pr, 2);
+            pc += __shfl_xor_sync(0xffffffffu, pc, 1); pc += __shfl_xor_sync(0xffffffffu, pc, 2);
+            if (l4 == 0) { nr[r] = pr; nr[PW_TILE + r] = pc; }
+        }
+        __syncthreads();
+        const double* fr = Fr + (wr * 16 + g) * G2_PITCH + t;
+        const double* fc = Fc + (wc * 32 + g) * G2_PITCH + t;
+        const double n0 = nr[wr * 16 + g], n1 = nr[wr * 16 + 8 + g];
+#pragma unroll
+        for (int cb = 0; cb < 4; ++cb) {
+            const double2 nc = *reinterpret_cast<const double2*>(&nr[PW_TILE + wc * 32 + cb * 8 + 2 * t]);
+            c[0][cb][0] = -(n0 + nc.x); c[0][cb][1] = -(n0 + nc.y);
+            c[1][cb][0] = -(n1 + nc.x); c[1][cb][1] = -(n1 + nc.y);
+#pragma unroll
+            for (int rb = 0; rb < 2; ++rb)
+#pragma unroll
+                for (int e = 0; e < 2; ++e) snap[rb][cb][e] = 4e-15 * c[rb][cb][e];
+        }
+        for (int kk = 0; kk < (mp >> 2); ++kk) {           // -d^2 = 2 f.g - |f|^2 - |g|^2
+            const double a0 = 2.0 * fr[kk * 4], a1 = 2.0 * fr[8 * G2_PITCH + kk * 4];
+            double b[4];
+#pragma unroll
+            for (int cb = 0; cb < 4; ++cb) b[cb] = fc[cb * 8 * G2_PITCH + kk * 4];
+#pragma unroll
+            for (int cb = 0; cb < 4; ++cb) {
+                dmma884(c[0][cb][0], c[0][cb][1], a0, b[cb]);
+                dmma884(c[1][cb][0], c[1][cb][1], a1, b[cb]);
+            }
+        }
+    }
+    double p0 = 0.0, p1 = 0.0;
+#pragma unroll
+    for (int rb = 0; rb < 2; ++rb) {
+        const int r = row0 + wr * 16 + rb * 8 + g;
+        const double ar = r < n ? alpha[r] : 0.0;
+#pragma unroll
+        for (int cb = 0; cb < 4; ++cb) {
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                const int cc = col0 + wc * 32 + cb * 8 + 2 * t + e;
+                if (r >= n || cc > r) continue;
+                double w0, w1;
+                if (STAT) {
+                    double x = c[rb][cb][e];
+                    x = (x > snap[rb][cb][e] || r == cc) ? 0.0 : x;
+                    outer_hyper_terms<OUTER>(-x, hyp, w0, w1);
+                    if (snap[rb][cb][e] != snap[rb][cb][e]) w0 = w1 = snap[rb][cb][e];     // NaN features reach the result
+                } else {
+                    outer_hyper_terms<OUTER>(0.0, hyp, w0, w1);
+                }
+                const double bw = (r == cc ? 1.0 : 2.0) * (Ainv[(size_t)r * ld + cc] - ar * alpha[cc]);
+                p0 = fma(bw, w0, p0);
+                p1 = fma(bw, w1, p1);
+            }
+        }
+    }
+    p0 = warp_sum(p0);
+    p1 = warp_sum(p1);
+    if (lane == 0) { s_red[0][warp] = p0; s_red[1][warp] = p1; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double s0 = 0.0, s1 = 0.0;
+#pragma unroll
+        for (int w = 0; w < PW_THREADS / 32; ++w) { s0 += s_red[0][w]; s1 += s_red[1][w]; }
+        partial[(size_t)blockIdx.x * 2] = c0 * s0;
+        partial[(size_t)blockIdx.x * 2 + 1] = c1 * s1;
+    }
+}
+
+// out = sigma tr(B) = sigma sum_j (A^-1_jj - alpha_j^2): strided per thread, then a fixed tree
+__global__ void __launch_bounds__(256) grad_noise_kernel(const double* __restrict__ Ainv, int ld, const double* __restrict__ alpha, int n,
+                                                         double sigma, double* __restrict__ out) {
+    __shared__ double s[256];
+    double acc = 0.0;
+    for (int j = threadIdx.x; j < n; j += 256) acc += Ainv[(size_t)j * ld + j] - alpha[j] * alpha[j];
+    s[threadIdx.x] = acc;
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {
+        if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *out = sigma * s[0];
+}
+
 static inline int grad_tiles(int n) {
     const int t = (n + PW_TILE - 1) / PW_TILE;
     return t * (t + 1) / 2;
@@ -516,6 +634,54 @@ int dqgp_grad_projected(int outer, const double* h_hyp, const double* d_Ainv, in
     DQGP_LAUNCH_CHECK("grad_projected_dmma_kernel");
     grad_reduce_kernel<<<P, 256, 0, st>>>(partial, tiles, P, 0.5 / (2.0 * h), d_grad);
     DQGP_LAUNCH_CHECK("grad_reduce_kernel");
+    return 0;
+}
+
+size_t dqgp_grad_outer_hyperparameters_workspace_bytes(int n) {
+    if (n <= 0) return 0;
+    return sizeof(double) * 2 * (size_t)dqgp::grad_tiles(n);
+}
+
+int dqgp_grad_outer_hyperparameters(int outer, const double* h_hyp, const double* d_Ainv, int ld, const double* d_alpha, const double* d_F,
+                                    int n, int m, double* d_grad, void* d_work, void* stream) {
+    using namespace dqgp;
+    DQGP_REQUIRE(d_Ainv && d_alpha && d_F && d_grad && d_work, "dqgp_grad_outer_hyperparameters: NULL argument");
+    DQGP_REQUIRE(n >= 1 && ld >= n && m >= 1 && m <= PW_MAX_M, "dqgp_grad_outer_hyperparameters: bad shape (n %d, ld %d, m %d)", n, ld, m);
+    OuterHyp hyp;
+    if (make_outer_hyp(outer, h_hyp, &hyp)) return -1;
+    // c0, c1 of outer_hyper_terms, from the values as given in h_hyp (NULL = all 1)
+    const double pi = 3.14159265358979323846;
+    const double h0 = h_hyp ? h_hyp[0] : 1.0;
+    double c0 = 1.0, c1 = 0.0;
+    int count = 1;
+    switch (outer) {
+        case DQGP_OUTER_MATERN15: c0 = hyp.a; break;
+        case DQGP_OUTER_EXPSINE2: c0 = 4.0 * hyp.a * hyp.a * hyp.a; c1 = 4.0 * hyp.a * hyp.a * hyp.b * hyp.b / pi; count = 2; break;
+        case DQGP_OUTER_RATQUAD: c0 = 2.0 * hyp.b / h0; c1 = 1.0; count = 2; break;
+        case DQGP_OUTER_DOTPRODUCT: c0 = 2.0 * h0; break;
+        default: break;
+    }
+    const int tiles = grad_tiles(n);
+    cudaStream_t st = as_stream(stream);
+    double* partial = static_cast<double*>(d_work);
+    switch (outer) {
+#define DQGP_GH(OUT) case OUT: grad_hyper_dmma_kernel<OUT><<<tiles, PW_THREADS, 0, st>>>(d_Ainv, ld, d_alpha, d_F, n, m, hyp, c0, c1, partial); break;
+        DQGP_GH(DQGP_OUTER_GAUSSIAN) DQGP_GH(DQGP_OUTER_MATERN15) DQGP_GH(DQGP_OUTER_EXPSINE2) DQGP_GH(DQGP_OUTER_RATQUAD)
+        DQGP_GH(DQGP_OUTER_DOTPRODUCT)
+#undef DQGP_GH
+    }
+    DQGP_LAUNCH_CHECK("grad_hyper_dmma_kernel");
+    grad_reduce_kernel<<<count, 256, 0, st>>>(partial, tiles, 2, 0.5, d_grad);
+    DQGP_LAUNCH_CHECK("grad_reduce_kernel");
+    return 0;
+}
+
+int dqgp_grad_noise_std(const double* d_Ainv, int ld, const double* d_alpha, int n, double noise_std, double* d_out, void* stream) {
+    using namespace dqgp;
+    DQGP_REQUIRE(d_Ainv && d_alpha && d_out, "dqgp_grad_noise_std: NULL argument");
+    DQGP_REQUIRE(n >= 1 && ld >= n, "dqgp_grad_noise_std: bad shape (n %d, ld %d)", n, ld);
+    grad_noise_kernel<<<1, 256, 0, as_stream(stream)>>>(d_Ainv, ld, d_alpha, n, noise_std, d_out);
+    DQGP_LAUNCH_CHECK("grad_noise_kernel");
     return 0;
 }
 

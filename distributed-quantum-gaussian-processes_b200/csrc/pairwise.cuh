@@ -170,6 +170,39 @@ __device__ __forceinline__ double outer_analytic_weight(double s, const OuterHyp
     }
 }
 
+// The hyper-parameter gradient's per-pair terms (grad_hyper_dmma_kernel) from s = |f_j - f_k|^2 >= 0: dK/dh_0 and dK/dh_1 up to
+// per-kernel constants c_0, c_1 that the host folds into the tile sums (outer_hyper_scales), with d = sqrt(s), a and b as in OuterHyp.
+//   Gaussian {gamma}:                        w0 = -s K                               c0 = 1
+//   Matern 1.5 {l}, k = sqrt(3) a d:         w0 = k^2 e^{-k}                         c0 = a = 1/l
+//   ExpSineSquared {l, p}, z = b d:          w0 = sin^2 z K,  w1 = d sin z cos z K   c0 = 4 a^3,  c1 = 4 a^2 b^2 / pi
+//   RationalQuadratic {l, alpha}, u = a s:   w0 = u/(1+u) K,  w1 = (u/(1+u) - log1p u) K   c0 = 2 alpha / l,  c1 = 1
+//   DotProduct {sigma_0}:                    w0 = 1                                  c0 = 2 sigma_0
+// Every stationary term is exactly 0 at s = 0 (libm sqrt, no guard).  Exponents are clamped at -700.  Not warp-collective.
+template <int OUTER>
+__device__ __forceinline__ void outer_hyper_terms(double s, const OuterHyp& h, double& w0, double& w1) {
+    w1 = 0.0;
+    if (OUTER == DQGP_OUTER_GAUSSIAN) {
+        w0 = -s * fast_exp(fmax(-h.a * s, -700.0));
+    } else if (OUTER == DQGP_OUTER_MATERN15) {
+        const double k = sqrt(s) * h.a * 1.7320508075688772;
+        w0 = (k * k) * fast_exp(fmax(-k, -700.0));
+    } else if (OUTER == DQGP_OUTER_EXPSINE2) {
+        const double d = sqrt(s);
+        double sn, cs;
+        sincos(h.b * d, &sn, &cs);
+        const double K = fast_exp(fmax(-2.0 * (h.a * h.a) * (sn * sn), -700.0));
+        w0 = (sn * sn) * K;
+        w1 = (d * sn * cs) * K;
+    } else if (OUTER == DQGP_OUTER_RATQUAD) {
+        const double u = s * h.a, lp = log1p(u), r = u / (1.0 + u);
+        const double K = fast_exp(fmax(-h.b * lp, -700.0));
+        w0 = r * K;
+        w1 = (r - lp) * K;
+    } else {
+        w0 = 1.0;
+    }
+}
+
 // out[row] = add (+ |F[row]|^2 when with_norm), rows of m features (gram.cu)
 void launch_self_kernel(const double* F, long long rows, int m, double add, bool with_norm, double* out, cudaStream_t st);
 

@@ -24,6 +24,8 @@ from ._lib import OUTER_KERNELS, DqgpError, check
 from .kernels import EncodingCircuit, _require_cuda, dev_f64, outer_hyp, stream_ptr
 
 PERIOD = float(np.pi)
+HYPER_NAMES = {"gaussian": ("gamma",), "matern": ("length_scale",), "expsinesquared": ("length_scale", "periodicity"),
+               "rationalquadratic": ("length_scale", "alpha"), "dotproduct": ("sigma_0",), "pairwisekernel": ()}
 
 
 class _DeviceMatrix:
@@ -71,14 +73,22 @@ class Solver:
 class AgentEngine:
     def __init__(self, X, Y, *, encoding_type, kernel_type, num_qubits, num_layers, noise_std, rho, L,
                  outer_kernel="gaussian", shift_value=np.pi / 8, training_ignores_outer_kernel=True, cholesky_outer_blocks=0,
-                 gradient="central_difference"):
+                 gradient="central_difference", outer_kernel_params=None, hyper_gradient=False):
         """``gradient``: "central_difference" = the reference's rule (dK_i = (K(p + h e_i) - K(p - h e_i)) / 2h, h = pi/8,
         agent_riemannian.py:275) - the parity path; "analytic" (opt-in, SURVEY 8(f) row 3) = the exact derivative of the NLL:
         feature Jacobian from one extra suffix simulation per parameter and ONE pass over the n^2 Gram entries.  The analytic
         mode does NOT reproduce the reference's trajectories (its h = pi/8 difference is far from the derivative).  It takes
         every outer kernel of the projected kernel and the fidelity kernel up to 12 qubits.  It keeps the derivative of every
         sample's state (fidelity) or features (projected) for every parameter resident: P * n * 2^q * 16 bytes for the fidelity
-        kernel, e.g. 5.4 GB at q = 10, n = 8192, P = 40, plus a workspace of about 16 n^2 bytes from 2^q = 128 on."""
+        kernel, e.g. 5.4 GB at q = 10, n = 8192, P = 40, plus a workspace of about 16 n^2 bytes from 2^q = 128 on.
+
+        ``outer_kernel_params``: hyper-parameters of the outer kernel in the reference's format ({"gamma": 0.5},
+        {"length_scale": 0.7, "periodicity": 1.3}, ...; kernels.outer_hyp), used by the training Gram and both gradient modes.
+        None = scikit-learn's defaults.  Only meaningful when the training kernel honours `outer_kernel`: with
+        training_ignores_outer_kernel=True (Gaussian, gamma = 1) or the fidelity kernel a value raises ValueError.
+        ``hyper_gradient``: every gradient() also computes dNLL/dh for the hyper-parameters h of the outer kernel the training
+        Gram uses (the Gaussian's gamma under training_ignores_outer_kernel=True) and dNLL/dsigma for the noise level (a pass over
+        the lower tiles of A^-1 and one over its diagonal); read them with `hyper_gradient()`."""
         _require_cuda()
         self._lib = _lib.load()
         X = np.asarray(X, dtype=np.float64)
@@ -93,8 +103,13 @@ class AgentEngine:
         # Q1: the reference's shifted-kernel workers never receive the outer kernel, so training Grams are
         # always Gaussian(gamma=1); training_ignores_outer_kernel=False honours `outer_kernel` instead.
         self.outer_kernel = "gaussian" if training_ignores_outer_kernel else outer_kernel
+        if outer_kernel_params is not None and (training_ignores_outer_kernel or kernel_type != "projected"):
+            raise ValueError("outer_kernel_params needs kernel_type='projected' and training_ignores_outer_kernel=False: "
+                             "otherwise the training kernel is not the outer kernel they parametrise")
         self._outer_id = OUTER_KERNELS[self.outer_kernel] if kernel_type == "projected" else 0
-        self._hyp = _lib.hyp_array(outer_hyp(self.outer_kernel)) if kernel_type == "projected" else None
+        self._hyp = _lib.hyp_array(outer_hyp(self.outer_kernel, outer_kernel_params)) if kernel_type == "projected" else None
+        # scikit-learn's names of the differentiated hyper-parameters, in h_hyp order (PairwiseKernel(metric="linear") has none)
+        self.hyper_names = list(HYPER_NAMES[self.outer_kernel]) if kernel_type == "projected" else []
         self.noise_std, self.rho, self.L, self.h = float(noise_std), float(rho), float(L), float(shift_value)
         self.d_X = dev_f64(X)
         self.d_Y = dev_f64(np.asarray(Y, dtype=np.float64).reshape(-1))
@@ -121,6 +136,11 @@ class AgentEngine:
         self.d_grad = torch.empty(self.P, **f64)
         self.d_nll = torch.empty(4, **f64)
         self.d_work = torch.empty(max(1, self._lib.dqgp_grad_workspace_bytes(self.n, self.P) // 8), **f64)
+        self.hyper_gradient_enabled = bool(hyper_gradient)
+        if self.hyper_gradient_enabled:
+            # [dNLL/dh in h_hyp order, dNLL/dsigma]
+            self.d_hyper_grad = torch.empty(len(self.hyper_names) + 1, **f64)
+            self.d_work_h = torch.empty(max(1, self._lib.dqgp_grad_outer_hyperparameters_workspace_bytes(self.n) // 8), **f64)
         self.entries_per_step = self.S * self.n * self.n    # SURVEY §8(d): full squares, all 2P+1 sets
         self.share_prefix = True
 
@@ -251,6 +271,23 @@ class AgentEngine:
                   "grad fidelity")
         check(lib.dqgp_nll_terms(self.d_logdet.data_ptr(), self.d_Y.data_ptr(), self.d_alpha.data_ptr(), self.n,
                                  self.d_nll.data_ptr(), st), "nll")
+        if self.hyper_gradient_enabled:
+            k = len(self.hyper_names)
+            if k:
+                check(lib.dqgp_grad_outer_hyperparameters(self._outer_id, self._hyp, s.inverse_ptr, s.ld, self.d_alpha.data_ptr(),
+                                                          self.d_feat.data_ptr(), self.n, self.m, self.d_hyper_grad.data_ptr(),
+                                                          self.d_work_h.data_ptr(), st), "grad outer hyper-parameters")
+            check(lib.dqgp_grad_noise_std(s.inverse_ptr, s.ld, self.d_alpha.data_ptr(), self.n, self.noise_std,
+                                          self.d_hyper_grad[k:].data_ptr(), st), "grad noise_std")
+
+    def hyper_gradient(self):
+        """dNLL/dh of the last gradient() (synchronises): {scikit-learn's hyper-parameter name: value} for the hyper-parameters of
+        the training Gram's outer kernel (none for the fidelity kernel and PairwiseKernel), plus
+        "noise_std": dNLL/dsigma.  Derivatives with respect to log h are h times these."""
+        if not self.hyper_gradient_enabled:
+            raise ValueError("hyper_gradient() needs AgentEngine(..., hyper_gradient=True)")
+        g = self.d_hyper_grad.cpu().numpy()
+        return {**{name: float(v) for name, v in zip(self.hyper_names, g)}, "noise_std": float(g[-1])}
 
     def update(self, d_psi, d_theta_out, d_psi_out):
         # z wrapped to the manifold = row 0 of the parameter-set table (agent_riemannian.py:378)
@@ -273,8 +310,9 @@ class AgentEngine:
         levels = int(np.ceil(np.log2(nblk))) if nblk > 1 else 0
         potrf = self._lib.dqgp_solver_potrf_launches(self.solver.handle) + (1 if nblk > 1 else 0)   # + copy of the panels
         pad = 1 + (1 if self.n % 128 else 0)
+        hyper = (2 * (len(self.hyper_names) > 0) + 1) if self.hyper_gradient_enabled else 0   # (pass, reduce) noise
         return (2 + 2 + pad + potrf + 2 * levels + 3 + 1        # sets, sim, gram, diag, pad, potrf, trtri, solve, lauum
-                + (3 if self.kernel_type == "projected" else 2) + 1 + 1)   # (norms) grad reduce, nll, local update
+                + (3 if self.kernel_type == "projected" else 2) + 1 + 1 + hyper)   # (norms) grad reduce, nll, local update
 
     def check_info(self):
         """Host check of the Cholesky status (syncs).  >0 = index of the first non-positive pivot."""
@@ -417,6 +455,14 @@ class AdmmEngine:
     def replay(self):
         self._graph.replay()
         self._exchange()
+
+    def hyper_gradients(self):
+        """(A_local, k) array of the local agents' last hyper-gradients (synchronises; needs hyper_gradient=True): each row is
+        [dNLL/dh in h_hyp order, dNLL/dsigma] (names in `agents[0].hyper_names` + "noise_std").  Every agent shares the
+        hyper-parameters, so the sum over rows (and over ranks) is the gradient of the summed local NLLs."""
+        if not all(a.hyper_gradient_enabled for a in self.agents):
+            raise ValueError("hyper_gradients() needs AdmmEngine(..., hyper_gradient=True)")
+        return torch.stack([a.d_hyper_grad for a in self.agents]).cpu().numpy()
 
     def state(self):
         """(z, theta, psi, per-agent NLL) on the host (synchronises)."""

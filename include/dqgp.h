@@ -220,6 +220,25 @@ int dqgp_grad_projected_analytic(int outer, const double* h_hyp, const double* d
                                  const double* d_F, const double* d_J, int n, int m, int P, double* d_grad, void* d_work,
                                  void* stream);
 
+/* ---- NLL gradient with respect to the outer kernel's hyper-parameters and the noise level (type-II maximum likelihood; the
+ *      reference has none: it never applies outer-kernel hyper-parameters).  With A = K + sigma^2 I, alpha = A^-1 y,
+ *      B = A^-1 - alpha alpha^T and NLL = 1/2 log det A + 1/2 y^T alpha:
+ *        dNLL/dh = 1/2 sum_jk B_jk dK_jk/dh,   dNLL/dsigma = sigma tr(B),
+ *      h the values exactly as given in h_hyp; the log-space gradient dNLL/dlog h is h times these.  With d = |f_j - f_k|, s = d^2:
+ *        gaussian {gamma}: -s K;   matern (nu = 1.5) {length_scale}: k^2 e^{-k} / l, k = sqrt(3) d / l;
+ *        expsinesquared {length_scale, periodicity}: (4 sin^2(pi d / p) / l^3) K ; (2 pi d / (l^2 p^2)) sin(2 pi d / p) K;
+ *        rationalquadratic {length_scale, alpha}: 2 alpha u K / (l (1 + u)) ; K (u / (1 + u) - log1p(u)), u = s / (2 alpha l^2);
+ *        dotproduct {sigma_0}: 2 sigma_0 (every entry, diagonal included).
+ *      dqgp_grad_outer_hyperparameters: d_grad gets one entry per h_hyp value (1, 1, 2, 2, 1 by outer id), d_F (n, m) the
+ *      features the Gram was built from, m <= 36.  Only A^-1[j][k] with j >= k is read (want_inverse = 1 or 2, or the LU rung);
+ *      duplicates and the diagonal follow the Gram's s = 0 rules; NaN features give NaN (stationary kernels).
+ *      d_work: dqgp_grad_outer_hyperparameters_workspace_bytes(n).  dqgp_grad_noise_std writes d_out[0] = sigma tr(B) for either
+ *      kernel type.  Both only enqueue (no synchronisation, graph-capturable) and are deterministic: a second call gives the same bits. */
+size_t dqgp_grad_outer_hyperparameters_workspace_bytes(int n);
+int dqgp_grad_outer_hyperparameters(int outer, const double* h_hyp, const double* d_Ainv, int ld, const double* d_alpha,
+                                    const double* d_F, int n, int m, double* d_grad, void* d_work, void* stream);
+int dqgp_grad_noise_std(const double* d_Ainv, int ld, const double* d_alpha, int n, double noise_std, double* d_out, void* stream);
+
 /* ---- NLL terms (agent_riemannian.py:441-452): d_out[4] = {1/2 logdet, 1/2 y^T alpha, n/2 log 2pi, total} */
 int dqgp_nll_terms(const double* d_logdet, const double* d_y, const double* d_alpha, int n, double* d_out, void* stream);
 
