@@ -63,17 +63,11 @@ __global__ void admm_consensus_kernel(const double* __restrict__ theta, const do
 // agent_riemannian.py:447-452
 __global__ void nll_terms_kernel(const double* __restrict__ logdet, const double* __restrict__ y, const double* __restrict__ alpha,
                                  int n, double* __restrict__ out) {
-    __shared__ double s[256];
     double acc = 0.0;
     for (int i = threadIdx.x; i < n; i += 256) acc = fma(y[i], alpha[i], acc);
-    s[threadIdx.x] = acc;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o];
-        __syncthreads();
-    }
+    const double ya = block_sum_256(acc);
     if (threadIdx.x == 0) {
-        const double ld = 0.5 * logdet[0], q = 0.5 * s[0], c = 0.5 * n * log(6.283185307179586);
+        const double ld = 0.5 * logdet[0], q = 0.5 * ya, c = 0.5 * n * log(6.283185307179586);
         out[0] = ld; out[1] = q; out[2] = c; out[3] = ld + q + c;
     }
 }
@@ -106,16 +100,10 @@ __global__ void predict_finish_kernel(const double* __restrict__ Kst, int nt, in
     }
 }
 __global__ void mean_kernel(const double* __restrict__ v, int n, double* __restrict__ out) {
-    __shared__ double s[256];
     double acc = 0.0;
     for (int i = threadIdx.x; i < n; i += 256) acc += v[i];
-    s[threadIdx.x] = acc;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) out[0] = s[0] / n;
+    const double sum = block_sum_256(acc);
+    if (threadIdx.x == 0) out[0] = sum / n;
 }
 
 }  // namespace dqgp

@@ -30,6 +30,20 @@ int cuda_fail(cudaError_t e, const char* what);
     } while (0)
 
 static inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
+
+// Raise KERNEL's dynamic shared memory limit to `bytes`.  The attribute belongs to the device, so it is set once per device
+// (on every call for a device id of 64 or more).
+template <auto KERNEL>
+int set_max_dynamic_smem(int bytes) {
+    static bool done[64] = {false};
+    int dev = 0;
+    DQGP_CUDA(cudaGetDevice(&dev));
+    if (dev >= 0 && dev < 64 && done[dev]) return 0;
+    DQGP_CUDA(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    if (dev >= 0 && dev < 64) done[dev] = true;
+    return 0;
+}
+
 int sm_count();
 int circuit_on_device(const dqgp_circuit* c);  // uploads the gate program on first use
 
@@ -94,6 +108,19 @@ __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
+}
+
+// Fixed-order sum over a block of 256 threads, each holding `acc` (its strided partial sum): a halving tree through shared memory,
+// so the result is bit-reproducible run to run.  Every thread gets the sum; call it from all 256 threads.
+__device__ __forceinline__ double block_sum_256(double acc) {
+    __shared__ double s[256];
+    s[threadIdx.x] = acc;
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {
+        if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o];
+        __syncthreads();
+    }
+    return s[0];
 }
 
 }  // namespace dqgp

@@ -59,10 +59,7 @@ __global__ void __launch_bounds__(PW_THREADS, 1) fidelity_dmma_kernel(const doub
     __syncthreads();
     int bi, bj;
     if (MODE != 0) {
-        bi = int((sqrt(8.0 * blockIdx.x + 1.0) - 1.0) * 0.5);
-        while ((bi + 1) * (bi + 2) / 2 <= (int)blockIdx.x) ++bi;
-        while (bi * (bi + 1) / 2 > (int)blockIdx.x) --bi;
-        bj = blockIdx.x - bi * (bi + 1) / 2;
+        tile_from_index(blockIdx.x, bi, bj);
     } else {
         bi = blockIdx.y; bj = blockIdx.x;
     }
@@ -205,22 +202,8 @@ __global__ void __launch_bounds__(PW_THREADS, 1) fidelity_dmma_kernel(const doub
     }
 }
 
-static int fd_attr() {
-    static bool done_dev[64] = {false};      // the attribute is per DEVICE
-    int dev = 0;
-    cudaGetDevice(&dev);
-    bool& done = done_dev[(dev >= 0 && dev < 64) ? dev : 0];
-    if (!done) {
-        DQGP_CUDA(cudaFuncSetAttribute(fidelity_dmma_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FD_SMEM));
-        DQGP_CUDA(cudaFuncSetAttribute(fidelity_dmma_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FD_SMEM));
-        DQGP_CUDA(cudaFuncSetAttribute(fidelity_dmma_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FD_SMEM));
-        done = true;
-    }
-    return 0;
-}
-
 int fidelity_gram_dmma(const double* Psi1, int n1, const double* Psi2, int n2, int dim, double* K, int ldk, cudaStream_t st) {
-    int rc = fd_attr();
+    int rc = set_max_dynamic_smem<fidelity_dmma_kernel<0>>((int)FD_SMEM);
     if (rc) return rc;
     dim3 grid((n2 + PW_TILE - 1) / PW_TILE, (n1 + PW_TILE - 1) / PW_TILE);
     CUtensorMap tmap;                                                       // unused by the Gram (two state arrays): per-row bulk copies
@@ -232,7 +215,7 @@ int fidelity_gram_dmma(const double* Psi1, int n1, const double* Psi2, int n2, i
 
 int fidelity_grad_dmma(const double* Ainv, int ld, const double* alpha, const double* Psi, int n, int dim, int P, double* partial,
                        int tiles, cudaStream_t st) {
-    int rc = fd_attr();
+    int rc = set_max_dynamic_smem<fidelity_dmma_kernel<1>>((int)FD_SMEM);
     if (rc) return rc;
     // the state tiles of a parameter set as two boxes of a 3-D tensor map (one issuing thread).  For the arguments the entry point
     // accepts (16-byte aligned base, 16 dim-byte rows, box of 36 x 64, dimensions below 2^32) the driver has no reason to refuse it.
@@ -247,7 +230,7 @@ int fidelity_grad_dmma(const double* Ainv, int ld, const double* alpha, const do
 
 int fidelity_weights_dmma(const double* Ainv, int ld, const double* alpha, const double* Psi, int n, int dim, double* W, int n_pad,
                           cudaStream_t st) {
-    int rc = fd_attr();
+    int rc = set_max_dynamic_smem<fidelity_dmma_kernel<2>>((int)FD_SMEM);
     if (rc) return rc;
     CUtensorMap tmap;
     memset(&tmap, 0, sizeof(tmap));

@@ -218,15 +218,10 @@ __device__ __forceinline__ void gemm_tile(const GemmTask& T, int local, double* 
 }
 
 int gemm_init() {
-    static bool done[64] = {false};
-    int dev = 0;
-    DQGP_CUDA(cudaGetDevice(&dev));
-    if (dev >= 0 && dev < 64 && done[dev]) return 0;
-    DQGP_CUDA(cudaFuncSetAttribute(gemm_group_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GemmBig::SMEM_BYTES));
-    DQGP_CUDA(cudaFuncSetAttribute(gemm_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GemmSmall::SMEM_BYTES));
-    DQGP_CUDA(cudaFuncSetAttribute(gemm_group_tmap_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GemmBig::SMEM_BYTES + 128));
-    if (dev >= 0 && dev < 64) done[dev] = true;
-    return 0;
+    int rc = set_max_dynamic_smem<gemm_group_kernel>((int)GemmBig::SMEM_BYTES);
+    if (!rc) rc = set_max_dynamic_smem<gemm_small_kernel>((int)GemmSmall::SMEM_BYTES);
+    if (!rc) rc = set_max_dynamic_smem<gemm_group_tmap_kernel>((int)GemmBig::SMEM_BYTES + 128);
+    return rc;
 }
 
 // ---- tensor maps: registered task tables -> device arrays of (A map, B map) per task -----------------------------------------

@@ -15,13 +15,6 @@
 
 namespace dqgp {
 
-__device__ __forceinline__ void tile_from_index(int local, int& bi, int& bj) {
-    bi = int((sqrt(8.0 * local + 1.0) - 1.0) * 0.5);
-    while ((bi + 1) * (bi + 2) / 2 <= local) ++bi;
-    while (bi * (bi + 1) / 2 > local) --bi;
-    bj = local - bi * (bi + 1) / 2;
-}
-
 // ---- v2: Gram-identity formulation on the DMMA pipe ---------------------------------------------------------------
 // -gamma*||f-g||^2 = 2*gamma*f.g - gamma*||f||^2 - gamma*||g||^2: the accumulator of an 8x8 DMMA block is
 // initialised with the (pre-scaled) norms, the row operand is scaled by 2*gamma at fragment load, and m/4
@@ -101,7 +94,7 @@ __global__ void __launch_bounds__(PW_THREADS, 2) grad_projected_dmma_kernel(cons
         __syncthreads();
     }
     constexpr bool STAT = outer_is_stationary(OUTER);
-    const double gam = (OUTER == DQGP_OUTER_GAUSSIAN) ? hyp.a * DQGP_EXP_S32 : 1.0;      // Gaussian: argument in units of ln2/32
+    const double gam = outer_grad_gamma_eff(OUTER, hyp);                               // Gaussian: argument in units of ln2/32
     const double a_scale = STAT ? 2.0 * gam : 1.0;                                      // dot product: sigma_0^2 + f.g
     const double tab = exp_table_entry();
 
@@ -225,17 +218,11 @@ __global__ void feature_norms_kernel(const double* __restrict__ F, long long row
 // grad[i] = scale * sum_tiles partial[tile][i], fixed summation order (strided per thread, then a fixed tree)
 __global__ void __launch_bounds__(256) grad_reduce_kernel(const double* __restrict__ partial, int n_tiles, int P, double scale,
                                                           double* __restrict__ grad) {
-    __shared__ double s[256];
     const int i = blockIdx.x;
     double acc = 0.0;
     for (int t = threadIdx.x; t < n_tiles; t += 256) acc += partial[(size_t)t * P + i];
-    s[threadIdx.x] = acc;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) grad[i] = scale * s[0];
+    const double sum = block_sum_256(acc);
+    if (threadIdx.x == 0) grad[i] = scale * sum;
 }
 
 // ---- analytic gradient (opt-in; SURVEY 8(f) row 3: NOT the reference's central difference, Q3) -------------------------------
@@ -307,17 +294,11 @@ __global__ void grad_analytic_sum_kernel(const double* __restrict__ Gpart, size_
 // grad[i] = scale * <J_i, G>  (n*m products, strided per thread then a fixed tree)
 __global__ void __launch_bounds__(256) grad_analytic_contract_kernel(const double* __restrict__ J, const double* __restrict__ G, size_t count,
                                                                      double scale, double* __restrict__ grad) {
-    __shared__ double sred[256];
     const double* Ji = J + (size_t)blockIdx.x * count;
     double acc = 0.0;
     for (size_t e = threadIdx.x; e < count; e += 256) acc = fma(Ji[e], G[e], acc);
-    sred[threadIdx.x] = acc;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) sred[threadIdx.x] += sred[threadIdx.x + o];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) grad[blockIdx.x] = scale * sred[0];
+    const double sum = block_sum_256(acc);
+    if (threadIdx.x == 0) grad[blockIdx.x] = scale * sum;
 }
 
 // Fidelity kernel, analytic gradient: K_jk = |s_jk|^2, s_jk = <psi_k|psi_j>, and with d_i psi_j from dqgp_states_jacobian
@@ -400,20 +381,14 @@ __global__ void grad_fid_pack_kernel(const double2* __restrict__ Psi, int n, int
 constexpr int GFD_SLICES = 64;
 __global__ void __launch_bounds__(256) grad_fid_contract_kernel(const double* __restrict__ D, const double* __restrict__ G, size_t count, int P,
                                                                 double* __restrict__ partial) {
-    __shared__ double sred[256];
     const size_t per = (count + gridDim.x - 1) / gridDim.x;
     const size_t b = (size_t)blockIdx.x * per, e = min(count, b + per);
     const double* Di = D + (size_t)blockIdx.y * count;
     double acc = 0.0;
 #pragma unroll 4
     for (size_t k = b + threadIdx.x; k < e; k += 256) acc = fma(Di[k], G[k], acc);
-    sred[threadIdx.x] = acc;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) sred[threadIdx.x] += sred[threadIdx.x + o];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) partial[(size_t)blockIdx.x * P + blockIdx.y] = sred[0];
+    const double sum = block_sum_256(acc);
+    if (threadIdx.x == 0) partial[(size_t)blockIdx.x * P + blockIdx.y] = sum;
 }
 // the task table is written on the device so the entry point stays capturable into a CUDA graph (a host copy would synchronise)
 __global__ void grad_fid_task_kernel(GemmTask t, GemmTask* __restrict__ dst) { *dst = t; }
@@ -441,21 +416,7 @@ __global__ void __launch_bounds__(PW_THREADS) grad_hyper_dmma_kernel(const doubl
     const int wr = warp >> 1, wc = warp & 1, g = lane >> 2, t = lane & 3;
     double c[2][4][2], snap[2][4][2];
     if (STAT) {
-        {   // stage both tiles (zero padding in k and past the matrix edge) and their squared norms, as gram_projected_dmma_kernel
-            const int r = threadIdx.x >> 2, l4 = threadIdx.x & 3;
-            const bool vr = row0 + r < n, vc = col0 + r < n;
-            const double* sr = F + (size_t)min(row0 + r, n - 1) * m;
-            const double* sc = F + (size_t)min(col0 + r, n - 1) * m;
-            double pr = 0.0, pc = 0.0;
-            for (int k = l4; k < mp; k += 4) {
-                const double a = (k < m && vr) ? sr[k] : 0.0, b = (k < m && vc) ? sc[k] : 0.0;
-                Fr[r * G2_PITCH + k] = a; Fc[r * G2_PITCH + k] = b;
-                pr = fma(a, a, pr); pc = fma(b, b, pc);
-            }
-            pr += __shfl_xor_sync(0xffffffffu, pr, 1); pr += __shfl_xor_sync(0xffffffffu, pr, 2);
-            pc += __shfl_xor_sync(0xffffffffu, pc, 1); pc += __shfl_xor_sync(0xffffffffu, pc, 2);
-            if (l4 == 0) { nr[r] = pr; nr[PW_TILE + r] = pc; }
-        }
+        pw_stage_two_tiles(Fr, Fc, nr, F, n, F, n, m, mp, row0, col0, threadIdx.x);
         __syncthreads();
         const double* fr = Fr + (wr * 16 + g) * G2_PITCH + t;
         const double* fc = Fc + (wc * 32 + g) * G2_PITCH + t;
@@ -524,16 +485,10 @@ __global__ void __launch_bounds__(PW_THREADS) grad_hyper_dmma_kernel(const doubl
 // out = sigma tr(B) = sigma sum_j (A^-1_jj - alpha_j^2): strided per thread, then a fixed tree
 __global__ void __launch_bounds__(256) grad_noise_kernel(const double* __restrict__ Ainv, int ld, const double* __restrict__ alpha, int n,
                                                          double sigma, double* __restrict__ out) {
-    __shared__ double s[256];
     double acc = 0.0;
     for (int j = threadIdx.x; j < n; j += 256) acc += Ainv[(size_t)j * ld + j] - alpha[j] * alpha[j];
-    s[threadIdx.x] = acc;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) *out = sigma * s[0];
+    const double sum = block_sum_256(acc);
+    if (threadIdx.x == 0) *out = sigma * sum;
 }
 
 static inline int grad_tiles(int n) {
@@ -573,17 +528,11 @@ int dqgp_grad_projected(int outer, const double* h_hyp, const double* d_Ainv, in
     double* partial = static_cast<double*>(d_work);
     double* norms = partial + (size_t)tiles * P;
     const long long rows = (long long)(2 * P + 1) * n;
-    // the norms arrive pre-multiplied by -gamma_eff (and, Gaussian, by 32/ln2: the exponent's argument then leaves the DMMA in the
-    // units its range reduction wants): the kernel only adds them.  The dot product's "norms" are sigma_0^2 / 2 each, so the
-    // accumulator starts at exactly sigma_0^2.
-    const double gam_eff = (outer == DQGP_OUTER_GAUSSIAN) ? hyp.a * DQGP_EXP_S32 : 1.0;
-    if (outer_is_stationary(outer)) feature_norms_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(d_F, rows, m, -gam_eff, norms);
-    else launch_self_kernel(nullptr, rows, m, 0.5 * hyp.a, false, norms, st);
-    // Pauli features lie in [-1, 1]: gamma d^2 <= 4 m gamma, so the exponent guard is only needed for large gamma
-    // the exponent's argument is bounded below by -gamma 4m (Gaussian), -sqrt(3) 2 sqrt(m) / l (Matern), -2 / l^2 (ExpSineSquared)
-    const double worst = outer == DQGP_OUTER_GAUSSIAN ? 4.0 * m * hyp.a
-                         : outer == DQGP_OUTER_MATERN15 ? 1.7320508075688772 * 2.0 * sqrt((double)m) * hyp.a : 2.0 * hyp.a * hyp.a;
-    const bool no_clamp = hyp.a > 0.0 && worst < 650.0;
+    // the norms arrive pre-multiplied by -gamma_eff: the kernel only adds them (outer_grad_gamma_eff, outer_grad_dot_norm)
+    if (outer_is_stationary(outer))
+        feature_norms_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(d_F, rows, m, -outer_grad_gamma_eff(outer, hyp), norms);
+    else launch_self_kernel(nullptr, rows, m, outer_grad_dot_norm(hyp), false, norms, st);
+    const bool no_clamp = outer_grad_no_clamp(outer, hyp, m);
     // feature tiles as two boxes of a 3-D tensor map per parameter set (one thread issues them); odd m (rows not 16-byte multiples),
     // a misaligned d_F or a map the driver refuses take the per-thread cp.async kernel, with the exponent guard (CLAMP only changes
     // results below -700, where no_clamp is never set, so both kernels give the same gradient)
@@ -591,46 +540,23 @@ int dqgp_grad_projected(int outer, const double* h_hyp, const double* d_Ainv, in
     memset(&tmap, 0, sizeof(tmap));
     const bool have_tmap = (m & 1) == 0 && (reinterpret_cast<uintptr_t>(d_F) & 15) == 0 &&
                            make_rows_tensor_map(&tmap, d_F, m, n, 2 * P + 1, G2_PITCH, PW_TILE);
-#define DQGP_G2(OUT)                                                                                                         \
-    do {                                                                                                                     \
-        static bool attr_done_dev[64] = {false};        /* the attribute is per DEVICE (as gemm_init's flags) */            \
-        int dev_ = 0;                                                                                                        \
-        cudaGetDevice(&dev_);                                                                                                \
-        bool& attr_done = attr_done_dev[(dev_ >= 0 && dev_ < 64) ? dev_ : 0];                                                \
-        if (!attr_done) {                                                                                                    \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
-            attr_done = true;                                                                                                \
-        }                                                                                                                    \
-        if (have_tmap && no_clamp) grad_projected_dmma_kernel<OUT, false, true><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-        else if (have_tmap) grad_projected_dmma_kernel<OUT, true, true><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-        else grad_projected_dmma_kernel<OUT, true, false><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-    } while (0)
-    // RationalQuadratic and DotProduct have no exponent to guard: only their CLAMP = false kernels exist, one per staging path
-#define DQGP_G2_NOEXP(OUT)                                                                                                   \
-    do {                                                                                                                     \
-        static bool attr_done_dev[64] = {false};                                                                             \
-        int dev_ = 0;                                                                                                        \
-        cudaGetDevice(&dev_);                                                                                                \
-        bool& attr_done = attr_done_dev[(dev_ >= 0 && dev_ < 64) ? dev_ : 0];                                                \
-        if (!attr_done) {                                                                                                    \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
-            DQGP_CUDA(cudaFuncSetAttribute(grad_projected_dmma_kernel<OUT, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM)); \
-            attr_done = true;                                                                                                \
-        }                                                                                                                    \
-        if (have_tmap) grad_projected_dmma_kernel<OUT, false, true><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-        else grad_projected_dmma_kernel<OUT, false, false><<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap); \
-    } while (0)
-    switch (outer) {
-        case DQGP_OUTER_GAUSSIAN: DQGP_G2(DQGP_OUTER_GAUSSIAN); break;
-        case DQGP_OUTER_MATERN15: DQGP_G2(DQGP_OUTER_MATERN15); break;
-        case DQGP_OUTER_RATQUAD: DQGP_G2_NOEXP(DQGP_OUTER_RATQUAD); break;
-        case DQGP_OUTER_DOTPRODUCT: DQGP_G2_NOEXP(DQGP_OUTER_DOTPRODUCT); break;
-        default: DQGP_G2(DQGP_OUTER_EXPSINE2); break;
-    }
-#undef DQGP_G2_NOEXP
-#undef DQGP_G2
+    const int rc = with_outer(outer, [&](auto o) {
+        constexpr int OUTER = decltype(o)::value;
+        auto launch = [&](auto clamp, auto tma) {
+            constexpr auto kernel = grad_projected_dmma_kernel<OUTER, decltype(clamp)::value, decltype(tma)::value>;
+            const int e = set_max_dynamic_smem<kernel>((int)G2_SMEM);
+            if (!e) kernel<<<tiles, PW_THREADS, G2_SMEM, st>>>(d_Ainv, ld, d_alpha, d_F, norms, n, m, P, hyp, partial, tmap);
+            return e;
+        };
+        // an outer kernel without an exponent has only its CLAMP = false forms, one per staging path
+        if constexpr (outer_has_exponent(OUTER)) {
+            if (have_tmap && no_clamp) return launch(std::false_type{}, std::true_type{});
+            return have_tmap ? launch(std::true_type{}, std::true_type{}) : launch(std::true_type{}, std::false_type{});
+        } else {
+            return have_tmap ? launch(std::false_type{}, std::true_type{}) : launch(std::false_type{}, std::false_type{});
+        }
+    });
+    if (rc) return rc;
     DQGP_LAUNCH_CHECK("grad_projected_dmma_kernel");
     grad_reduce_kernel<<<P, 256, 0, st>>>(partial, tiles, P, 0.5 / (2.0 * h), d_grad);
     DQGP_LAUNCH_CHECK("grad_reduce_kernel");
@@ -649,27 +575,14 @@ int dqgp_grad_outer_hyperparameters(int outer, const double* h_hyp, const double
     DQGP_REQUIRE(n >= 1 && ld >= n && m >= 1 && m <= PW_MAX_M, "dqgp_grad_outer_hyperparameters: bad shape (n %d, ld %d, m %d)", n, ld, m);
     OuterHyp hyp;
     if (make_outer_hyp(outer, h_hyp, &hyp)) return -1;
-    // c0, c1 of outer_hyper_terms, from the values as given in h_hyp (NULL = all 1)
-    const double pi = 3.14159265358979323846;
-    const double h0 = h_hyp ? h_hyp[0] : 1.0;
-    double c0 = 1.0, c1 = 0.0;
-    int count = 1;
-    switch (outer) {
-        case DQGP_OUTER_MATERN15: c0 = hyp.a; break;
-        case DQGP_OUTER_EXPSINE2: c0 = 4.0 * hyp.a * hyp.a * hyp.a; c1 = 4.0 * hyp.a * hyp.a * hyp.b * hyp.b / pi; count = 2; break;
-        case DQGP_OUTER_RATQUAD: c0 = 2.0 * hyp.b / h0; c1 = 1.0; count = 2; break;
-        case DQGP_OUTER_DOTPRODUCT: c0 = 2.0 * h0; break;
-        default: break;
-    }
+    double c0, c1;
+    const int count = outer_hyper_scales(outer, hyp, h_hyp, c0, c1);
     const int tiles = grad_tiles(n);
     cudaStream_t st = as_stream(stream);
     double* partial = static_cast<double*>(d_work);
-    switch (outer) {
-#define DQGP_GH(OUT) case OUT: grad_hyper_dmma_kernel<OUT><<<tiles, PW_THREADS, 0, st>>>(d_Ainv, ld, d_alpha, d_F, n, m, hyp, c0, c1, partial); break;
-        DQGP_GH(DQGP_OUTER_GAUSSIAN) DQGP_GH(DQGP_OUTER_MATERN15) DQGP_GH(DQGP_OUTER_EXPSINE2) DQGP_GH(DQGP_OUTER_RATQUAD)
-        DQGP_GH(DQGP_OUTER_DOTPRODUCT)
-#undef DQGP_GH
-    }
+    with_outer(outer, [&](auto o) {
+        grad_hyper_dmma_kernel<decltype(o)::value><<<tiles, PW_THREADS, 0, st>>>(d_Ainv, ld, d_alpha, d_F, n, m, hyp, c0, c1, partial);
+    });
     DQGP_LAUNCH_CHECK("grad_hyper_dmma_kernel");
     grad_reduce_kernel<<<count, 256, 0, st>>>(partial, tiles, 2, 0.5, d_grad);
     DQGP_LAUNCH_CHECK("grad_reduce_kernel");
@@ -703,27 +616,16 @@ int dqgp_grad_projected_analytic(int outer, const double* h_hyp, const double* d
     const int seg_cols = ((n + GA_SEGMENTS - 1) / GA_SEGMENTS + GA_CHUNK - 1) / GA_CHUNK * GA_CHUNK;
     const int segments = (n + seg_cols - 1) / seg_cols;
     dim3 grid((n + GA_ROWS - 1) / GA_ROWS, segments);
-    double scale = 2.0;                        // stationary: 2 sum_j <J_j, G_j>
-    switch (outer) {
-        case DQGP_OUTER_GAUSSIAN:
-            launch_grad_analytic_rows<DQGP_OUTER_GAUSSIAN, false>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart);
-            scale = -2.0 * hyp.a;              // the weight is e^{-gamma s}: kappa' = -gamma e^{-gamma s}
-            break;
-        case DQGP_OUTER_MATERN15: launch_grad_analytic_rows<DQGP_OUTER_MATERN15, false>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart); break;
-        case DQGP_OUTER_EXPSINE2: launch_grad_analytic_rows<DQGP_OUTER_EXPSINE2, false>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart); break;
-        case DQGP_OUTER_RATQUAD:
-            if (hyp.b == 1.0) launch_grad_analytic_rows<DQGP_OUTER_RATQUAD, true>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart);
-            else launch_grad_analytic_rows<DQGP_OUTER_RATQUAD, false>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart);
-            break;
-        default:                               // DQGP_OUTER_DOTPRODUCT: make_outer_hyp refused every other id
-            launch_grad_analytic_rows<DQGP_OUTER_DOTPRODUCT, false>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart);
-            scale = 1.0;                       // sum_j <J_j, (B F)_j>
-            break;
-    }
+    with_outer(outer, [&](auto o) {
+        constexpr int OUTER = decltype(o)::value;
+        if (outer_analytic_alpha1(OUTER, hyp))
+            launch_grad_analytic_rows<OUTER, outer_has_alpha1_form(OUTER)>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart);
+        else launch_grad_analytic_rows<OUTER, false>(m, grid, st, d_Ainv, ld, d_alpha, d_F, n, hyp, seg_cols, Gpart);
+    });
     DQGP_LAUNCH_CHECK("grad_analytic_rows_kernel");
     const size_t count = (size_t)n * m;
     grad_analytic_sum_kernel<<<(unsigned)((count + 255) / 256), 256, 0, st>>>(Gpart, count, segments, G);
-    grad_analytic_contract_kernel<<<P, 256, 0, st>>>(d_J, G, count, scale, d_grad);
+    grad_analytic_contract_kernel<<<P, 256, 0, st>>>(d_J, G, count, outer_analytic_scale(outer, hyp), d_grad);
     DQGP_LAUNCH_CHECK("grad_analytic kernels");
     return 0;
 }

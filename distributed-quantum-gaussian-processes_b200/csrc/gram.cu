@@ -22,30 +22,13 @@ __global__ void __launch_bounds__(PW_THREADS) gram_projected_dmma_kernel(const d
     __shared__ __align__(16) double nr[2 * PW_TILE];
     int bi, bj;
     if (SYM) {
-        bi = int((sqrt(8.0 * blockIdx.x + 1.0) - 1.0) * 0.5);
-        while ((bi + 1) * (bi + 2) / 2 <= (int)blockIdx.x) ++bi;
-        while (bi * (bi + 1) / 2 > (int)blockIdx.x) --bi;
-        bj = blockIdx.x - bi * (bi + 1) / 2;
+        tile_from_index(blockIdx.x, bi, bj);
     } else {
         bi = blockIdx.y; bj = blockIdx.x;
     }
     const int row0 = bi * PW_TILE, col0 = bj * PW_TILE;
     const int mp = (m + 3) & ~3;
-    {   // stage both tiles (zero padding in k and past the matrix edge) and their squared norms
-        const int r = threadIdx.x >> 2, l4 = threadIdx.x & 3;
-        const bool vr = row0 + r < n1, vc = col0 + r < n2;
-        const double* sr = F1 + (size_t)min(row0 + r, n1 - 1) * m;
-        const double* sc = F2 + (size_t)min(col0 + r, n2 - 1) * m;
-        double pr = 0.0, pc = 0.0;
-        for (int k = l4; k < mp; k += 4) {
-            const double a = (k < m && vr) ? sr[k] : 0.0, b = (k < m && vc) ? sc[k] : 0.0;
-            Fr[r * G2_PITCH + k] = a; Fc[r * G2_PITCH + k] = b;
-            pr = fma(a, a, pr); pc = fma(b, b, pc);
-        }
-        pr += __shfl_xor_sync(0xffffffffu, pr, 1); pr += __shfl_xor_sync(0xffffffffu, pr, 2);
-        pc += __shfl_xor_sync(0xffffffffu, pc, 1); pc += __shfl_xor_sync(0xffffffffu, pc, 2);
-        if (l4 == 0) { nr[r] = pr; nr[PW_TILE + r] = pc; }
-    }
+    pw_stage_two_tiles(Fr, Fc, nr, F1, n1, F2, n2, m, mp, row0, col0, threadIdx.x);
     __syncthreads();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int wr = warp >> 1, wc = warp & 1, g = lane >> 2, t = lane & 3;
@@ -156,20 +139,12 @@ int dqgp_gram_projected(int outer, const double* h_hyp, const double* d_F1, int 
     cudaStream_t st = as_stream(stream);
     const bool sym = same && d_F1 == d_F2 && n1 == n2;
     const int tsym = grid.y * (grid.y + 1) / 2;
-#define DQGP_GRAM(OUT)                                                                                                     \
-    do {                                                                                                                   \
-        if (sym && same == 2) gram_projected_dmma_kernel<OUT, 2><<<tsym, PW_THREADS, 0, st>>>(d_F1, n1, d_F2, n2, m, hyp, d_K, ldk); \
-        else if (sym) gram_projected_dmma_kernel<OUT, 1><<<tsym, PW_THREADS, 0, st>>>(d_F1, n1, d_F2, n2, m, hyp, d_K, ldk); \
-        else gram_projected_dmma_kernel<OUT, 0><<<grid, PW_THREADS, 0, st>>>(d_F1, n1, d_F2, n2, m, hyp, d_K, ldk);        \
-    } while (0)
-    switch (outer) {
-        case DQGP_OUTER_GAUSSIAN: DQGP_GRAM(DQGP_OUTER_GAUSSIAN); break;
-        case DQGP_OUTER_MATERN15: DQGP_GRAM(DQGP_OUTER_MATERN15); break;
-        case DQGP_OUTER_RATQUAD: DQGP_GRAM(DQGP_OUTER_RATQUAD); break;
-        case DQGP_OUTER_DOTPRODUCT: DQGP_GRAM(DQGP_OUTER_DOTPRODUCT); break;
-        default: DQGP_GRAM(DQGP_OUTER_EXPSINE2); break;
-    }
-#undef DQGP_GRAM
+    with_outer(outer, [&](auto o) {
+        constexpr int OUTER = decltype(o)::value;
+        if (sym && same == 2) gram_projected_dmma_kernel<OUTER, 2><<<tsym, PW_THREADS, 0, st>>>(d_F1, n1, d_F2, n2, m, hyp, d_K, ldk);
+        else if (sym) gram_projected_dmma_kernel<OUTER, 1><<<tsym, PW_THREADS, 0, st>>>(d_F1, n1, d_F2, n2, m, hyp, d_K, ldk);
+        else gram_projected_dmma_kernel<OUTER, 0><<<grid, PW_THREADS, 0, st>>>(d_F1, n1, d_F2, n2, m, hyp, d_K, ldk);
+    });
     DQGP_LAUNCH_CHECK("gram_projected_dmma_kernel");
     return 0;
 }

@@ -303,13 +303,8 @@ int dqgp_lu_solve_inv(double* d_A, int lda, int n, const double* d_y, double* d_
     if (d_slogdet) lu_slogdet_kernel<<<1, 256, 0, st>>>(d_A, lda, n, piv, d_slogdet);
     if (!d_Ainv && !d_y) return 0;
     if ((size_t)n * sizeof(int) <= 160 * 1024) {
-        static bool attr_dev[64] = {false};
-        int dev = 0;
-        cudaGetDevice(&dev);
-        if (dev >= 0 && dev < 64 && !attr_dev[dev]) {
-            DQGP_CUDA(cudaFuncSetAttribute(lu_perm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-            attr_dev[dev] = true;
-        }
+        int rc = set_max_dynamic_smem<lu_perm_kernel>(160 * 1024);
+        if (rc) return rc;
         lu_perm_kernel<<<1, 256, (size_t)n * sizeof(int), st>>>(piv, n, perm);
     } else {
         lu_perm_global_kernel<<<1, 256, 0, st>>>(piv, n, perm);

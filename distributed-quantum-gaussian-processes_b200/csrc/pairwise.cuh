@@ -3,6 +3,7 @@
 // A CTA of 256 threads owns a 64x64 tile of (row sample j, column sample k) pairs; its 8 warps (4x2) each own a
 // 16x32 sub-tile as 2x4 DMMA 8x8 blocks.  Sample rows live in shared memory [sample][feature] with pitch G2_PITCH.
 #pragma once
+#include <type_traits>
 #include "common.cuh"
 #include "fastmath.cuh"
 
@@ -11,6 +12,7 @@ namespace dqgp {
 constexpr int PW_TILE = 64;
 constexpr int PW_THREADS = 256;
 constexpr int PW_MAX_M = 3 * MAX_QUBITS;
+constexpr int G2_PITCH = 36;   // doubles per staged sample row: = 4 (mod 16) -> conflict-free DMMA fragment loads
 
 struct OuterHyp {
     double a;   // gaussian: gamma        | matern: 1/length_scale | expsine2: 1/length_scale   | ratquad: 1/(2 alpha l^2) | dot: sigma_0^2
@@ -54,6 +56,47 @@ static inline int make_outer_hyp(int outer, const double* h_hyp, OuterHyp* out) 
     }
     set_error("unknown outer kernel id %d (hot path covers gaussian, matern, expsinesquared, rationalquadratic, dotproduct)", outer);
     return -1;
+}
+
+// f(std::integral_constant<int, OUTER>{}) for a run-time outer id, the one place an id becomes a template argument.  An id
+// make_outer_hyp refuses maps to ExpSineSquared, as the else-branch of every formula below does; the entry points validate first.
+template <class F>
+static inline auto with_outer(int outer, F&& f) {
+    switch (outer) {
+        case DQGP_OUTER_GAUSSIAN: return f(std::integral_constant<int, DQGP_OUTER_GAUSSIAN>{});
+        case DQGP_OUTER_MATERN15: return f(std::integral_constant<int, DQGP_OUTER_MATERN15>{});
+        case DQGP_OUTER_RATQUAD: return f(std::integral_constant<int, DQGP_OUTER_RATQUAD>{});
+        case DQGP_OUTER_DOTPRODUCT: return f(std::integral_constant<int, DQGP_OUTER_DOTPRODUCT>{});
+        default: return f(std::integral_constant<int, DQGP_OUTER_EXPSINE2>{});
+    }
+}
+
+// Lower 64x64 tile (bi >= bj) number `local` of a symmetric tile grid, row-major over the lower triangle
+__device__ __forceinline__ void tile_from_index(int local, int& bi, int& bj) {
+    bi = int((sqrt(8.0 * local + 1.0) - 1.0) * 0.5);
+    while ((bi + 1) * (bi + 2) / 2 <= local) ++bi;
+    while (bi * (bi + 1) / 2 > local) --bi;
+    bj = local - bi * (bi + 1) / 2;
+}
+
+// Stage the 64-sample tiles of F1 from row0 and of F2 from col0 into Fr and Fc (zero padding in k up to mp = m rounded up to 4,
+// and past n1 / n2) and their squared norms into nr[0, 64) and nr[64, 128): four threads per sample row.  tid = threadIdx.x, read
+// by the kernel, where the compiler knows it is below the launch bound (so row0 + r is an OR).
+__device__ __forceinline__ void pw_stage_two_tiles(double* Fr, double* Fc, double* nr, const double* __restrict__ F1, int n1,
+                                                   const double* __restrict__ F2, int n2, int m, int mp, int row0, int col0, int tid) {
+    const int r = tid >> 2, l4 = tid & 3;
+    const bool vr = row0 + r < n1, vc = col0 + r < n2;
+    const double* sr = F1 + (size_t)min(row0 + r, n1 - 1) * m;
+    const double* sc = F2 + (size_t)min(col0 + r, n2 - 1) * m;
+    double pr = 0.0, pc = 0.0;
+    for (int k = l4; k < mp; k += 4) {
+        const double a = (k < m && vr) ? sr[k] : 0.0, b = (k < m && vc) ? sc[k] : 0.0;
+        Fr[r * G2_PITCH + k] = a; Fc[r * G2_PITCH + k] = b;
+        pr = fma(a, a, pr); pc = fma(b, b, pc);
+    }
+    pr += __shfl_xor_sync(0xffffffffu, pr, 1); pr += __shfl_xor_sync(0xffffffffu, pr, 2);
+    pc += __shfl_xor_sync(0xffffffffu, pc, 1); pc += __shfl_xor_sync(0xffffffffu, pc, 2);
+    if (l4 == 0) { nr[r] = pr; nr[PW_TILE + r] = pc; }
 }
 
 // 1/x from the MUFU.RCP64H seed and one cubic Newton step y (1 + e + e^2), e = 1 - x y: 3 DFMA, no range branch.  Meant for
@@ -136,9 +179,32 @@ __device__ __forceinline__ double outer_grad_from_neg_gd2(double v, const OuterH
     }
 }
 
+// Whether outer_grad_from_neg_gd2 has an exponent to clamp: only these outer kernels have a CLAMP = true form
+__host__ __device__ constexpr bool outer_has_exponent(int outer) {
+    return outer != DQGP_OUTER_RATQUAD && outer != DQGP_OUTER_DOTPRODUCT;
+}
+
+// Whether the fused gradient may skip the exponent clamp (CLAMP = false).  Pauli features lie in [-1, 1], so the exponent's
+// argument is bounded below by -gamma 4m (Gaussian), -sqrt(3) 2 sqrt(m) / l (Matern), -2 / l^2 (ExpSineSquared).
+static inline bool outer_grad_no_clamp(int outer, const OuterHyp& h, int m) {
+    const double worst = outer == DQGP_OUTER_GAUSSIAN ? 4.0 * m * h.a
+                         : outer == DQGP_OUTER_MATERN15 ? 1.7320508075688772 * 2.0 * sqrt((double)m) * h.a : 2.0 * h.a * h.a;
+    return h.a > 0.0 && worst < 650.0;
+}
+
+// gamma_eff of the fused gradient's v = -gamma_eff d^2.  The Gaussian folds 32/ln2 into it, so the exponent's argument leaves the
+// DMMA in the units its range reduction wants.  The host pre-multiplies the norm buffer by -gamma_eff, the kernel its row operand
+// by 2 gamma_eff.
+__host__ __device__ __forceinline__ double outer_grad_gamma_eff(int outer, const OuterHyp& h) {
+    return outer == DQGP_OUTER_GAUSSIAN ? h.a * DQGP_EXP_S32 : 1.0;
+}
+
+// The dot product's entries of the fused gradient's norm buffer: sigma_0^2 / 2 each, so the accumulator starts at exactly sigma_0^2
+static inline double outer_grad_dot_norm(const OuterHyp& h) { return 0.5 * h.a; }
+
 // The analytic gradient's per-pair weight (grad_analytic_rows_kernel) from s = |f_j - f_k|^2, for a stationary outer kernel
 // K = kappa(s): kappa'(s), with d = sqrt(s), a and b as in OuterHyp.  The Gaussian returns e^{-gamma s} and leaves -gamma to the
-// contraction's scale.
+// contraction's scale (outer_analytic_scale).
 //   Matern 1.5:        -(3/2) a^2 e^{-sqrt(3) a d}
 //   ExpSineSquared:    -a^2 b (sin(2 b d) / d) kappa, kappa = e^{-2 a^2 sin^2(b d)}
 //   RationalQuadratic: -alpha a base^{-alpha-1}, base = 1 + a s (alpha = 1: -a / base^2)
@@ -168,6 +234,16 @@ __device__ __forceinline__ double outer_analytic_weight(double s, const OuterHyp
         const double k = fast_exp(fmax(-2.0 * (h.a * h.a) * (sn * sn), -700.0));
         return (-2.0 * h.a * h.a * h.b) * (sn * cs / d) * k;
     }
+}
+
+// ALPHA1 of outer_analytic_weight: only RationalQuadratic has the alpha = 1 form, which the host picks per launch when alpha is 1
+__host__ __device__ constexpr bool outer_has_alpha1_form(int outer) { return outer == DQGP_OUTER_RATQUAD; }
+static inline bool outer_analytic_alpha1(int outer, const OuterHyp& h) { return outer_has_alpha1_form(outer) && h.b == 1.0; }
+
+// The analytic gradient's contraction scale: grad_i = scale sum_j <J_ij, G_j>.  Stationary kernels give 2 (the Gaussian -2 gamma,
+// the -gamma its weight leaves out); the dot product, whose G_j = (B F)_j, gives 1.
+static inline double outer_analytic_scale(int outer, const OuterHyp& h) {
+    return outer == DQGP_OUTER_GAUSSIAN ? -2.0 * h.a : outer == DQGP_OUTER_DOTPRODUCT ? 1.0 : 2.0;
 }
 
 // The hyper-parameter gradient's per-pair terms (grad_hyper_dmma_kernel) from s = |f_j - f_k|^2 >= 0: dK/dh_0 and dK/dh_1 up to
@@ -203,6 +279,20 @@ __device__ __forceinline__ void outer_hyper_terms(double s, const OuterHyp& h, d
     }
 }
 
+// c0 and c1 of outer_hyper_terms, from the hyper-parameters as given in h_hyp (NULL = all 1); returns the number of derivatives
+static inline int outer_hyper_scales(int outer, const OuterHyp& h, const double* h_hyp, double& c0, double& c1) {
+    const double pi = 3.14159265358979323846;
+    const double h0 = h_hyp ? h_hyp[0] : 1.0;
+    c0 = 1.0; c1 = 0.0;
+    switch (outer) {
+        case DQGP_OUTER_MATERN15: c0 = h.a; return 1;
+        case DQGP_OUTER_EXPSINE2: c0 = 4.0 * h.a * h.a * h.a; c1 = 4.0 * h.a * h.a * h.b * h.b / pi; return 2;
+        case DQGP_OUTER_RATQUAD: c0 = 2.0 * h.b / h0; c1 = 1.0; return 2;
+        case DQGP_OUTER_DOTPRODUCT: c0 = 2.0 * h0; return 1;
+        default: return 1;
+    }
+}
+
 // out[row] = add (+ |F[row]|^2 when with_norm), rows of m features (gram.cu)
 void launch_self_kernel(const double* F, long long rows, int m, double add, bool with_norm, double* out, cudaStream_t st);
 
@@ -213,7 +303,5 @@ int fidelity_grad_dmma(const double* Ainv, int ld, const double* alpha, const do
 // W = [B o Re S | B o Im S] (n_pad x 2 n_pad, every entry written), S_jk = <psi_k|psi_j>, B = A^-1 - alpha alpha^T
 int fidelity_weights_dmma(const double* Ainv, int ld, const double* alpha, const double* Psi, int n, int dim, double* W, int n_pad,
                           cudaStream_t st);
-
-constexpr int G2_PITCH = 36;   // doubles per staged sample row: = 4 (mod 16) -> conflict-free DMMA fragment loads
 
 }  // namespace dqgp

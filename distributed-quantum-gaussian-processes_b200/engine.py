@@ -21,11 +21,10 @@ import torch
 
 from . import _lib
 from ._lib import OUTER_KERNELS, DqgpError, check
-from .kernels import EncodingCircuit, _require_cuda, dev_f64, outer_hyp, stream_ptr
+from .kernels import OUTER_HYPERPARAMETERS, EncodingCircuit, _require_cuda, dev_f64, outer_hyp, stream_ptr
 
 PERIOD = float(np.pi)
-HYPER_NAMES = {"gaussian": ("gamma",), "matern": ("length_scale",), "expsinesquared": ("length_scale", "periodicity"),
-               "rationalquadratic": ("length_scale", "alpha"), "dotproduct": ("sigma_0",), "pairwisekernel": ()}
+HYPER_NAMES = {kernel: tuple(name for name, _ in hyper) for kernel, hyper in OUTER_HYPERPARAMETERS.items()}
 
 
 class _DeviceMatrix:

@@ -86,29 +86,34 @@ class Executor:
         return f"Executor({self.name}) [dqgp_b200 statevector]"
 
 
+# scikit-learn's hyper-parameters of each outer kernel with their defaults (the only values the reference reaches, Q2), in the
+# order of the h_hyp vector: gaussian {gamma}; matern {length_scale} (nu = 1.5); expsinesquared {length_scale, periodicity};
+# rationalquadratic {length_scale, alpha}; dotproduct {sigma_0}.  pairwisekernel has none: scikit-learn's
+# PairwiseKernel(metric="linear") is f.g, the dot product with sigma_0 = 0 (its gamma is accepted and ignored, as
+# filter_params=True does).
+OUTER_HYPERPARAMETERS = {
+    "gaussian": (("gamma", 1.0),),
+    "matern": (("length_scale", 1.0),),
+    "expsinesquared": (("length_scale", 1.0), ("periodicity", 1.0)),
+    "rationalquadratic": (("length_scale", 1.0), ("alpha", 1.0)),
+    "dotproduct": (("sigma_0", 1.0),),
+    "pairwisekernel": (),
+}
+
+
 def outer_hyp(outer_kernel, params=None):
-    """Host hyper-parameter vector of an outer kernel: gaussian {gamma}; matern {length_scale} (nu = 1.5);
-    expsinesquared {length_scale, periodicity}; rationalquadratic {length_scale, alpha}; dotproduct {sigma_0};
-    pairwisekernel {0.0}: scikit-learn's PairwiseKernel(metric="linear") is f.g, the dot product with sigma_0 = 0 (its
-    gamma is accepted and ignored, as filter_params=True does).  Defaults = the only values the reference reaches (Q2)."""
+    """Host hyper-parameter vector of an outer kernel (OUTER_HYPERPARAMETERS) from the reference's dict format;
+    pairwisekernel gives {0.0}, the dot product's sigma_0."""
     params = dict(params or {})
-    if outer_kernel == "gaussian":
-        return [float(params.get("gamma", 1.0))]
-    if outer_kernel == "matern":
-        if float(params.get("nu", 1.5)) != 1.5:
-            raise ValueError("only Matern nu=1.5 is on the hot path")
-        return [float(params.get("length_scale", 1.0))]
-    if outer_kernel == "expsinesquared":
-        return [float(params.get("length_scale", 1.0)), float(params.get("periodicity", 1.0))]
-    if outer_kernel == "rationalquadratic":
-        return [float(params.get("length_scale", 1.0)), float(params.get("alpha", 1.0))]
-    if outer_kernel == "dotproduct":
-        return [float(params.get("sigma_0", 1.0))]
+    if outer_kernel not in OUTER_HYPERPARAMETERS:
+        raise ValueError(f"outer kernel {outer_kernel!r} is outside the hot path (supported: {sorted(OUTER_KERNELS)})")
+    if outer_kernel == "matern" and float(params.get("nu", 1.5)) != 1.5:
+        raise ValueError("only Matern nu=1.5 is on the hot path")
     if outer_kernel == "pairwisekernel":
         if params.get("metric", "linear") != "linear":
             raise ValueError(f"only PairwiseKernel metric='linear' is on the hot path (got {params['metric']!r})")
         return [0.0]
-    raise ValueError(f"outer kernel {outer_kernel!r} is outside the hot path (supported: {sorted(OUTER_KERNELS)})")
+    return [float(params.get(name, default)) for name, default in OUTER_HYPERPARAMETERS[outer_kernel]]
 
 
 class _QuantumKernel:
