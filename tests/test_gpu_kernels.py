@@ -178,9 +178,9 @@ def test_dgemm_rejects_bad_shapes(d):
     assert b"multiples" in lib.dqgp_last_error()
 
 
-@pytest.mark.parametrize("dim,offset,message", [(3, 0, b"2^q"), (24, 0, b"2^q"), (8, 1, b"16-byte aligned")])
+@pytest.mark.parametrize("dim,offset,message", [(3, 0, b"2^q"), (24, 0, b"2^q"), (8192, 0, b"2^q"), (8, 1, b"16-byte aligned")])
 def test_fidelity_entry_points_reject_unsupported_states(d, dim, offset, message):
-    """dqgp_gram_fidelity / dqgp_grad_fidelity take 2^q amplitudes (q >= 1) per state and 16-byte aligned state arrays: the DMMA
+    """dqgp_gram_fidelity / dqgp_grad_fidelity take 2^q amplitudes (1 <= q <= 12) per state and 16-byte aligned state arrays: the DMMA
     kernel splits every state into chunks of 4k doubles and copies them with the TMA engine.  Anything else is refused before a
     launch, with a message."""
     n, P = 5, 1
